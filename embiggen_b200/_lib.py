@@ -106,6 +106,10 @@ SIGNATURES = {
     "b2e_cooccurrence": (ctypes.c_int, [_H, _U64, _U64, _U64, _U64, ctypes.c_int, _P(_U64)]),
     "b2e_cooccurrence_export": (ctypes.c_int, [_H, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "b2e_glove_train": (ctypes.c_int, [_H, _F32]),
+    "b2e_glove_walk_epoch": (ctypes.c_int, [_H, _U64, _U64, _U64]),
+    "b2e_glove_shard_count": (ctypes.c_int, [_H, _U32, _U32, ctypes.c_void_p, _P(_U32)]),
+    "b2e_glove_shard_train": (ctypes.c_int, [_H, _F32, _U32]),
+    "b2e_glove_merge": (ctypes.c_int, [_H]),
     "b2e_number_of_sources": (_U64, [_H]),
     "b2e_row_stride": (_U64, [_H]),
     "b2e_fit": (ctypes.c_int, [_H, _U64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),

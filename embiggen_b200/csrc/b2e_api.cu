@@ -1115,16 +1115,19 @@ extern "C" int b2e_glove_train(b2e_handle *h, float learning_rate) {
     return B2E_OK;
 }
 
-// One GloVe epoch whose co-occurrence exceeds one sort (glove.cu, "co-occurrence by centre
-// range"): walk the whole epoch, bucket the token positions by centre range, then count and train
-// range by range in ascending order of centre.  x_max is the largest count of the WHOLE epoch, so
-// with more than one range the ranges are counted twice: once for x_max, once to train.
-static int glove_epoch_by_ranges(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t per_epoch, float lr,
-                                 uint64_t capacity_slots) {
-    const b2e_config &c = h->cfg;
+// ---- GloVe by centre range (glove.cu, "co-occurrence by centre range") ----
+// An epoch whose co-occurrence exceeds one sort is walked whole, its token positions are bucketed
+// by range of centre id, and the ranges are counted and trained one by one in ascending order of
+// centre.  x_max is the largest count of the WHOLE epoch, so with more than one range the ranges
+// are counted twice: once for x_max, once to train.  The same steps make the sharded epoch of
+// several GPUs: every rank walks the whole epoch, then counts and trains only the centres it owns.
+
+// the walks of a whole epoch into HBM, and their token histogram (host copy in g.histogram)
+static int glove_walk_epoch(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t per_epoch) {
     GloveState &g = h->glove;
-    const uint32_t L = c.walk_length, W = c.window_size;
+    const uint32_t L = h->cfg.walk_length;
     const uint64_t tokens = per_epoch * L;
+    g.histogram.clear();
     CUDA_TRY(glove_reserve((void **)&g.d_epoch_walks, &g.epoch_walks_bytes, tokens * sizeof(uint32_t)));
     CUDA_TRY(glove_reserve((void **)&g.d_histogram, &g.histogram_bytes, h->n * sizeof(uint32_t)));
     for (uint64_t done = 0; done < per_epoch; done += h->chunk_cap) {
@@ -1137,56 +1140,90 @@ static int glove_epoch_by_ranges(b2e_handle *h, uint64_t seed, uint64_t first_wa
                              h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     h->launches += 2;
-    // ranges of centre ids holding at most capacity_slots key slots each (one node may exceed it)
-    std::vector<uint32_t> bounds(1, 0u);
+    g.histogram.swap(histogram);
+    g.epoch_tokens = tokens;
+    return B2E_OK;
+}
+
+// Cut the centres [lo, hi) into ranges holding at most capacity_slots key slots each (one node
+// may exceed it) and bucket the positions of their tokens by range (tokens of other centres are
+// skipped).
+static int glove_bucket_ranges(b2e_handle *h, uint32_t lo, uint32_t hi, uint64_t capacity_slots) {
+    GloveState &g = h->glove;
+    const uint32_t W = h->cfg.window_size;
+    std::vector<uint32_t> bounds(1, lo);
     std::vector<unsigned long long> offsets(1, 0ull);
     uint64_t in_range = 0, placed = 0;
-    for (uint64_t v = 0; v < h->n; ++v) {
-        const uint64_t slots = (uint64_t)histogram[v] * 2ull * W;
+    for (uint64_t v = lo; v < hi; ++v) {
+        const uint64_t slots = (uint64_t)g.histogram[v] * 2ull * W;
         if (in_range && in_range + slots > capacity_slots) {
             bounds.push_back((uint32_t)v);
             offsets.push_back(placed);
             in_range = 0;
         }
         in_range += slots;
-        placed += histogram[v];
+        placed += g.histogram[v];
         if (slots >= (1ull << 31))
             return fail(B2E_ERR_INVALID, "one node alone has 2^31 co-occurrence slots in an epoch: lower walk_length, "
                                          "window_size or iterations");
     }
-    bounds.push_back((uint32_t)h->n);
+    bounds.push_back(hi);
     offsets.push_back(placed);
     const uint32_t ranges = (uint32_t)bounds.size() - 1u;
     g.last_ranges = ranges;
+    g.range_kept = false;
     CUDA_TRY(glove_reserve((void **)&g.d_bounds, &g.bounds_bytes, bounds.size() * sizeof(uint32_t)));
     CUDA_TRY(glove_reserve((void **)&g.d_cursor, &g.cursor_bytes, ranges * sizeof(unsigned long long)));
     CUDA_TRY(glove_reserve((void **)&g.d_positions, &g.positions_bytes, std::max<uint64_t>(placed, 1) * sizeof(unsigned long long)));
     CUDA_TRY(cudaMemcpyAsync(g.d_bounds, bounds.data(), bounds.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->walk_stream));
     CUDA_TRY(cudaMemcpyAsync(g.d_cursor, offsets.data(), ranges * sizeof(unsigned long long), cudaMemcpyHostToDevice, h->walk_stream));
-    CUDA_TRY(glove_bucket_positions(g.d_epoch_walks, tokens, g.d_bounds, ranges, g.d_cursor, g.d_positions, h->walk_stream));
+    CUDA_TRY(glove_bucket_positions(g.d_epoch_walks, g.epoch_tokens, g.d_bounds, ranges, g.d_cursor, g.d_positions,
+                                    h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     ++h->launches;
-    uint32_t x_max = 1;
-    if (ranges > 1) {
-        for (uint32_t r = 0; r < ranges; ++r) {
-            CUDA_TRY(glove_range_triples(g, g.d_epoch_walks, L, W, g.d_positions + offsets[r], offsets[r + 1] - offsets[r],
-                                         h->walk_stream));
-            uint32_t local = 0;
-            CUDA_TRY(glove_max_count(g, &local, h->walk_stream));
-            x_max = std::max(x_max, local);
-            h->launches += 2;
-        }
-    }
+    g.range_bounds.swap(bounds);
+    g.range_offsets.swap(offsets);
+    return B2E_OK;
+}
+
+static int glove_count_range(b2e_handle *h, uint32_t r) {
+    GloveState &g = h->glove;
+    CUDA_TRY(glove_range_triples(g, g.d_epoch_walks, h->cfg.walk_length, h->cfg.window_size,
+                                 g.d_positions + g.range_offsets[r], g.range_offsets[r + 1] - g.range_offsets[r],
+                                 h->walk_stream));
+    h->launches += 2;
+    return B2E_OK;
+}
+
+// the largest count of the bucketed ranges (0 without triples); a single range keeps its triples
+static int glove_count_ranges(b2e_handle *h, uint32_t *largest) {
+    GloveState &g = h->glove;
+    const uint32_t ranges = (uint32_t)g.range_bounds.size() - 1u;
+    *largest = 0;
     for (uint32_t r = 0; r < ranges; ++r) {
-        CUDA_TRY(glove_range_triples(g, g.d_epoch_walks, L, W, g.d_positions + offsets[r], offsets[r + 1] - offsets[r],
-                                     h->walk_stream));
-        h->launches += 2;
+        if (int rc = glove_count_range(h, r)) return rc;
+        uint32_t local = 0;
+        CUDA_TRY(glove_max_count(g, &local, h->walk_stream));
+        *largest = std::max(*largest, local);
+    }
+    g.range_kept = ranges == 1;
+    return B2E_OK;
+}
+
+// one SGD pass over the bucketed ranges in ascending order of centre, weights against x_max
+static int glove_train_ranges(b2e_handle *h, float lr, uint32_t x_max) {
+    GloveState &g = h->glove;
+    const uint32_t ranges = (uint32_t)g.range_bounds.size() - 1u;
+    for (uint32_t r = 0; r < ranges; ++r) {
+        if (!g.range_kept)
+            if (int rc = glove_count_range(h, r)) return rc;
         if (g.n_triples == 0) continue;
         CUDA_TRY(glove_finalise(g, h->n, h->walk_stream));
-        if (ranges > 1) g.max_count = x_max;
+        g.max_count = x_max;
         if (int rc = b2e_glove_train(h, lr)) return rc;
         CUDA_TRY(cudaStreamSynchronize(h->train_stream));  // the triples are replaced by the next range
     }
+    g.range_kept = false;
     return B2E_OK;
 }
 
@@ -1194,6 +1231,92 @@ static int glove_epoch_by_ranges(b2e_handle *h, uint64_t seed, uint64_t first_wa
 static uint64_t glove_capacity_slots() {
     if (const char *env = getenv("B2E_GLOVE_SLOTS")) return std::max<uint64_t>(64, strtoull(env, nullptr, 10));
     return 1ull << 28;
+}
+
+static int glove_epoch_by_ranges(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t per_epoch, float lr,
+                                 uint64_t capacity_slots) {
+    if (int rc = glove_walk_epoch(h, seed, first_walk, per_epoch)) return rc;
+    if (int rc = glove_bucket_ranges(h, 0, (uint32_t)h->n, capacity_slots)) return rc;
+    uint32_t x_max = 0;
+    if (int rc = glove_count_ranges(h, &x_max)) return rc;
+    return glove_train_ranges(h, lr, x_max);
+}
+
+// Owners of a sharded epoch: with S the key slots of the epoch (2 W per token) and c_v the slots
+// of the nodes before v, rank r owns the nodes with r S / G <= c_v < (r + 1) S / G; nodes past the
+// last slot go to the last rank.  A pure function of the histogram: every rank finds the same bounds.
+static void glove_owner_bounds(const std::vector<uint32_t> &histogram, uint32_t W, uint32_t world, uint32_t *bounds) {
+    const uint64_t n = histogram.size();
+    uint64_t total = 0;
+    for (const uint32_t tokens : histogram) total += (uint64_t)tokens * 2ull * W;
+    bounds[0] = 0;
+    uint32_t r = 1;
+    uint64_t before = 0;
+    for (uint64_t v = 0; v < n && r < world; ++v) {
+        while (r < world && before * world >= r * total) bounds[r++] = (uint32_t)v;
+        before += (uint64_t)histogram[v] * 2ull * W;
+    }
+    while (r <= world) bounds[r++] = (uint32_t)n;
+}
+
+static int require_glove(b2e_handle *h) {
+    if (int rc = require_graph(h)) return rc;
+    if (h->cfg.model != B2E_GLOVE) return fail(B2E_ERR_STATE, "the handle was not created for GloVe");
+    return B2E_OK;
+}
+
+extern "C" int b2e_glove_walk_epoch(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t n_walks) {
+    REQUIRE_HANDLE(h);
+    if (int rc = require_glove(h)) return rc;
+    if (h->n_src == 0) return fail(B2E_ERR_INVALID, "the graph has no node with outgoing edges");
+    if (int rc = b2e_sync(h)) return rc;
+    return glove_walk_epoch(h, seed, first_walk, n_walks);
+}
+
+extern "C" int b2e_glove_shard_count(b2e_handle *h, uint32_t world, uint32_t rank, uint32_t *owner_bounds,
+                                     uint32_t *local_max) {
+    REQUIRE_HANDLE(h);
+    if (int rc = require_glove(h)) return rc;
+    if (int rc = check_world(world, rank)) return rc;
+    if (!local_max) return fail(B2E_ERR_INVALID, "null argument");
+    GloveState &g = h->glove;
+    if (g.histogram.size() != h->n) return fail(B2E_ERR_STATE, "b2e_glove_walk_epoch must be called first");
+    if (int rc = b2e_sync(h)) return rc;
+    glove_owner_bounds(g.histogram, h->cfg.window_size, world, g.owner_bounds);
+    g.owner_world = world;
+    if (owner_bounds) memcpy(owner_bounds, g.owner_bounds, (world + 1) * sizeof(uint32_t));
+    if (int rc = glove_bucket_ranges(h, g.owner_bounds[rank], g.owner_bounds[rank + 1], glove_capacity_slots())) return rc;
+    return glove_count_ranges(h, local_max);
+}
+
+extern "C" int b2e_glove_shard_train(b2e_handle *h, float learning_rate, uint32_t max_count) {
+    REQUIRE_HANDLE(h);
+    if (int rc = require_glove(h)) return rc;
+    GloveState &g = h->glove;
+    if (g.owner_world == 0 || g.range_bounds.empty())
+        return fail(B2E_ERR_STATE, "b2e_glove_shard_count must be called first");
+    if (g.owner_world > 1) {  // the base of the merge: T1 before this epoch's training (same stream, ordered)
+        const size_t bytes = h->n * (size_t)h->row_stride * sizeof(float);
+        CUDA_TRY(glove_reserve((void **)&g.d_t1_snapshot, &g.t1_snapshot_bytes, bytes));
+        CUDA_TRY(cudaMemcpyAsync(g.d_t1_snapshot, h->d_t1, bytes, cudaMemcpyDeviceToDevice, h->train_stream));
+    }
+    const int rc = glove_train_ranges(h, learning_rate, std::max(max_count, 1u));
+    g.range_bounds.clear();  // trained: the next epoch counts anew
+    return rc;
+}
+
+extern "C" int b2e_glove_merge(b2e_handle *h) {
+    REQUIRE_HANDLE(h);
+    if (int rc = require_glove(h)) return rc;
+    if (h->world < 2) return B2E_OK;
+    GloveState &g = h->glove;
+    if (g.owner_world != h->world || !g.d_t1_snapshot)
+        return fail(B2E_ERR_STATE, "b2e_glove_shard_count and b2e_glove_shard_train with the world of the exchange "
+                                   "must come first");
+    CUDA_TRY(launch_glove_merge(h->peer_t0, h->peer_t1, g.d_t1_snapshot, g.owner_bounds, h->world, h->rank, h->n,
+                                h->row_stride, (h->cfg.embedding_size + 3u) / 4u, h->sm_count, h->train_stream));
+    ++h->launches;
+    return B2E_OK;
 }
 
 static int fit_glove(b2e_handle *h, uint64_t seed, float *table0, float *table1, float *epoch_loss) {

@@ -113,6 +113,15 @@ struct GloveState {
     unsigned long long *d_positions = nullptr, *d_cursor = nullptr;
     size_t epoch_walks_bytes = 0, histogram_bytes = 0, bounds_bytes = 0, positions_bytes = 0, cursor_bytes = 0;
     uint32_t last_ranges = 0;  // how many centre ranges the last epoch took (1 = one piece)
+    uint64_t epoch_tokens = 0;                    // tokens of the walked epoch (d_epoch_walks)
+    std::vector<uint32_t> histogram;              // tokens per node of the walked epoch (host copy)
+    std::vector<uint32_t> range_bounds;           // range r: range_bounds[r] <= centre < range_bounds[r + 1]
+    std::vector<unsigned long long> range_offsets;  // bucketed occurrences before range r
+    bool range_kept = false;                      // one range: its triples are resident, counted once
+    // sharded epoch (several GPUs): rank r owns the centres [owner_bounds[r], owner_bounds[r + 1])
+    uint32_t owner_world = 0, owner_bounds[B2E_MAX_WORLD + 1] = {0};
+    float *d_t1_snapshot = nullptr;  // T1 as it stood before this epoch's training (the merge's base)
+    size_t t1_snapshot_bytes = 0;
 };
 uint64_t glove_chunk_walks(uint32_t walk_length, uint32_t window);
 cudaError_t glove_accumulate(GloveState &g, const uint32_t *d_walks, uint64_t n_walks, uint32_t walk_length,
@@ -153,6 +162,12 @@ cudaError_t launch_row_filter_build(const int64_t *indptr, const uint32_t *indic
 cudaError_t launch_exchange_average(float *const t0[], float *const t1[], uint32_t world, uint32_t rank,
                                     uint64_t n, uint32_t row_stride, uint32_t chunks, int sm_count,
                                     cudaStream_t stream, uint32_t rows_per_iteration = 0);
+// GloVe's merge of a sharded epoch: every replica takes row v of T0 from the replica of its owner
+// and T1 = snapshot + sum over the ranks of (T1_g - snapshot); this rank reduces the rows
+// [n rank / world, n (rank + 1) / world)
+cudaError_t launch_glove_merge(float *const t0[], float *const t1[], const float *snapshot,
+                               const uint32_t *owner_bounds, uint32_t world, uint32_t rank, uint64_t n,
+                               uint32_t row_stride, uint32_t chunks, int sm_count, cudaStream_t stream);
 cudaError_t launch_pack_rows(const float *table, uint64_t rows, uint32_t row_stride, uint32_t dim, float *dense,
                              int sm_count, cudaStream_t stream);
 cudaError_t launch_tables_digest(const float *t0, const float *t1, uint64_t n, uint32_t row_stride,

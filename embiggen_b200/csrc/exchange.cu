@@ -119,6 +119,99 @@ cudaError_t launch_exchange_average(float *const t0[], float *const t1[], uint32
     return cudaGetLastError();
 }
 
+// GloVe's merge of a sharded epoch.  Every rank trained only the centres it owns, so averaging the
+// replicas would divide each owner's T0 change and each rank's T1 change by G.  Instead: row v of
+// T0 is taken from the replica of owner(v) (the only one that changed it), and T1 becomes
+// snapshot + ((T1_0 - snapshot) + (T1_1 - snapshot) + ...), rank order, every operation rounded
+// to nearest -- the sum of all ranks' changes on the common starting point.  The snapshot is the
+// same on every replica (they were bit-identical when it was taken), so each rank reads its own.
+// Rows are split among the ranks and moved like exchange_average_kernel's (one warp per (table,
+// row), only the ceil(D / 4) live chunks); afterwards the replicas are bit-identical again.
+struct GloveMergeParams {
+    float *t[2][B2E_MAX_WORLD];
+    const float *snapshot;
+    uint32_t owner_bounds[B2E_MAX_WORLD + 1];
+    uint32_t world;
+    uint64_t row_begin, row_end;
+    uint32_t row_stride, chunks;
+};
+
+template <int G>
+__global__ void __launch_bounds__(256) glove_merge_kernel(const GloveMergeParams p) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint64_t warps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
+    const uint64_t rows = p.row_end - p.row_begin, items = 2 * rows;
+    constexpr int GG = G ? G : B2E_MAX_WORLD;
+    const uint32_t world = G ? (uint32_t)G : p.world;
+    for (uint64_t item = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; item < items; item += warps) {
+        const bool second = item >= rows;  // warp-uniform
+        const uint64_t row = p.row_begin + (second ? item - rows : item), at = row * p.row_stride;
+        if (!second) {
+            uint32_t owner = 0;  // last rank whose interval starts at or before the row
+            while (owner + 1 < world && row >= p.owner_bounds[owner + 1]) ++owner;
+            for (uint32_t c = lane; c < p.chunks; c += 32u) {
+                const float4 v = __ldcg(reinterpret_cast<const float4 *>(p.t[0][owner] + at) + c);
+#pragma unroll
+                for (int g = 0; g < GG; ++g)
+                    if ((uint32_t)g < world && (uint32_t)g != owner)
+                        __stcg(reinterpret_cast<float4 *>(p.t[0][g] + at) + c, v);
+            }
+            continue;
+        }
+        for (uint32_t c = lane; c < p.chunks; c += 32u) {
+            const float4 s = __ldcg(reinterpret_cast<const float4 *>(p.snapshot + at) + c);
+            float4 v[GG];
+#pragma unroll
+            for (int g = 0; g < GG; ++g)
+                if ((uint32_t)g < world) v[g] = __ldcg(reinterpret_cast<const float4 *>(p.t[1][g] + at) + c);
+            float4 d = make_float4(__fsub_rn(v[0].x, s.x), __fsub_rn(v[0].y, s.y), __fsub_rn(v[0].z, s.z),
+                                   __fsub_rn(v[0].w, s.w));
+#pragma unroll
+            for (int g = 1; g < GG; ++g) {
+                if ((uint32_t)g < world) {
+                    d.x = __fadd_rn(d.x, __fsub_rn(v[g].x, s.x));
+                    d.y = __fadd_rn(d.y, __fsub_rn(v[g].y, s.y));
+                    d.z = __fadd_rn(d.z, __fsub_rn(v[g].z, s.z));
+                    d.w = __fadd_rn(d.w, __fsub_rn(v[g].w, s.w));
+                }
+            }
+            const float4 out = make_float4(__fadd_rn(s.x, d.x), __fadd_rn(s.y, d.y), __fadd_rn(s.z, d.z),
+                                           __fadd_rn(s.w, d.w));
+#pragma unroll
+            for (int g = 0; g < GG; ++g)
+                if ((uint32_t)g < world) __stcg(reinterpret_cast<float4 *>(p.t[1][g] + at) + c, out);
+        }
+    }
+}
+
+cudaError_t launch_glove_merge(float *const t0[], float *const t1[], const float *snapshot,
+                               const uint32_t *owner_bounds, uint32_t world, uint32_t rank, uint64_t n,
+                               uint32_t row_stride, uint32_t chunks, int sm_count, cudaStream_t stream) {
+    if (world < 2 || n == 0) return cudaSuccess;
+    GloveMergeParams p;
+    for (uint32_t g = 0; g < world; ++g) {
+        p.t[0][g] = t0[g];
+        p.t[1][g] = t1[g];
+    }
+    for (uint32_t r = 0; r <= world; ++r) p.owner_bounds[r] = owner_bounds[r];
+    p.snapshot = snapshot;
+    p.world = world;
+    p.row_begin = n * rank / world;
+    p.row_end = n * (rank + 1ull) / world;
+    p.row_stride = row_stride;
+    p.chunks = chunks;
+    const uint64_t rows = p.row_end - p.row_begin;
+    if (rows == 0) return cudaSuccess;
+    const unsigned grid = (unsigned)std::min<uint64_t>((2 * rows + 7) / 8, (uint64_t)sm_count * 8);
+    switch (world) {
+        case 2: glove_merge_kernel<2><<<grid, 256, 0, stream>>>(p); break;
+        case 4: glove_merge_kernel<4><<<grid, 256, 0, stream>>>(p); break;
+        case 8: glove_merge_kernel<8><<<grid, 256, 0, stream>>>(p); break;
+        default: glove_merge_kernel<0><<<grid, 256, 0, stream>>>(p); break;
+    }
+    return cudaGetLastError();
+}
+
 // Strip the row padding on the device: `rows` rows of `chunks` float4 each leave their 128 B-aligned
 // pitch for a dense buffer that one contiguous DMA then carries to the host (a pitched 2-D copy of
 // 400-byte rows moved 80 GB in 12 s; packed and double-buffered it is bound by PCIe).

@@ -447,15 +447,17 @@ __global__ void __launch_bounds__(256) token_histogram_kernel(const uint32_t *__
     }
 }
 
-// position p of a walk token goes to the range that holds its node: bounds[r] <= node < bounds[r + 1]
+// position p of a walk token goes to the range that holds its node: bounds[r] <= node < bounds[r + 1];
+// tokens of nodes outside [bounds[0], bounds[ranges]) (centres another rank owns) are skipped
 __global__ void __launch_bounds__(256) bucket_positions_kernel(const uint32_t *__restrict__ walks, uint64_t tokens,
                                                                const uint32_t *__restrict__ bounds, uint32_t ranges,
                                                                unsigned long long *__restrict__ cursor,
                                                                unsigned long long *__restrict__ positions) {
+    const uint32_t first = __ldg(bounds), last = __ldg(bounds + ranges);
     for (uint64_t p = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; p < tokens;
          p += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t v = __ldg(walks + p);
-        if (v == PAD) continue;
+        if (v == PAD || v < first || v >= last) continue;
         uint32_t lo = 0, hi = ranges;  // last r with bounds[r] <= v
         while (hi - lo > 1) {
             const uint32_t mid = (lo + hi) >> 1;
@@ -565,7 +567,7 @@ void glove_free(GloveState &g) {
     cudaFree(g.d_keys); cudaFree(g.d_counts); cudaFree(g.d_rowptr); cudaFree(g.d_scratch_keys);
     cudaFree(g.d_merge_keys); cudaFree(g.d_merge_counts); cudaFree(g.d_temp); cudaFree(g.d_scalar);
     cudaFree(g.d_epoch_walks); cudaFree(g.d_histogram); cudaFree(g.d_bounds); cudaFree(g.d_positions);
-    cudaFree(g.d_cursor);
+    cudaFree(g.d_cursor); cudaFree(g.d_t1_snapshot);
     g = GloveState();
 }
 

@@ -202,9 +202,7 @@ class Node2VecB200(B200Embedder):
                 node_types, edge_types = as_types(graph)  # a graph without types walks untyped
                 engine.load_types(node_types if self.is_using_node_types() else None,
                                   edge_types if self.is_using_edge_types() else None)
-            if world > 1 and self.MODELS[self.model_name()] == "GloVe":
-                raise NotImplementedError("GloVe runs on one GPU: the co-occurrence counts are not sharded.")
-            if world > 1:
+            if world > 1:  # GloVe shards its centres over the ranks (Engine._fit_glove_distributed)
                 _, _, losses = engine.fit_distributed(seed, self._model_kwargs["sync_interval"],
                                                       table0=central, table1=contextual)
             else:

@@ -260,6 +260,37 @@ class Engine:
     def glove_train(self, learning_rate: float) -> None:
         check(self._lib.b2e_glove_train(self._handle, learning_rate))
 
+    # ---- GloVe on several GPUs: centres sharded over the ranks, replicas merged once per epoch ----
+    def glove_walk_epoch(self, seed: int, first_walk: int, n_walks: int) -> None:
+        """Walk a whole epoch into HBM and take its token histogram (the same on every rank)."""
+        check(self._lib.b2e_glove_walk_epoch(self._handle, seed, first_walk, n_walks))
+
+    def glove_shard_count(self, world: int, rank: int) -> Tuple[int, np.ndarray]:
+        """Count the centres this rank owns; returns (their largest count, the world + 1 owner bounds)."""
+        bounds = np.zeros(world + 1, dtype=np.uint32)
+        local_max = ctypes.c_uint32()
+        check(self._lib.b2e_glove_shard_count(self._handle, world, rank, bounds.ctypes.data,
+                                              ctypes.byref(local_max)))
+        return int(local_max.value), bounds
+
+    def glove_shard_train(self, learning_rate: float, max_count: int) -> None:
+        """One SGD pass over this rank's centres, weights against the epoch's largest count."""
+        check(self._lib.b2e_glove_shard_train(self._handle, learning_rate, max_count))
+
+    def glove_merge(self) -> None:
+        """Launch this rank's share of the GloVe merge (asynchronous); see :meth:`merge`."""
+        check(self._lib.b2e_glove_merge(self._handle))
+
+    def merge(self, process_group=None) -> None:
+        """GloVe's exchange step: every replica takes each T0 row from the rank that owns the
+        centre and the sum of all ranks' T1 changes (bit-identical replicas afterwards)."""
+        import torch.distributed as dist
+        self.sync()                        # my training pass is done ...
+        dist.barrier(group=process_group)  # ... and so is everybody else's
+        self.glove_merge()
+        self.sync()
+        dist.barrier(group=process_group)  # every rank has written its rows to every replica
+
     # ---- K2 parity/debug export ----
     def walks(self, seed: int, first_walk: int, n_walks: int, walk_id_stride: int = 1) -> np.ndarray:
         out = np.empty((n_walks, self.config.walk_length), dtype=np.uint32)
@@ -306,10 +337,13 @@ class Engine:
     def sync(self) -> None:
         check(self._lib.b2e_sync(self._handle))
 
-    def export_tables(self) -> Tuple[np.ndarray, np.ndarray]:
-        """Raw (input table T0, output table T1), padding stripped."""
+    def export_tables(self, table0: Optional[np.ndarray] = None,
+                      table1: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+        """Raw (input table T0, output table T1), padding stripped; into the given C-contiguous
+        float32 buffers when there are any."""
         shape = (self.n, self.config.embedding_size)
-        t0, t1 = np.empty(shape, dtype=np.float32), np.empty(shape, dtype=np.float32)
+        t0 = np.empty(shape, dtype=np.float32) if table0 is None else table0
+        t1 = np.empty(shape, dtype=np.float32) if table1 is None else table1
         check(self._lib.b2e_export_tables(self._handle, t0.ctypes.data, t1.ctypes.data))
         return t0, t1
 
@@ -398,6 +432,7 @@ class Engine:
         Replicas are averaged every ``sync_interval`` chunks and at each epoch end.  Returns
         role-ordered tables like :meth:`fit`; with ``gather="rank0"`` only rank 0 copies them to
         the host (the others return ``None`` tables: at C5 a host copy is 80 GB per rank).
+        A GloVe handle runs :meth:`_fit_glove_distributed` instead (``sync_interval`` does not apply).
         """
         import torch
         import torch.distributed as dist
@@ -405,6 +440,8 @@ class Engine:
         cfg = self.config
         if gather not in ("all", "rank0"):
             raise ValueError("gather must be 'all' or 'rank0'")
+        if self.model == "glove":
+            return self._fit_glove_distributed(seed, process_group, gather, table0, table1)
         self.timings = {}
         self.init_tables(seed)  # identical on every rank (counter-based init)
         opened = world == 1
@@ -456,13 +493,72 @@ class Engine:
             dist.barrier(group=process_group)
             self.close_exchange()
             self.timings["close_exchange_s"] = time.perf_counter() - begin
+        return self._gather_tables(rank, gather, table0, table1, losses)
+
+    def _gather_tables(self, rank, gather, table0, table1, losses):
+        """The end of a data-parallel fit: role-ordered tables to the host on every rank, or on
+        rank 0 only (``gather="rank0"``)."""
         if gather == "rank0" and rank != 0:
             return None, None, losses
-        shape = (self.n, cfg.embedding_size)
+        shape = (self.n, self.config.embedding_size)
         t0 = np.empty(shape, dtype=np.float32) if table0 is None else table0
         t1 = np.empty(shape, dtype=np.float32) if table1 is None else table1
         first, second = (t1, t0) if self.model == "cbow" else (t0, t1)
         begin = time.perf_counter()
-        check(self._lib.b2e_export_tables(self._handle, first.ctypes.data, second.ctypes.data))
+        self.export_tables(first, second)
         self.timings["export_tables_s"] = time.perf_counter() - begin
         return t0, t1, losses
+
+    def _fit_glove_distributed(self, seed, process_group, gather, table0, table1):
+        """GloVe's data-parallel epoch (DESIGN.md K7): every rank walks the whole epoch (walks
+        are a pure function of (seed, walk id)), counts and trains the centres it owns -- exact
+        global counts, weights against the largest count of the whole epoch, taken as a maximum
+        over the ranks -- and the replicas are merged once per epoch (:meth:`merge`).
+        ``timings`` holds the seconds of each phase, summed over the epochs."""
+        import torch
+        import torch.distributed as dist
+        rank, world = dist.get_rank(process_group), dist.get_world_size(process_group)
+        cfg = self.config
+        on_device = dist.get_backend(process_group) == "nccl"
+
+        def all_reduce(values, dtype, op):
+            tensor = torch.tensor(values, dtype=dtype)
+            if on_device:
+                tensor = tensor.to(f"cuda:{cfg.device}")
+            dist.all_reduce(tensor, op=op, group=process_group)
+            return tensor.cpu()
+
+        self.timings = {"walk_histogram_s": 0.0, "count_s": 0.0, "train_s": 0.0, "merge_s": 0.0}
+        self.init_tables(seed)  # identical on every rank (counter-based init)
+        if world > 1:
+            begin = time.perf_counter()
+            self.open_exchange(process_group)
+            self.timings["open_exchange_s"] = time.perf_counter() - begin
+        per_epoch = self.walks_per_epoch
+        lr = np.float32(cfg.learning_rate)
+        losses = []
+        for epoch in range(cfg.epochs):
+            self.reset_counters()
+            begin = time.perf_counter()
+            self.glove_walk_epoch(seed, epoch * per_epoch, per_epoch)
+            mark = time.perf_counter()
+            self.timings["walk_histogram_s"] += mark - begin
+            local_max, _ = self.glove_shard_count(world, rank)
+            x_max = int(all_reduce([local_max], torch.int64, dist.ReduceOp.MAX)[0])
+            begin = time.perf_counter()
+            self.timings["count_s"] += begin - mark
+            self.glove_shard_train(float(lr), x_max)
+            self.sync()
+            mark = time.perf_counter()
+            self.timings["train_s"] += mark - begin
+            if world > 1:
+                self.merge(process_group)
+                self.timings["merge_s"] += time.perf_counter() - mark
+            c = self.counters()
+            stats = all_reduce([c["loss_sum"], float(c["pairs"])], torch.float64, dist.ReduceOp.SUM)
+            losses.append(float(stats[0] / max(float(stats[1]), 1.0)))
+            lr = np.float32(lr * np.float32(cfg.learning_rate_decay))
+        if world > 1:
+            dist.barrier(group=process_group)
+            self.close_exchange()
+        return self._gather_tables(rank, gather, table0, table1, losses)

@@ -146,6 +146,31 @@ int b2e_cooccurrence(b2e_handle *handle, uint64_t seed, uint64_t first_walk, uin
 int b2e_cooccurrence_export(b2e_handle *handle, uint32_t *centre, uint32_t *context, uint32_t *count);
 int b2e_glove_train(b2e_handle *handle, float learning_rate);
 
+/*
+ * GloVe on several GPUs: the centre ids are sharded over the ranks, the tables merged once per
+ * epoch (csrc/exchange.cu; normative statement: oracle.glove_fit_sharded).  Per epoch, on every rank:
+ *   b2e_glove_walk_epoch   walks the whole epoch (ids first_walk .. first_walk + n_walks - 1) into
+ *                          HBM and takes its token histogram; identical on every rank;
+ *   b2e_glove_shard_count  splits [0, n) into `world` intervals of centre id balanced by key slots
+ *                          (owner_bounds, may be NULL, receives world + 1 entries: rank r owns
+ *                          [owner_bounds[r], owner_bounds[r + 1])) and counts this rank's centres,
+ *                          range by range within the sort capacity; *local_max receives their
+ *                          largest count (0 if none);
+ *   b2e_glove_shard_train  one SGD pass over this rank's centres in ascending order, weights against
+ *                          max_count, the largest count of the whole epoch (the maximum of the ranks'
+ *                          local_max); with world > 1 it first snapshots T1 on the device;
+ *   b2e_glove_merge        asynchronous on the train stream, over the peers of b2e_exchange_open*:
+ *                          every replica takes row v of T0 from the owner of v, and T1 becomes
+ *                          snapshot + sum over the ranks of (T1_rank - snapshot); bracketed by
+ *                          barriers like b2e_exchange_average.  Afterwards the replicas are
+ *                          bit-identical.  A no-op with world 1.
+ */
+int b2e_glove_walk_epoch(b2e_handle *handle, uint64_t seed, uint64_t first_walk, uint64_t n_walks);
+int b2e_glove_shard_count(b2e_handle *handle, uint32_t world, uint32_t rank, uint32_t *owner_bounds,
+                          uint32_t *local_max);
+int b2e_glove_shard_train(b2e_handle *handle, float learning_rate, uint32_t max_count);
+int b2e_glove_merge(b2e_handle *handle);
+
 uint64_t b2e_number_of_sources(const b2e_handle *handle);
 uint64_t b2e_row_stride(const b2e_handle *handle); /* floats per table row on the device */
 
