@@ -165,12 +165,6 @@ extern "C" int b2e_create(const b2e_config *config, b2e_handle **out) {
     // rows start on 128 B lines: a random row then touches the fewest lines (measured with
     // scripts/microbench_rows: +13 % rows/s over a dense 400 B pitch for D = 100)
     h->row_stride = (c.embedding_size + 31u) / 32u * 32u;
-    if (const char *env = getenv("B2E_PREFETCH")) h->prefetch = (uint32_t)atoi(env);
-    if (const char *env = getenv("B2E_VARIANT")) h->variant = (uint32_t)atoi(env);
-    if (const char *env = getenv("B2E_WALK_OCC")) h->walk_occupancy = (uint32_t)atoi(env);
-    if (const char *env = getenv("B2E_BULK")) h->bulk = (uint32_t)atoi(env);
-    if (const char *env = getenv("B2E_SGD_OCC")) h->sgd_occupancy = (uint32_t)atoi(env);
-    if (const char *env = getenv("B2E_EXCHANGE_ROWS")) h->exchange_rows = (uint32_t)atoi(env);
     thresholds(c.return_weight, c.explore_weight, h->thr);
     h->second_order = !(c.return_weight == 1.0f && c.explore_weight == 1.0f);
     for (int s = 0; s < 2; ++s) {
@@ -586,7 +580,6 @@ static int walk_into(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t
     const unsigned long long *thr = h->fold_excess && !typed ? h->thr_fold : h->thr;
     p.fold_excess = typed ? 0 : h->fold_excess;
     p.filter = h->d_filter;
-    p.occupancy = h->walk_occupancy;
     p.thr_return = thr[0];
     p.thr_common = thr[1];
     p.thr_explore = thr[2];
@@ -679,12 +672,7 @@ static int train_slot(b2e_handle *h, uint64_t seed, uint32_t slot, float learnin
     p.normalize_lr = c.normalize_learning_rate_by_degree ? 1u : 0u;
     p.downsample = c.stochastic_downsample_by_degree ? h->max_degree + 1u : 0u;
     p.scale_dot = c.scale_by_sqrt_dim ? 1u : 0u;
-    p.prefetch = h->prefetch;
-    p.variant = h->variant;
-    p.bulk = h->bulk;
     p.shared_negatives = c.shared_negatives ? 1u : 0u;
-    p.no_full_rows = getenv("B2E_NO_FULL_ROWS") ? 1u : 0u;
-    p.sgd_occupancy = h->sgd_occupancy;
     p.alias = h->d_alias;
     p.indptr = h->d_indptr;
     p.t0 = h->d_t0;
@@ -896,8 +884,7 @@ extern "C" int b2e_exchange_average(b2e_handle *h) {
     if (int rc = require_graph(h)) return rc;
     if (h->world < 2) return B2E_OK;
     CUDA_TRY(launch_exchange_average(h->peer_t0, h->peer_t1, h->world, h->rank, h->n, h->row_stride,
-                                     (h->cfg.embedding_size + 3u) / 4u, h->sm_count, h->train_stream,
-                                     h->exchange_rows));
+                                     (h->cfg.embedding_size + 3u) / 4u, h->sm_count, h->train_stream));
     ++h->launches;
     return B2E_OK;
 }
@@ -1110,7 +1097,7 @@ extern "C" int b2e_glove_train(b2e_handle *h, float learning_rate) {
                                                        : std::max<uint64_t>(16, h->n / 16);
     CUDA_TRY(b2e::glove_train(h->glove, h->n, h->row_stride, c.embedding_size, c.glove_alpha, c.clipping_value,
                               learning_rate, h->d_t0, h->d_t1, h->d_counters, c.deterministic != 0,
-                              h->sm_count, max_warps, h->variant, h->train_stream));
+                              h->sm_count, max_warps, h->train_stream));
     if (h->glove.n_triples) ++h->launches;
     return B2E_OK;
 }

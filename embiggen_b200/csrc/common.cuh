@@ -67,7 +67,6 @@ struct WalkParams {
     uint32_t undirected;     // every edge has its mirror (verified at load): allows the short-row check
     const unsigned long long *filter;  // per-row blocked Bloom filters over the neighbour lists, or nullptr
     unsigned long long fold_excess;    // E > 0: the return edge is folded out of the envelope (TAG_FOLD)
-    uint32_t occupancy;                // resident CTAs per SM the second-order kernel is compiled for (4, 5, 6)
     int sm_count;
 };
 
@@ -82,12 +81,7 @@ struct TrainParams {
     float clip, lr, inv_scale;
     uint32_t use_alias, normalize_lr, scale_dot;
     uint32_t downsample;  // stochastic_downsample_by_degree: max degree + 1, 0 = off
-    uint32_t prefetch;  // 1: L2-prefetch the rows of the next draw site
-    uint32_t variant;   // tuning variant of the launch (0 = default)
-    uint32_t sgd_occupancy;  // CTAs per SM of the SkipGram kernel (0: by table size, see launch_train_pipe)
-    uint32_t no_full_rows;  // B2E_NO_FULL_ROWS: keep the generic CBOW kernel for 32-chunk rows (A/B)
     uint32_t shared_negatives;  // SkipGram: one set of negatives per centre (skipgram_shared_kernel)
-    uint32_t bulk;      // SkipGram rows by cp.async.bulk + mbarrier instead of per-lane cp.async (experiment)
     const uint2 *alias;  // {threshold, alias} per node
     const int64_t *indptr;
     float *t0, *t1;
@@ -129,8 +123,7 @@ cudaError_t glove_accumulate(GloveState &g, const uint32_t *d_walks, uint64_t n_
 cudaError_t glove_finalise(GloveState &g, uint64_t n, cudaStream_t stream);
 cudaError_t glove_train(const GloveState &g, uint64_t n, uint32_t row_stride, uint32_t embedding_size,
                         float alpha, float clip, float lr, float *t0, float *t1, DeviceCounters *counters,
-                        bool deterministic, int sm_count, uint64_t max_warps, uint32_t variant,
-                        cudaStream_t stream);
+                        bool deterministic, int sm_count, uint64_t max_warps, cudaStream_t stream);
 // co-occurrence by centre range (glove.cu): histogram of the epoch's tokens, occurrences bucketed
 // by range, the triples of one range
 cudaError_t glove_token_histogram(const uint32_t *d_walks, uint64_t tokens, uint32_t *d_histogram, uint64_t n,
@@ -161,7 +154,7 @@ cudaError_t launch_row_filter_build(const int64_t *indptr, const uint32_t *indic
                                     unsigned long long *filter, int sm_count, cudaStream_t stream);
 cudaError_t launch_exchange_average(float *const t0[], float *const t1[], uint32_t world, uint32_t rank,
                                     uint64_t n, uint32_t row_stride, uint32_t chunks, int sm_count,
-                                    cudaStream_t stream, uint32_t rows_per_iteration = 0);
+                                    cudaStream_t stream);
 // GloVe's merge of a sharded epoch: every replica takes row v of T0 from the replica of its owner
 // and T1 = snapshot + sum over the ranks of (T1_g - snapshot); this rank reduces the rows
 // [n rank / world, n (rank + 1) / world)
@@ -234,12 +227,6 @@ struct b2e_handle {
     unsigned long long thr[3] = {0, 0, 0};
     bool second_order = false;
     bool undirected = false;
-    uint32_t prefetch = 1;
-    uint32_t variant = 0;
-    uint32_t sgd_occupancy = 0;  // B2E_SGD_OCC (0: automatic)
-    uint32_t bulk = 0;  // B2E_BULK
-    uint32_t exchange_rows = 0;  // B2E_EXCHANGE_ROWS (0: the default of launch_exchange_average)
-    uint32_t walk_occupancy = 6;  // B2E_WALK_OCC: see walk_kernel
     uint64_t launches = 0;
     std::vector<uint32_t> h_alias_thr, h_alias_idx;
     // the exchange step: replicas of the tables on the other GPUs of the node

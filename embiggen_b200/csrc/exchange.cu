@@ -80,7 +80,7 @@ __global__ void __launch_bounds__(256) exchange_average_kernel(const ExchangePar
 
 cudaError_t launch_exchange_average(float *const t0[], float *const t1[], uint32_t world, uint32_t rank,
                                     uint64_t n, uint32_t row_stride, uint32_t chunks, int sm_count,
-                                    cudaStream_t stream, uint32_t rows_per_iteration) {
+                                    cudaStream_t stream) {
     if (world < 2 || n == 0) return cudaSuccess;
     ExchangeParams p;
     for (uint32_t g = 0; g < world; ++g) {
@@ -96,24 +96,12 @@ cudaError_t launch_exchange_average(float *const t0[], float *const t1[], uint32
     const uint64_t rows = p.row_end - p.row_begin;
     if (rows == 0) return cudaSuccess;
     const unsigned grid = (unsigned)std::min<uint64_t>((2 * rows + 7) / 8, (uint64_t)sm_count * 8);
-    // rows per warp iteration: enough loads in flight per lane to cover an NVLink round trip
-    // (B2E_EXCHANGE_ROWS overrides the default for tuning)
-    const uint32_t u = rows_per_iteration;
+    // rows per warp iteration: enough loads in flight per lane to cover an NVLink round trip, the
+    // G x U loads of a lane held to eight float4
     switch (world) {
-        case 2:
-            if (u == 1) exchange_average_kernel<2, 1><<<grid, 256, 0, stream>>>(p);
-            else if (u == 8) exchange_average_kernel<2, 8><<<grid, 256, 0, stream>>>(p);
-            else exchange_average_kernel<2, 4><<<grid, 256, 0, stream>>>(p);
-            break;
-        case 4:
-            if (u == 1) exchange_average_kernel<4, 1><<<grid, 256, 0, stream>>>(p);
-            else if (u == 4) exchange_average_kernel<4, 4><<<grid, 256, 0, stream>>>(p);
-            else exchange_average_kernel<4, 2><<<grid, 256, 0, stream>>>(p);
-            break;
-        case 8:
-            if (u == 2) exchange_average_kernel<8, 2><<<grid, 256, 0, stream>>>(p);
-            else exchange_average_kernel<8, 1><<<grid, 256, 0, stream>>>(p);
-            break;
+        case 2: exchange_average_kernel<2, 4><<<grid, 256, 0, stream>>>(p); break;
+        case 4: exchange_average_kernel<4, 2><<<grid, 256, 0, stream>>>(p); break;
+        case 8: exchange_average_kernel<8, 1><<<grid, 256, 0, stream>>>(p); break;
         default: exchange_average_kernel<0, 1><<<grid, 256, 0, stream>>>(p); break;
     }
     return cudaGetLastError();

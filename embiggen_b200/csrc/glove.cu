@@ -400,8 +400,7 @@ cudaError_t glove_finalise(GloveState &g, uint64_t n, cudaStream_t stream) {
 
 cudaError_t glove_train(const GloveState &g, uint64_t n, uint32_t row_stride, uint32_t embedding_size,
                         float alpha, float clip, float lr, float *t0, float *t1, DeviceCounters *counters,
-                        bool deterministic, int sm_count, uint64_t max_warps, uint32_t variant,
-                        cudaStream_t stream) {
+                        bool deterministic, int sm_count, uint64_t max_warps, cudaStream_t stream) {
     if (g.n_triples == 0) return cudaSuccess;
     GloveParams p;
     p.keys = g.d_keys;
@@ -418,9 +417,7 @@ cudaError_t glove_train(const GloveState &g, uint64_t n, uint32_t row_stride, ui
     p.t1 = t1;
     p.counters = counters;
     // 4 rows per batch: 64 registers, 4 CTAs per SM -- 6.0 G triples/s against 3.8 G with 8 rows
-    // (95 registers, 2 CTAs per SM) on R-MAT 1 M / 16 M; B2E_VARIANT=1 keeps the larger batch
-    if (p.chunks <= 32 && variant == 1 && !deterministic)
-        return launch_glove_one<1, 8>(p, g.n_triples, deterministic, sm_count, max_warps, stream);
+    // (95 registers, 2 CTAs per SM) on R-MAT 1 M / 16 M
     if (p.chunks <= 32) return launch_glove_one<1, 4>(p, g.n_triples, deterministic, sm_count, max_warps, stream);
     if (p.chunks <= 64) return launch_glove_one<2, 4>(p, g.n_triples, deterministic, sm_count, max_warps, stream);
     if (p.chunks <= 128) return launch_glove_one<4, 2>(p, g.n_triples, deterministic, sm_count, max_warps, stream);

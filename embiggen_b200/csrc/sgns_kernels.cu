@@ -64,7 +64,6 @@ __device__ __forceinline__ uint32_t draw_resolve(const TrainParams &p, const Dra
 // of T1, slots 1..K = the valid negatives (T1), slot K+1 = row `extra` of T0 (PAD: none).
 __device__ __forceinline__ void prefetch_site(const TrainParams &p, uint32_t lane, uint32_t first,
                                               uint32_t neg, uint32_t vmask, uint32_t extra) {
-    if (p.prefetch == 0) return;
     const uint32_t row_bytes = p.chunks * 16u;
     const uint32_t slots = p.negatives + 2u;
     for (uint32_t first_t = 0; first_t < slots * 5u; first_t += 32u) {  // warp-uniform trip count
@@ -340,14 +339,6 @@ static cudaError_t launch_model(const TrainParams &p, bool deterministic, int sm
                                 uint64_t max_warps, cudaStream_t stream) {
     const uint32_t chunks = p.chunks;
     if (chunks <= 32) {
-        // tuning variants (rows per load batch x resident CTAs per SM), B2E_VARIANT selects
-        switch (p.variant) {
-            case 1: return launch_one<MODEL, 1, 11, 2>(p, deterministic, sm_count, max_warps, stream);
-            case 2: return launch_one<MODEL, 1, 6, 3>(p, deterministic, sm_count, max_warps, stream);
-            case 3: return launch_one<MODEL, 1, 6, 4>(p, deterministic, sm_count, max_warps, stream);
-            case 4: return launch_one<MODEL, 1, 4, 4>(p, deterministic, sm_count, max_warps, stream);
-            default: break;
-        }
         if (p.negatives + 1 <= 6) return launch_one<MODEL, 1, 6, 3>(p, deterministic, sm_count, max_warps, stream);
         return launch_one<MODEL, 1, 11, 2>(p, deterministic, sm_count, max_warps, stream);
     }
@@ -359,10 +350,10 @@ static cudaError_t launch_model(const TrainParams &p, bool deterministic, int sm
 cudaError_t launch_train(const TrainParams &p, uint32_t model, bool deterministic, int sm_count,
                          uint64_t max_warps, cudaStream_t stream) {
     if (p.n_walks == 0) return cudaSuccess;
-    // production path: shared-memory pipelined kernel; B2E_VARIANT >= 1 keeps the register path
+    // production path: shared-memory pipelined kernel; the register path takes the other shapes
     if (model == B2E_SKIPGRAM && p.shared_negatives)  // one kernel, no register-staged twin
         return launch_train_pipe(p, model, deterministic, sm_count, max_warps, stream);
-    if (p.variant == 0 && pipe_supported(p, model))
+    if (pipe_supported(p, model))
         return launch_train_pipe(p, model, deterministic, sm_count, max_warps, stream);
     if (model == B2E_SKIPGRAM) return launch_model<B2E_SKIPGRAM>(p, deterministic, sm_count, max_warps, stream);
     return launch_model<B2E_CBOW>(p, deterministic, sm_count, max_warps, stream);

@@ -43,37 +43,6 @@ __device__ __forceinline__ void cp_async8(void *smem, const void *gmem) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
-// ---- bulk-copy variant (B2E_BULK=1): one cp.async.bulk (UBLKCP) per row, issued by lane 0 and
-// completed on a per-warp, per-stage mbarrier, instead of one 16 B LDGSTS per lane and row ----
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(a), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(a), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    const uint32_t a = (uint32_t)__cvta_generic_to_shared(bar);
-    asm volatile(
-        "{\n\t"
-        ".reg .pred P1;\n\t"
-        "B2E_WAIT:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1, 0x989680;\n\t"
-        "@P1 bra B2E_DONE;\n\t"
-        "bra B2E_WAIT;\n\t"
-        "B2E_DONE:\n\t"
-        "}" ::"r"(a), "r"(parity)
-        : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(void *smem, const void *gmem, uint32_t bytes, uint64_t *bar) {
-    const uint32_t d = (uint32_t)__cvta_generic_to_shared(smem), b = (uint32_t)__cvta_generic_to_shared(bar);
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(d),
-                 "l"(gmem), "r"(bytes), "r"(b)
-                 : "memory");
-}
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 __device__ __forceinline__ float4 lds128(const float *smem) {
     return *reinterpret_cast<const float4 *>(smem);
 }
@@ -176,33 +145,6 @@ __device__ __forceinline__ void issue_rows(const TrainParams &p, const PipeSmem 
         cp_async16(dst + slots * sm.pitch, v.row0(centre_or_pad));
 }
 
-// the same copies as issue_rows, as bulk copies: every lane orders its earlier generic-proxy
-// accesses (stores to the rows, reads of the stage) before the async proxy, lane 0 arms the
-// stage's mbarrier with the byte count and issues one bulk copy per row
-template <int KP1>
-__device__ __forceinline__ void issue_rows_bulk(const TrainParams &p, const PipeSmem &sm, uint32_t stage,
-                                                uint32_t lane, uint32_t my_id, uint32_t vmask,
-                                                uint32_t centre_or_pad, uint64_t *bar) {
-    if (lane < PIPE_SLOTS) sm.ids(stage)[lane] = my_id;
-    fence_proxy_async();
-    __syncwarp();
-    if (lane == 0) {
-        const uint32_t slots = KP1 ? (uint32_t)KP1 : p.negatives + 1u;
-        const uint32_t row = p.chunks * 16u;
-        const uint32_t on = vmask & ((1u << slots) - 1u);
-        mbar_expect_tx(bar, (__popc(on) + (centre_or_pad != PAD ? 1u : 0u)) * row);
-        float *dst = sm.rows(stage);
-        const uint32_t *ids = sm.ids(stage);
-        constexpr int S = KP1 ? KP1 : PIPE_SLOTS;
-#pragma unroll
-        for (int s = 0; s < S; ++s)
-            if ((uint32_t)s < slots && ((on >> s) & 1u))
-                bulk_copy_g2s(dst + (uint32_t)s * sm.pitch, p.t1 + (uint64_t)ids[s] * p.row_stride, row, bar);
-        if (centre_or_pad != PAD)
-            bulk_copy_g2s(dst + slots * sm.pitch, p.t0 + (uint64_t)centre_or_pad * p.row_stride, row, bar);
-    }
-}
-
 // dots, sigmoid, axpy and scatter of the targets of one draw site out of stage `stage`;
 // returns this lane's chunk of sum g * row (rows as they were before the update)
 // SHARED: every slot is a negative that stands for `weight` pairs (skipgram_shared_kernel)
@@ -280,9 +222,9 @@ __device__ __forceinline__ void add4(float4 &a, const float4 &b) {
     a.w = __fadd_rn(a.w, b.w);
 }
 
-// MINB: CTAs per SM the register allocation is held to (4: 121 registers; 5: 96 registers and
-// 32 bytes of spills, 20 instead of 16 warps per SM keep more row copies in flight)
-template <int KP1, bool BULK = false, int MINB = 4>
+// MINB: CTAs per SM the register allocation is held to (4: 121 registers; 3 for tables of 32 GiB
+// and more, see launch_train_pipe)
+template <int KP1, int MINB = 4>
 __global__ void __launch_bounds__(128, MINB) skipgram_pipe_kernel(const TrainParams p) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
@@ -290,19 +232,8 @@ __global__ void __launch_bounds__(128, MINB) skipgram_pipe_kernel(const TrainPar
     const uint32_t L = p.walk_length, W = p.window;
     const uint32_t full_mask = (2u << K) - 1u;  // K + 1 ones
     PipeSmem sm;
-    uint64_t *bars = nullptr;  // BULK: one mbarrier per stage, behind the warp's slab
-    uint32_t parity = 0u;      // bit s: phase of stage s's barrier
     {
-        unsigned char *base = smem_raw + warp * (pipe_warp_bytes(K, p.chunks, L) + (BULK ? 16u : 0u));
-        if (BULK) {
-            bars = reinterpret_cast<uint64_t *>(base + pipe_warp_bytes(K, p.chunks, L));
-            if (lane == 0) {
-                mbar_init(bars, 1);
-                mbar_init(bars + 1, 1);
-                asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-            }
-            __syncwarp();
-        }
+        unsigned char *base = smem_raw + warp * pipe_warp_bytes(K, p.chunks, L);
         sm.pitch = p.chunks * 4u;
         sm.stage_floats = (K + 2u) * sm.pitch;
         sm.rows_base = reinterpret_cast<float *>(base);
@@ -361,8 +292,7 @@ __global__ void __launch_bounds__(128, MINB) skipgram_pipe_kernel(const TrainPar
             return (__ballot_sync(FULL, valid) << 1) | 1u;
         };
         auto issue = [&](uint32_t stage, uint32_t ids, uint32_t vmask, uint32_t centre_or_pad) {
-            if (BULK) issue_rows_bulk<KP1>(p, sm, stage, lane, ids, vmask, centre_or_pad, bars + stage);
-            else if (vmask == full_mask) issue_rows<KP1, true>(p, sm, v, stage, lane, ids, vmask, centre_or_pad);
+            if (vmask == full_mask) issue_rows<KP1, true>(p, sm, v, stage, lane, ids, vmask, centre_or_pad);
             else issue_rows<KP1, false>(p, sm, v, stage, lane, ids, vmask, centre_or_pad);
         };
 
@@ -392,10 +322,6 @@ __global__ void __launch_bounds__(128, MINB) skipgram_pipe_kernel(const TrainPar
         float lr = p.lr;
         while (ok_cur) {
             cp_async_wait_all();  // rows of `cur` (this stage) and alias entries of `nxt` are here
-            if (BULK) {           // ... the rows through the stage's mbarrier
-                mbar_wait(bars + stage, (parity >> stage) & 1u);
-                parity ^= 1u << stage;
-            }
             // Memory ordering between lanes: the copies above were waited for by the lane that
             // issued them, and the ids / alias slots of the other stage were last read in the
             // previous iteration.  The warp is converged here anyway (ballot / match follow); the
@@ -1076,29 +1002,23 @@ cudaError_t launch_train_pipe(const TrainParams &p, uint32_t model, bool determi
         const size_t ring = (size_t)cbow_ring_slots(p.window) * p.chunks * 16u - 2u * p.chunks * 16u;
         switch (p.negatives) {
             case 10:
-                // four CTAs per SM (128 registers, 54.6 KB each) unless B2E_SGD_OCC=3: the kernel is bound by
-                // the dependency chain of a warp, not by HBM -- C3 2.61 G against 2.20 G pairs/s, C5 2.51 G
-                // (profiles/r02x_*)
-                if (p.sgd_occupancy != 3 && !deterministic)
+                // four CTAs per SM (128 registers, 54.6 KB each) rather than three: the kernel is bound
+                // by the dependency chain of a warp, not by HBM -- C3 2.61 G against 2.20 G pairs/s, C5
+                // 2.51 G (profiles/r02x_*)
+                if (!deterministic)
                     return launch_pipe(skipgram_shared_kernel<10, 4>, p, deterministic, sm_count, max_warps, stream, ring);
                 return launch_pipe(skipgram_shared_kernel<10>, p, deterministic, sm_count, max_warps, stream, ring);
             case 5: return launch_pipe(skipgram_shared_kernel<5>, p, deterministic, sm_count, max_warps, stream, ring);
             default: return launch_pipe(skipgram_shared_kernel<0>, p, deterministic, sm_count, max_warps, stream, ring);
         }
     }
-    if (model == B2E_SKIPGRAM && p.bulk && p.negatives + 1u == 11u)  // B2E_BULK=1: the UBLKCP experiment
-        return launch_pipe(skipgram_pipe_kernel<11, true>, p, deterministic, sm_count, max_warps, stream, 16);
-    // CTAs per SM of the SkipGram kernel (B2E_SGD_OCC overrides).  Measured in pairs/s at 5 / 4 / 3 / 2:
-    // C2 543 / 605 / 596 / -, C3 537 / 587 / 583 / -, C5 473 / 503 / 516 / 460 M (profiles/r02p_*):
-    // four while the tables are a few GB, three once random rows spread over tens of GB (fewer
-    // streams keep more DRAM pages open); the switch-over is put at 32 GiB of tables.
-    uint32_t occupancy = p.sgd_occupancy;
-    if (occupancy == 0) occupancy = 2ull * p.n * p.row_stride * sizeof(float) >= (32ull << 30) ? 3u : 4u;
-    if (model == B2E_SKIPGRAM && occupancy == 5 && p.negatives + 1u == 11u && !deterministic)
-        return launch_pipe(skipgram_pipe_kernel<11, false, 5>, p, deterministic, sm_count, max_warps, stream);
-    if (model == B2E_SKIPGRAM && (occupancy == 3 || occupancy == 2) && p.negatives + 1u == 11u && !deterministic)
-        return launch_pipe(skipgram_pipe_kernel<11, false, 3>, p, deterministic, sm_count, max_warps, stream, 0,
-                           (int)occupancy);
+    // CTAs per SM of the SkipGram kernel, measured in pairs/s at 5 / 4 / 3 / 2 with a switch since
+    // removed: C2 543 / 605 / 596 / -, C3 537 / 587 / 583 / -, C5 473 / 503 / 516 / 460 M
+    // (profiles/r02p_*): four while the tables are a few GB, three once random rows spread over
+    // tens of GB (fewer streams keep more DRAM pages open); the switch-over is put at 32 GiB of tables.
+    const bool large_tables = 2ull * p.n * p.row_stride * sizeof(float) >= (32ull << 30);
+    if (model == B2E_SKIPGRAM && large_tables && p.negatives + 1u == 11u && !deterministic)
+        return launch_pipe(skipgram_pipe_kernel<11, 3>, p, deterministic, sm_count, max_warps, stream, 0, 3);
     if (model == B2E_SKIPGRAM) {
         switch (p.negatives + 1u) {
             case 11: return launch_pipe(skipgram_pipe_kernel<11>, p, deterministic, sm_count, max_warps, stream);
@@ -1107,7 +1027,7 @@ cudaError_t launch_train_pipe(const TrainParams &p, uint32_t model, bool determi
         }
     }
     const size_t ring = (size_t)cbow_ring_slots(p.window) * p.chunks * 16u;
-    if (p.chunks == 32u && p.negatives + 1u == 11u && !p.no_full_rows)
+    if (p.chunks == 32u && p.negatives + 1u == 11u)
         return launch_pipe(cbow_pipe_kernel<11, true>, p, deterministic, sm_count, max_warps, stream, ring);
     switch (p.negatives + 1u) {
         case 11: return launch_pipe(cbow_pipe_kernel<11>, p, deterministic, sm_count, max_warps, stream, ring);

@@ -189,8 +189,9 @@ __device__ __forceinline__ uint32_t propose(const uint2 *__restrict__ table, int
 // one Philox block per trial (tag 12): x decides slot vs row, y proposes, z accepts; see
 // oracle/walks.c (orc_fold_thresholds) for the normative statement.
 // MINB: resident CTAs per SM the register allocation is held to (4: 64 registers, no spills;
-// 6: 40 registers and a few spilled words -- more chains in flight per SM; measured on C3:
-// 7.8 / 8.6 / 9.4 G steps/s at 4 / 5 / 6, profiles/r02c_*)
+// 6: 40 registers and a few spilled words -- more chains in flight per SM).  The vectorised
+// second-order unweighted walks use 6: on C3 they ran at 7.8 / 8.6 / 9.4 G steps/s at 4 / 5 / 6
+// and 9.3 at 8 (profiles/r02c_*, r02d_bench_c3_occ8, measured with a switch since removed).
 template <bool SECOND, bool VEC, bool WEIGHTED, bool FOLD, int MINB = 4>
 __global__ void __launch_bounds__(256, MINB) walk_kernel(const WalkParams p) {
     const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -508,22 +509,13 @@ cudaError_t launch_walks(const WalkParams &p, bool second_order, cudaStream_t st
                else walk_general_kernel<false, false><<<grid, block, 0, stream>>>(p); }
         return cudaGetLastError();
     }
-#define B2E_LAUNCH_WALK(S, V, W, F) walk_kernel<S, V, W, F><<<grid, block, 0, stream>>>(p)
-    if (second_order && !weighted && vec && p.occupancy >= 5) {  // the headline shapes, tunable occupancy
-        if (p.fold_excess) {
-            if (p.occupancy == 5) walk_kernel<true, true, false, true, 5><<<grid, block, 0, stream>>>(p);
-            else if (p.occupancy >= 8) walk_kernel<true, true, false, true, 8><<<grid, block, 0, stream>>>(p);
-            else walk_kernel<true, true, false, true, 6><<<grid, block, 0, stream>>>(p);
-        } else {
-            if (p.occupancy == 5) walk_kernel<true, true, false, false, 5><<<grid, block, 0, stream>>>(p);
-            else if (p.occupancy >= 8) walk_kernel<true, true, false, false, 8><<<grid, block, 0, stream>>>(p);
-            else walk_kernel<true, true, false, false, 6><<<grid, block, 0, stream>>>(p);
-        }
-    } else if (second_order && !weighted && p.fold_excess) {
-        if (vec) B2E_LAUNCH_WALK(true, true, false, true); else B2E_LAUNCH_WALK(true, false, false, true);
+#define B2E_LAUNCH_WALK(...) walk_kernel<__VA_ARGS__><<<grid, block, 0, stream>>>(p)
+    if (second_order && !weighted && vec) {  // the headline shapes, six CTAs per SM
+        if (p.fold_excess) B2E_LAUNCH_WALK(true, true, false, true, 6); else B2E_LAUNCH_WALK(true, true, false, false, 6);
+    } else if (second_order && !weighted) {
+        if (p.fold_excess) B2E_LAUNCH_WALK(true, false, false, true); else B2E_LAUNCH_WALK(true, false, false, false);
     } else if (second_order) {
-        if (vec) { if (weighted) B2E_LAUNCH_WALK(true, true, true, false); else B2E_LAUNCH_WALK(true, true, false, false); }
-        else { if (weighted) B2E_LAUNCH_WALK(true, false, true, false); else B2E_LAUNCH_WALK(true, false, false, false); }
+        if (vec) B2E_LAUNCH_WALK(true, true, true, false); else B2E_LAUNCH_WALK(true, false, true, false);
     } else {
         if (vec) { if (weighted) B2E_LAUNCH_WALK(false, true, true, false); else B2E_LAUNCH_WALK(false, true, false, false); }
         else { if (weighted) B2E_LAUNCH_WALK(false, false, true, false); else B2E_LAUNCH_WALK(false, false, false, false); }

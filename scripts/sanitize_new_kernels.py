@@ -59,13 +59,6 @@ with Engine("GloVe", embedding_size=100, walk_length=33, window_size=4, iteratio
     engine.load_csr(graph.indptr, graph.indices)
     t0, t1, losses = engine.fit(7)
     assert np.isfinite(t0).all() and np.isfinite(t1).all()
-os.environ["B2E_BULK"] = "1"  # the cp.async.bulk + mbarrier variant of the SkipGram kernel
-with Engine("SkipGram", embedding_size=100, walk_length=40, window_size=4, iterations=1, epochs=1,
-            return_weight=2.0, explore_weight=0.5) as engine:
-    engine.load_csr(hub.indptr, hub.indices)
-    t0, t1, losses = engine.fit(7)
-    assert np.isfinite(t0).all() and np.isfinite(t1).all()
-del os.environ["B2E_BULK"]
 with Engine("CBOW", embedding_size=128, walk_length=40, window_size=4, iterations=1, epochs=1) as engine:  # full rows
     engine.load_csr(hub.indptr, hub.indices)
     t0, t1, losses = engine.fit(7)

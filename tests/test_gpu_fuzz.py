@@ -32,6 +32,9 @@ def cases():
             normalize=bool(rng.integers(0, 2)),
             seed=int(rng.integers(0, 2 ** 62)),
         ))
+    # walks longer than the pipelined kernels stage (1024 tokens) take the generic SkipGram kernel
+    out.append(dict(graph="small_ppi", model="SkipGram", D=100, K=5, w=3, L=1040, rw=0.25, ew=4.0, lr=0.025,
+                    alias=True, scale=False, normalize=False, seed=20261021))
     return out
 
 
