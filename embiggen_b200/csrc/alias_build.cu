@@ -19,29 +19,9 @@
 #include <cmath>
 #include <string>
 
-#include "common.cuh"
+#include "host.cuh"
 
 namespace b2e {
-
-struct DeviceScratch {
-    void *ptr = nullptr;
-    ~DeviceScratch() { cudaFree(ptr); }
-    cudaError_t get(size_t bytes) {
-        cudaFree(ptr);
-        ptr = nullptr;
-        return cudaMalloc(&ptr, bytes ? bytes : 1);
-    }
-    template <typename T> T *as() { return static_cast<T *>(ptr); }
-};
-
-#define AB_TRY(expr)                                                     \
-    do {                                                                 \
-        cudaError_t _e = (expr);                                         \
-        if (_e != cudaSuccess) {                                         \
-            error = std::string(#expr) + ": " + cudaGetErrorString(_e);  \
-            return _e;                                                   \
-        }                                                                \
-    } while (0)
 
 __device__ __forceinline__ double degree_weight_device(unsigned long long deg, int form) {
     const double d = (double)deg;
@@ -207,37 +187,39 @@ cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indpt
                               uint32_t *d_sources, uint64_t *n_src_out, uint64_t *max_degree_out, uint2 *d_table,
                               cudaStream_t stream, std::string &error) {
     typedef unsigned long long u64;
-    DeviceScratch weight, has_edges, rank, degree, temp, scalar, given;
-    AB_TRY(has_edges.get(n * sizeof(uint32_t)));
-    AB_TRY(rank.get(n * sizeof(uint32_t)));
-    AB_TRY(degree.get(n * sizeof(u64)));
-    AB_TRY(scalar.get(2 * sizeof(u64)));
+    DeviceBuffer<u64> weight, degree, scalar, given;
+    DeviceBuffer<uint32_t> has_edges, rank;
+    DeviceBuffer<> temp;
+    CUDA_CHECK(has_edges.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(rank.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(degree.reserve(n * sizeof(u64)));
+    CUDA_CHECK(scalar.reserve(2 * sizeof(u64)));
     size_t bytes = 0, need = 0;
     // pass 1: degrees, flags; the largest degree fixes the fixed-point format
-    alias_weight_kernel<<<grid_for(n), 256, 0, stream>>>(d_indptr, n, 0, 0, nullptr, nullptr, has_edges.as<uint32_t>(),
-                                                         degree.as<u64>());
-    AB_TRY(cudaGetLastError());
-    AB_TRY(cub::DeviceReduce::Max(nullptr, bytes, degree.as<u64>(), scalar.as<u64>(), n, stream));
+    alias_weight_kernel<<<grid_for(n), 256, 0, stream>>>(d_indptr, n, 0, 0, nullptr, nullptr, has_edges.get(),
+                                                         degree.get());
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cub::DeviceReduce::Max(nullptr, bytes, degree.get(), scalar.get(), n, stream));
     need = bytes;
-    AB_TRY(cub::DeviceScan::ExclusiveSum(nullptr, bytes, has_edges.as<uint32_t>(), rank.as<uint32_t>(), n, stream));
+    CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, bytes, has_edges.get(), rank.get(), n, stream));
     need = std::max(need, bytes);
-    AB_TRY(cub::DeviceScan::InclusiveSum(nullptr, bytes, degree.as<u64>(), degree.as<u64>(), n, stream));
+    CUDA_CHECK(cub::DeviceScan::InclusiveSum(nullptr, bytes, degree.get(), degree.get(), n, stream));
     need = std::max(need, bytes);
-    AB_TRY(cub::DeviceReduce::Sum(nullptr, bytes, degree.as<u64>(), scalar.as<u64>(), n, stream));
+    CUDA_CHECK(cub::DeviceReduce::Sum(nullptr, bytes, degree.get(), scalar.get(), n, stream));
     need = std::max(need, bytes);
-    AB_TRY(temp.get(need));
+    CUDA_CHECK(temp.reserve(std::max<size_t>(need, 1)));
     bytes = need;
-    AB_TRY(cub::DeviceReduce::Max(temp.ptr, bytes, degree.as<u64>(), scalar.as<u64>(), n, stream));
+    CUDA_CHECK(cub::DeviceReduce::Max(temp.get(), bytes, degree.get(), scalar.get(), n, stream));
     bytes = need;
-    AB_TRY(cub::DeviceScan::ExclusiveSum(temp.ptr, bytes, has_edges.as<uint32_t>(), rank.as<uint32_t>(), n, stream));
-    sources_kernel<<<grid_for(n), 256, 0, stream>>>(has_edges.as<uint32_t>(), rank.as<uint32_t>(), n, d_sources);
-    AB_TRY(cudaGetLastError());
+    CUDA_CHECK(cub::DeviceScan::ExclusiveSum(temp.get(), bytes, has_edges.get(), rank.get(), n, stream));
+    sources_kernel<<<grid_for(n), 256, 0, stream>>>(has_edges.get(), rank.get(), n, d_sources);
+    CUDA_CHECK(cudaGetLastError());
     u64 max_degree = 0;
     uint32_t last_rank = 0, last_flag = 0;
-    AB_TRY(cudaMemcpyAsync(&max_degree, scalar.ptr, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaMemcpyAsync(&last_rank, rank.as<uint32_t>() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaMemcpyAsync(&last_flag, has_edges.as<uint32_t>() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaMemcpyAsync(&max_degree, scalar.get(), sizeof(u64), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaMemcpyAsync(&last_rank, rank.get() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaMemcpyAsync(&last_flag, has_edges.get() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     const uint64_t n_src = (uint64_t)last_rank + last_flag;
     *n_src_out = n_src;
     *max_degree_out = max_degree;
@@ -250,7 +232,7 @@ cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indpt
     // pass 2: fixed-point weights and their total
     const int bits = alias_fraction_bits(n, max_degree, alpha);
     const int form = exact_form(alpha);
-    AB_TRY(weight.get(n * sizeof(u64)));
+    CUDA_CHECK(weight.reserve(n * sizeof(u64)));
     if (form < 0) {  // libm's pow on the host, like the oracle; one upload of 8 bytes per node
         if (!host_indptr) {
             error = "a negative_sampling_exponent other than 0, 0.5, 0.75, 1 needs the offsets on the host";
@@ -259,19 +241,19 @@ cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indpt
         std::vector<u64> host(n);
         for (uint64_t v = 0; v < n; ++v)
             host[v] = (u64)std::floor(std::ldexp(degree_weight_host((uint64_t)(host_indptr[v + 1] - host_indptr[v]), alpha), bits));
-        AB_TRY(given.get(n * sizeof(u64)));
-        AB_TRY(cudaMemcpyAsync(given.ptr, host.data(), n * sizeof(u64), cudaMemcpyHostToDevice, stream));
-        AB_TRY(cudaStreamSynchronize(stream));
+        CUDA_CHECK(given.reserve(n * sizeof(u64)));
+        CUDA_CHECK(cudaMemcpyAsync(given.get(), host.data(), n * sizeof(u64), cudaMemcpyHostToDevice, stream));
+        CUDA_CHECK(cudaStreamSynchronize(stream));
     }
     alias_weight_kernel<<<grid_for(n), 256, 0, stream>>>(d_indptr, n, form < 0 ? 0 : form, bits,
-                                                         form < 0 ? given.as<u64>() : nullptr, weight.as<u64>(),
-                                                         has_edges.as<uint32_t>(), degree.as<u64>());
-    AB_TRY(cudaGetLastError());
+                                                         form < 0 ? given.get() : nullptr, weight.get(),
+                                                         has_edges.get(), degree.get());
+    CUDA_CHECK(cudaGetLastError());
     bytes = need;
-    AB_TRY(cub::DeviceReduce::Sum(temp.ptr, bytes, weight.as<u64>(), scalar.as<u64>(), n, stream));
+    CUDA_CHECK(cub::DeviceReduce::Sum(temp.get(), bytes, weight.get(), scalar.get(), n, stream));
     u64 total = 0;
-    AB_TRY(cudaMemcpyAsync(&total, scalar.ptr, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaMemcpyAsync(&total, scalar.get(), sizeof(u64), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     if (total == 0) {
         error = "alias table: total weight is zero";
         return cudaErrorInvalidValue;
@@ -280,49 +262,50 @@ cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indpt
     const u64 excess = capacity * n - total, each = excess / n_src, first = excess % n_src;
 
     // pass 3: masses, classes, the two node lists with their deficits / surpluses
-    DeviceScratch is_light, light_rank, light, heavy, deficit, surplus;
-    AB_TRY(is_light.get(n * sizeof(uint32_t)));
-    AB_TRY(light_rank.get(n * sizeof(uint32_t)));
-    alias_mass_kernel<<<grid_for(n), 256, 0, stream>>>(weight.as<u64>(), has_edges.as<uint32_t>(), rank.as<uint32_t>(), n,
-                                                       each, first, capacity, is_light.as<uint32_t>());
-    AB_TRY(cudaGetLastError());
+    DeviceBuffer<uint32_t> is_light, light_rank, light, heavy;
+    DeviceBuffer<u64> deficit, surplus;
+    CUDA_CHECK(is_light.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(light_rank.reserve(n * sizeof(uint32_t)));
+    alias_mass_kernel<<<grid_for(n), 256, 0, stream>>>(weight.get(), has_edges.get(), rank.get(), n,
+                                                       each, first, capacity, is_light.get());
+    CUDA_CHECK(cudaGetLastError());
     bytes = need;
-    AB_TRY(cub::DeviceScan::ExclusiveSum(temp.ptr, bytes, is_light.as<uint32_t>(), light_rank.as<uint32_t>(), n, stream));
+    CUDA_CHECK(cub::DeviceScan::ExclusiveSum(temp.get(), bytes, is_light.get(), light_rank.get(), n, stream));
     uint32_t tail_rank = 0, tail_flag = 0;
-    AB_TRY(cudaMemcpyAsync(&tail_rank, light_rank.as<uint32_t>() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaMemcpyAsync(&tail_flag, is_light.as<uint32_t>() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    AB_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaMemcpyAsync(&tail_rank, light_rank.get() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaMemcpyAsync(&tail_flag, is_light.get() + (n - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     const uint64_t n_light = (uint64_t)tail_rank + tail_flag, n_heavy = n - n_light;
     if (n_heavy == 0) {  // impossible: the masses add up to n capacities
         error = "alias table: no heavy node";
         return cudaErrorInvalidValue;
     }
-    AB_TRY(light.get(n_light * sizeof(uint32_t)));
-    AB_TRY(heavy.get(n_heavy * sizeof(uint32_t)));
-    AB_TRY(deficit.get(n_light * sizeof(u64)));
-    AB_TRY(surplus.get(n_heavy * sizeof(u64)));
-    alias_split_kernel<<<grid_for(n), 256, 0, stream>>>(weight.as<u64>(), is_light.as<uint32_t>(),
-                                                        light_rank.as<uint32_t>(), n, capacity, light.as<uint32_t>(),
-                                                        heavy.as<uint32_t>(), deficit.as<u64>(), surplus.as<u64>());
-    AB_TRY(cudaGetLastError());
+    CUDA_CHECK(light.reserve(std::max<size_t>(n_light * sizeof(uint32_t), 1)));
+    CUDA_CHECK(heavy.reserve(n_heavy * sizeof(uint32_t)));
+    CUDA_CHECK(deficit.reserve(std::max<size_t>(n_light * sizeof(u64), 1)));
+    CUDA_CHECK(surplus.reserve(n_heavy * sizeof(u64)));
+    alias_split_kernel<<<grid_for(n), 256, 0, stream>>>(weight.get(), is_light.get(),
+                                                        light_rank.get(), n, capacity, light.get(),
+                                                        heavy.get(), deficit.get(), surplus.get());
+    CUDA_CHECK(cudaGetLastError());
     // running sums: the deficits keep their own copy (the light kernel needs both), in `degree`
-    u64 *deficit_sum = degree.as<u64>();
+    u64 *deficit_sum = degree.get();
     if (n_light) {
         bytes = need;
-        AB_TRY(cub::DeviceScan::InclusiveSum(temp.ptr, bytes, deficit.as<u64>(), deficit_sum, n_light, stream));
+        CUDA_CHECK(cub::DeviceScan::InclusiveSum(temp.get(), bytes, deficit.get(), deficit_sum, n_light, stream));
     }
     bytes = need;
-    AB_TRY(cub::DeviceScan::InclusiveSum(temp.ptr, bytes, surplus.as<u64>(), surplus.as<u64>(), n_heavy, stream));
+    CUDA_CHECK(cub::DeviceScan::InclusiveSum(temp.get(), bytes, surplus.get(), surplus.get(), n_heavy, stream));
     if (n_light) {
-        alias_light_kernel<<<grid_for(n_light), 256, 0, stream>>>(light.as<uint32_t>(), heavy.as<uint32_t>(),
-                                                                  deficit.as<u64>(), deficit_sum, surplus.as<u64>(),
+        alias_light_kernel<<<grid_for(n_light), 256, 0, stream>>>(light.get(), heavy.get(),
+                                                                  deficit.get(), deficit_sum, surplus.get(),
                                                                   n_light, n_heavy, capacity, d_table);
-        AB_TRY(cudaGetLastError());
+        CUDA_CHECK(cudaGetLastError());
     }
-    alias_heavy_kernel<<<grid_for(n_heavy), 256, 0, stream>>>(heavy.as<uint32_t>(), deficit_sum, surplus.as<u64>(), n_light,
+    alias_heavy_kernel<<<grid_for(n_heavy), 256, 0, stream>>>(heavy.get(), deficit_sum, surplus.get(), n_light,
                                                               n_heavy, capacity, d_table);
-    AB_TRY(cudaGetLastError());
-    AB_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     return cudaSuccess;
 }
 

@@ -7,33 +7,18 @@
 
 #include <algorithm>
 #include <chrono>
+#include <functional>
 #include <new>
 
-#include "common.cuh"
+#include "host.cuh"
 
 using namespace b2e;
-
-static thread_local std::string g_last_error;
-
-static int fail(int status, const std::string &message) {
-    g_last_error = message;
-    return status;
-}
-
-#define CUDA_TRY(expr)                                                                       \
-    do {                                                                                     \
-        cudaError_t _e = (expr);                                                             \
-        if (_e != cudaSuccess)                                                               \
-            return fail(B2E_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e));   \
-    } while (0)
 
 #define REQUIRE_HANDLE(h)                                                                    \
     do {                                                                                     \
         if (!(h)) return fail(B2E_ERR_INVALID, "null handle");                               \
         CUDA_TRY(cudaSetDevice((h)->cfg.device));                                            \
     } while (0)
-
-int b2e_set_error(int status, const std::string &message) { return fail(status, message); }  // edge_pred.cu
 
 extern "C" const char *b2e_last_error(void) { return g_last_error.c_str(); }
 extern "C" int b2e_abi_version(void) { return B2E_ABI_VERSION; }
@@ -49,25 +34,19 @@ extern "C" int b2e_device_count(void) {
     return usable;
 }
 
-extern "C" int b2e_select_device(int device) {
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || count == 0)
-        return fail(B2E_ERR_CUDA, std::string("no CUDA device available (there is no CPU fallback): ") +
-                                      cudaGetErrorString(e));
-    if (device < 0 || device >= count) return fail(B2E_ERR_INVALID, "device ordinal out of range");
-    CUDA_TRY(cudaSetDevice(device));
-    return B2E_OK;
+extern "C" int b2e_select_device(int device) { return select_device(device); }
+
+// an accept probability r as an integer threshold: floor(r 2^32), clamped to 2^32
+static unsigned long long quantise(double r) {
+    const double t = floor(r * 4294967296.0);
+    return t >= 4294967296.0 ? 4294967296ull : (unsigned long long)t;
 }
 
 // accept thresholds of the typed-walk tests, [same type, changed type] (oracle/walks.c)
 static void type_thresholds(float change_weight, unsigned long long q[2]) {
     const double w = (double)change_weight, m = w > 1.0 ? w : 1.0;
-    const double ratio[2] = {1.0 / m, w / m};
-    for (int i = 0; i < 2; ++i) {
-        const double t = std::floor(ratio[i] * 4294967296.0);
-        q[i] = t >= 4294967296.0 ? 4294967296ull : (unsigned long long)t;
-    }
+    q[0] = quantise(1.0 / m);
+    q[1] = quantise(w / m);
 }
 
 static bool walklet(const b2e_config &c) { return c.walklet_scale >= 2; }
@@ -79,14 +58,7 @@ static uint32_t sub_walk_length(const b2e_config &c) {
 static void thresholds(float return_weight, float explore_weight, unsigned long long out[3]) {
     const double w[3] = {(double)return_weight, 1.0, (double)explore_weight};
     const double wmax = std::max(w[0], std::max(w[1], w[2]));
-    for (int i = 0; i < 3; ++i) {
-        if (w[i] >= wmax) {
-            out[i] = 4294967296ull;
-        } else {
-            const double t = floor(w[i] / wmax * 4294967296.0);
-            out[i] = t >= 4294967296.0 ? 4294967296ull : (unsigned long long)t;
-        }
-    }
+    for (int i = 0; i < 3; ++i) out[i] = quantise(w[i] / wmax);  // w[i] = wmax gives exactly 2^32
 }
 
 // folded return edge (oracle/walks.c: orc_fold_thresholds): accept thresholds against the envelope
@@ -96,14 +68,7 @@ static void fold_thresholds(float return_weight, float explore_weight, unsigned 
     const double rw = (double)return_weight, ew = (double)explore_weight;
     const double wenv = ew > 1.0 ? ew : 1.0;
     const double w[3] = {wenv, 1.0, ew};
-    for (int i = 0; i < 3; ++i) {
-        if (w[i] >= wenv) {
-            out[i] = 4294967296ull;
-        } else {
-            const double t = floor(w[i] / wenv * 4294967296.0);
-            out[i] = t >= 4294967296.0 ? 4294967296ull : (unsigned long long)t;
-        }
-    }
+    for (int i = 0; i < 3; ++i) out[i] = quantise(w[i] / wenv);
     double e = rw > wenv ? floor((rw - wenv) / wenv * 1048576.0) : 0.0;
     if (e > 2147483648.0) e = 2147483648.0;
     *excess = (uint64_t)e;
@@ -146,13 +111,7 @@ extern "C" int b2e_create(const b2e_config *config, b2e_handle **out) {
     if (!(c.negative_sampling_exponent >= 0.0f))
         return fail(B2E_ERR_INVALID, "negative_sampling_exponent must be non-negative");
 
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || count == 0)
-        return fail(B2E_ERR_CUDA, std::string("no CUDA device available (there is no CPU fallback): ") +
-                                      cudaGetErrorString(e));
-    if (c.device < 0 || c.device >= count) return fail(B2E_ERR_INVALID, "device ordinal out of range");
-    CUDA_TRY(cudaSetDevice(c.device));
+    if (int rc = select_device(c.device)) return rc;
     cudaDeviceProp prop;
     CUDA_TRY(cudaGetDeviceProperties(&prop, c.device));
     if (prop.major < 10)
@@ -176,8 +135,8 @@ extern "C" int b2e_create(const b2e_config *config, b2e_handle **out) {
     }
     if (cudaStreamCreateWithFlags(&h->walk_stream, cudaStreamNonBlocking) != cudaSuccess ||
         cudaStreamCreateWithFlags(&h->train_stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaMalloc(&h->d_counters, sizeof(DeviceCounters)) != cudaSuccess ||
-        cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->train_stream) != cudaSuccess ||
+        h->d_counters.reserve(sizeof(DeviceCounters)) != cudaSuccess ||
+        cudaMemsetAsync(h->d_counters.get(), 0, sizeof(DeviceCounters), h->train_stream) != cudaSuccess ||
         cudaStreamSynchronize(h->train_stream) != cudaSuccess) {
         b2e_destroy(h);
         return fail(B2E_ERR_CUDA, "stream / counter allocation failed");
@@ -200,42 +159,21 @@ static void close_peers(b2e_handle *h) {
     h->peers_are_ipc = false;
 }
 
-static void release_graph(b2e_graph *g) {
-    if (!g || --g->references > 0) return;
-    cudaFree(g->csr.indptr);
-    cudaFree(g->csr.indices);
-    delete g;
+static int require_graph(b2e_handle *h) {
+    if (!h->graph.csr) return fail(B2E_ERR_STATE, "b2e_load_csr must be called first");
+    return B2E_OK;
 }
 
-static void free_graph(b2e_handle *h) {
+static void drop_graph(b2e_handle *h) {
     close_peers(h);
-    if (h->shared_graph) {  // the CSR belongs to a b2e_graph: drop this handle's reference
-        release_graph(h->shared_graph);
-        h->shared_graph = nullptr;
-        h->d_indptr = nullptr;
-        h->d_indices = nullptr;
-    }
-    cudaFree(h->d_indptr); h->d_indptr = nullptr;
-    cudaFree(h->d_indices); h->d_indices = nullptr;
-    cudaFree(h->d_edge_alias); h->d_edge_alias = nullptr;
-    cudaFree(h->d_node_types); h->d_node_types = nullptr;
-    cudaFree(h->d_edge_types); h->d_edge_types = nullptr;
-    cudaFree(h->d_sources); h->d_sources = nullptr;
-    cudaFree(h->d_filter); h->d_filter = nullptr;
-    cudaFree(h->d_alias); h->d_alias = nullptr;
-    cudaFree(h->d_t0); h->d_t0 = nullptr;
-    cudaFree(h->d_t1); h->d_t1 = nullptr;
-    for (int s = 0; s < 2; ++s) { cudaFree(h->d_walks[s]); h->d_walks[s] = nullptr; }
-    cudaFree(h->d_walk_raw); h->d_walk_raw = nullptr;
-    b2e::glove_free(h->glove);
+    h->graph = HandleGraph();
 }
 
 extern "C" void b2e_destroy(b2e_handle *h) {
     if (!h) return;
     cudaSetDevice(h->cfg.device);
     cudaDeviceSynchronize();
-    free_graph(h);
-    cudaFree(h->d_counters);
+    drop_graph(h);
     for (int s = 0; s < 2; ++s) {
         if (h->walk_done[s]) cudaEventDestroy(h->walk_done[s]);
         if (h->train_done[s]) cudaEventDestroy(h->train_done[s]);
@@ -288,18 +226,18 @@ static bool build_edge_alias(const int64_t *indptr, const float *weights, uint64
 
 extern "C" int b2e_load_types(b2e_handle *h, const uint32_t *node_types, const uint32_t *edge_types) {
     REQUIRE_HANDLE(h);
-    if (!h->d_indptr) return fail(B2E_ERR_STATE, "b2e_load_csr must be called first");
+    if (int rc = require_graph(h)) return rc;
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
-    cudaFree(h->d_node_types); h->d_node_types = nullptr;
-    cudaFree(h->d_edge_types); h->d_edge_types = nullptr;
+    h->graph.node_types.reset();
+    h->graph.edge_types.reset();
     if (node_types && h->n) {
-        CUDA_TRY(cudaMalloc(&h->d_node_types, h->n * sizeof(uint32_t)));
-        CUDA_TRY(cudaMemcpyAsync(h->d_node_types, node_types, h->n * sizeof(uint32_t),
+        CUDA_TRY(h->graph.node_types.reserve(h->n * sizeof(uint32_t)));
+        CUDA_TRY(cudaMemcpyAsync(h->graph.node_types.get(), node_types, h->n * sizeof(uint32_t),
                                  cudaMemcpyHostToDevice, h->walk_stream));
     }
     if (edge_types && h->nnz) {
-        CUDA_TRY(cudaMalloc(&h->d_edge_types, h->nnz * sizeof(uint32_t)));
-        CUDA_TRY(cudaMemcpyAsync(h->d_edge_types, edge_types, h->nnz * sizeof(uint32_t),
+        CUDA_TRY(h->graph.edge_types.reserve(h->nnz * sizeof(uint32_t)));
+        CUDA_TRY(cudaMemcpyAsync(h->graph.edge_types.get(), edge_types, h->nnz * sizeof(uint32_t),
                                  cudaMemcpyHostToDevice, h->walk_stream));
     }
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));  // the caller's buffers may go away
@@ -311,35 +249,156 @@ extern "C" int b2e_load_csr(b2e_handle *h, const int64_t *indptr, const uint32_t
     return b2e_load_csr_weighted(h, indptr, indices, nullptr, n, nnz);
 }
 
-// two int flags on the device, freed on every way out of a load
-struct DeviceFlags {
-    int *ptr = nullptr;
-    ~DeviceFlags() { cudaFree(ptr); }
-};
+// Everything a load builds on the device once the old graph is gone.  `d_flags` belongs to the
+// caller, so that a failed load frees it only after the device has been drained.
+static int build_graph(b2e_handle *h, const int64_t *indptr, const uint32_t *indices, const float *weights,
+                       b2e_graph *resident, DeviceBuffer<int> &d_flags,
+                       const std::function<void(const char *)> &lap) {
+    const b2e_config &c = h->cfg;
+    const uint64_t n = h->n, nnz = h->nnz;
+    HandleGraph &g = h->graph;
+    // K1: the two big copies into a graph of this handle's own (none when the CSR is resident
+    // already), then the checks on the device: offsets non-decreasing and within nnz; ids in
+    // range, rows strictly ascending (the kernels index with these ids and bisect these rows
+    // without looking again)
+    if (resident) {
+        ++resident->references;
+        g.csr.reset(resident);
+    } else {
+        g.csr.reset(new b2e_graph());
+        ResidentCsr &upload = g.csr->csr;
+        g.csr->device = c.device;
+        upload.n = n;
+        upload.nnz = nnz;
+        CUDA_TRY(upload.indptr.reserve((n + 1) * sizeof(int64_t)));
+        CUDA_TRY(upload.indices.reserve(nnz * sizeof(uint32_t)));
+        CUDA_TRY(cudaMemcpyAsync(upload.indptr.get(), indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice,
+                                 h->walk_stream));
+        CUDA_TRY(cudaMemcpyAsync(upload.indices.get(), indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice,
+                                 h->walk_stream));
+    }
+    const int64_t *d_indptr = g.csr->csr.indptr.get();
+    const uint32_t *d_indices = g.csr->csr.indices.get();
+    int flags[2] = {0, 1};
+    CUDA_TRY(d_flags.reserve(2 * sizeof(int)));
+    CUDA_TRY(cudaMemsetAsync(d_flags.get(), 0, 2 * sizeof(int), h->walk_stream));
+    CUDA_TRY(check_indptr_device(d_indptr, n, nnz, d_flags.get(), h->walk_stream));
+    CUDA_TRY(cudaMemcpyAsync(flags, d_flags.get(), sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
+    CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+    if (flags[0]) return fail(B2E_ERR_INVALID, "indptr must be non-decreasing and end at nnz");
+    CUDA_TRY(launch_csr_check(d_indptr, d_indices, n, d_flags.get(), h->sm_count, h->walk_stream));
+    h->launches += 2;
+    CUDA_TRY(cudaMemcpyAsync(flags, d_flags.get(), sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
+    CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+    lap("CSR upload + content checks");
+    if (flags[0]) {
+        return fail(B2E_ERR_INVALID, flags[0] & 1 ? "a destination node id is out of range"
+                                                  : "neighbour lists must be sorted strictly ascending within each row");
+    }
 
-// a failed load leaves the handle without a graph (require_graph() then fails cleanly)
-static int load_failed(b2e_handle *h, int rc) {
-    cudaDeviceSynchronize();
-    free_graph(h);
-    h->n = h->nnz = h->n_src = 0;
-    return rc;
-}
+    // K3 on the device: start nodes, maximum degree, alias table over deg^alpha (alias_build.cu)
+    h->h_alias_thr.clear();
+    h->h_alias_idx.clear();
+    {
+        DeviceBuffer<uint32_t> sources_all;
+        CUDA_TRY(sources_all.reserve(n * sizeof(uint32_t)));
+        if (c.use_scale_free_distribution && g.alias.reserve(n * sizeof(uint2)) != cudaSuccess)
+            return fail(B2E_ERR_CUDA, "out of device memory (alias table)");
+        std::string error;
+        uint64_t n_src = 0, max_degree = 0;
+        const cudaError_t e = build_node_tables(d_indptr, indptr, n, (double)c.negative_sampling_exponent,
+                                                sources_all.get(), &n_src, &max_degree, g.alias.get(), h->walk_stream,
+                                                error);
+        if (e != cudaSuccess) return fail(e == cudaErrorInvalidValue ? B2E_ERR_INVALID : B2E_ERR_CUDA, error);
+        CUDA_TRY(g.sources.reserve(std::max<uint64_t>(1, n_src) * sizeof(uint32_t)));
+        if (n_src)
+            CUDA_TRY(cudaMemcpy(g.sources.get(), sources_all.get(), n_src * sizeof(uint32_t), cudaMemcpyDeviceToDevice));
+        h->n_src = n_src;
+        h->max_degree = (uint32_t)std::min<uint64_t>(max_degree, 0xFFFFFFFEull);
+        h->launches += 8;
+    }
+    lap("start nodes + alias table (GPU)");
 
-#define LOAD_TRY(expr)                                                                                     \
-    do {                                                                                                   \
-        cudaError_t _e = (expr);                                                                           \
-        if (_e != cudaSuccess)                                                                             \
-            return load_failed(h, fail(B2E_ERR_CUDA, std::string(#expr) + ": " + cudaGetErrorString(_e))); \
-    } while (0)
+    // normalize_by_degree (.../node2vec_skipgram.py:94-96): the weight of v -> x divided by
+    // max(deg(x), 1), one float32 division per edge, folded into the proposal table -- no extra
+    // rejection however skewed the degrees (oracle: degree_normalised_weights)
+    std::vector<float> normalised;
+    std::vector<uint32_t> fetched_indices;
+    std::vector<int64_t> fetched_indptr;
+    if ((c.normalize_by_degree || weights) && !indptr) {  // resident graph: these options work on the host
+        fetched_indptr.resize(n + 1);
+        CUDA_TRY(cudaMemcpy(fetched_indptr.data(), d_indptr, (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost));
+        indptr = fetched_indptr.data();
+    }
+    if (c.normalize_by_degree) {
+        if (!indices) {  // resident graph: this rarely used option needs the ids on the host
+            fetched_indices.resize(nnz);
+            CUDA_TRY(cudaMemcpy(fetched_indices.data(), d_indices, nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+            indices = fetched_indices.data();
+        }
+        normalised.resize(nnz);
+        for (uint64_t e = 0; e < nnz; ++e) {
+            const uint32_t x = indices[e];
+            const float degree = (float)std::max<int64_t>(indptr[x + 1] - indptr[x], 1);
+            normalised[e] = (weights ? weights[e] : 1.0f) / degree;
+        }
+        weights = normalised.data();
+    }
+    if (weights) {
+        std::vector<uint2> edge_alias(nnz);
+        if (!build_edge_alias(indptr, weights, n, edge_alias))
+            return fail(B2E_ERR_INVALID, "edge weights must be non-negative numbers");
+        CUDA_TRY(g.edge_alias.reserve(nnz * sizeof(uint2)));
+        CUDA_TRY(cudaMemcpyAsync(g.edge_alias.get(), edge_alias.data(), nnz * sizeof(uint2), cudaMemcpyHostToDevice,
+                                 h->walk_stream));
+        CUDA_TRY(cudaStreamSynchronize(h->walk_stream));  // `edge_alias` dies here
+    }
 
-static int load_graph_common(b2e_handle *h, const int64_t *indptr, const uint32_t *indices, const float *weights,
-                             uint64_t n, uint64_t nnz, b2e_graph *resident);
+    lap("edge alias tables (weighted graphs)");
+    // Second-order walks: is the graph undirected (every edge mirrored)?  Verified here, never
+    // assumed: it allows the adjacency check in the shorter of the two rows and the folded return
+    // edge.  The row filters answer most adjacency checks with one gather (walk_kernels.cu).
+    h->undirected = false;
+    h->fold_excess = 0;
+    if (h->second_order) {
+        if (!getenv("B2E_ASSUME_DIRECTED")) {
+            CUDA_TRY(cudaMemcpyAsync(d_flags.get() + 1, flags + 1, sizeof(int), cudaMemcpyHostToDevice, h->walk_stream));
+            CUDA_TRY(launch_symmetry_check(d_indptr, d_indices, n, nnz, d_flags.get() + 1, h->walk_stream));
+            CUDA_TRY(cudaMemcpyAsync(flags + 1, d_flags.get() + 1, sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
+            CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+            h->undirected = flags[1] != 0;
+            ++h->launches;
+            lap("symmetry check");
+        }
+        uint64_t excess = 0;
+        fold_thresholds(c.return_weight, c.explore_weight, h->thr_fold, &excess);
+        if (h->undirected && !weights && !getenv("B2E_NO_FOLD")) h->fold_excess = excess;
+        if (!getenv("B2E_NO_FILTER")) {
+            const uint64_t words = row_filter_words(nnz);
+            CUDA_TRY(g.filter.reserve(words * sizeof(unsigned long long)));
+            CUDA_TRY(cudaMemsetAsync(g.filter.get(), 0, words * sizeof(unsigned long long), h->walk_stream));
+            CUDA_TRY(launch_row_filter_build(d_indptr, d_indices, n, g.filter.get(), h->sm_count, h->walk_stream));
+            ++h->launches;
+        }
+    }
+    lap("row filters");
 
-extern "C" int b2e_load_csr_weighted(b2e_handle *h, const int64_t *indptr, const uint32_t *indices,
-                                     const float *weights, uint64_t n, uint64_t nnz) {
-    REQUIRE_HANDLE(h);
-    if (!indptr || (!indices && nnz)) return fail(B2E_ERR_INVALID, "null CSR pointer");
-    return load_graph_common(h, indptr, indices, weights, n, nnz, nullptr);
+    CUDA_TRY(g.t0.reserve(n * (uint64_t)h->row_stride * sizeof(float)));
+    CUDA_TRY(g.t1.reserve(n * (uint64_t)h->row_stride * sizeof(float)));
+
+    const uint64_t per_epoch = (uint64_t)c.iterations * h->n_src;
+    // an explicit chunk_walks is honoured as given (parity tests feed host walks of that size)
+    const uint64_t cap = c.chunk_walks ? c.chunk_walks
+                                       : std::max<uint64_t>(1, std::min<uint64_t>(1ull << 20, per_epoch));
+    h->chunk_cap = cap;
+    // Walklets: a slot holds the k sub-walks of every walk, k * ceil(L / k) >= L tokens per walk
+    const uint64_t slot_tokens = walklet(c) ? (uint64_t)c.walklet_scale * sub_walk_length(c) : c.walk_length;
+    for (int s = 0; s < 2; ++s)
+        CUDA_TRY(g.walks[s].reserve(cap * slot_tokens * sizeof(uint32_t)));
+    if (walklet(c)) CUDA_TRY(g.walk_raw.reserve(cap * c.walk_length * sizeof(uint32_t)));
+    CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+    lap("tables + walk ring allocation");
+    return B2E_OK;
 }
 
 // `resident`: the CSR already lives in HBM (b2e_load_graph) -- `indptr` is a host copy of its
@@ -351,7 +410,6 @@ static int load_graph_common(b2e_handle *h, const int64_t *indptr, const uint32_
     if (nnz == 0) return fail(B2E_ERR_INVALID, "The provided graph does not have edges.");
     if (indptr && (indptr[0] != 0 || (uint64_t)indptr[n] != nnz))
         return fail(B2E_ERR_INVALID, "indptr must start at 0 and end at nnz");
-    const b2e_config &c = h->cfg;
     // B2E_LOAD_TIMING=1: where the time of a load goes, on stderr
     const bool timing = getenv("B2E_LOAD_TIMING") != nullptr;
     auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
@@ -368,156 +426,24 @@ static int load_graph_common(b2e_handle *h, const int64_t *indptr, const uint32_
             if (!(weights[e] >= 0.0f)) return fail(B2E_ERR_INVALID, "edge weights must be non-negative numbers");
 
     CUDA_TRY(cudaDeviceSynchronize());
-    free_graph(h);
+    drop_graph(h);
     h->n = n;
     h->nnz = nnz;
+    DeviceBuffer<int> d_flags;
+    const int rc = build_graph(h, indptr, indices, weights, resident, d_flags, lap);
+    if (rc != B2E_OK) {  // a failed load leaves the handle without a graph (require_graph() then fails cleanly)
+        cudaDeviceSynchronize();
+        drop_graph(h);
+        h->n = h->nnz = h->n_src = 0;
+    }
+    return rc;
+}
 
-    // K1: the two big copies (none when the CSR is resident already), then the checks on the
-    // device: offsets non-decreasing and within nnz; ids in range, rows strictly ascending (the
-    // kernels index with these ids and bisect these rows without looking again)
-    if (resident) {
-        h->shared_graph = resident;
-        ++resident->references;
-        h->d_indptr = resident->csr.indptr;
-        h->d_indices = resident->csr.indices;
-    } else {
-        LOAD_TRY(cudaMalloc(&h->d_indptr, (n + 1) * sizeof(int64_t)));
-        LOAD_TRY(cudaMalloc(&h->d_indices, nnz * sizeof(uint32_t)));
-        LOAD_TRY(cudaMemcpyAsync(h->d_indptr, indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice,
-                                 h->walk_stream));
-        LOAD_TRY(cudaMemcpyAsync(h->d_indices, indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice,
-                                 h->walk_stream));
-    }
-    DeviceFlags flag_words;
-    int flags[2] = {0, 1};
-    LOAD_TRY(cudaMalloc(&flag_words.ptr, 2 * sizeof(int)));
-    int *const d_flags = flag_words.ptr;
-    LOAD_TRY(cudaMemsetAsync(d_flags, 0, 2 * sizeof(int), h->walk_stream));
-    LOAD_TRY(check_indptr_device(h->d_indptr, n, nnz, d_flags, h->walk_stream));
-    LOAD_TRY(cudaMemcpyAsync(flags, d_flags, sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
-    LOAD_TRY(cudaStreamSynchronize(h->walk_stream));
-    if (flags[0]) return load_failed(h, fail(B2E_ERR_INVALID, "indptr must be non-decreasing and end at nnz"));
-    LOAD_TRY(launch_csr_check(h->d_indptr, h->d_indices, n, d_flags, h->sm_count, h->walk_stream));
-    h->launches += 2;
-    LOAD_TRY(cudaMemcpyAsync(flags, d_flags, sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
-    LOAD_TRY(cudaStreamSynchronize(h->walk_stream));
-    lap("CSR upload + content checks");
-    if (flags[0]) {
-        return load_failed(h, fail(B2E_ERR_INVALID, flags[0] & 1
-                                        ? "a destination node id is out of range"
-                                        : "neighbour lists must be sorted strictly ascending within each row"));
-    }
-
-    // K3 on the device: start nodes, maximum degree, alias table over deg^alpha (alias_build.cu)
-    h->h_alias_thr.clear();
-    h->h_alias_idx.clear();
-    {
-        uint32_t *d_sources_all = nullptr;
-        LOAD_TRY(cudaMalloc(&d_sources_all, n * sizeof(uint32_t)));
-        if (c.use_scale_free_distribution && cudaMalloc(&h->d_alias, n * sizeof(uint2)) != cudaSuccess) {
-            cudaFree(d_sources_all);
-            return load_failed(h, fail(B2E_ERR_CUDA, "out of device memory (alias table)"));
-        }
-        std::string error;
-        uint64_t n_src = 0, max_degree = 0;
-        cudaError_t e = build_node_tables(h->d_indptr, indptr, n, (double)c.negative_sampling_exponent, d_sources_all,
-                                          &n_src, &max_degree, h->d_alias, h->walk_stream, error);
-        if (e == cudaSuccess) e = cudaMalloc(&h->d_sources, std::max<uint64_t>(1, n_src) * sizeof(uint32_t));
-        if (e == cudaSuccess && n_src)
-            e = cudaMemcpy(h->d_sources, d_sources_all, n_src * sizeof(uint32_t), cudaMemcpyDeviceToDevice);
-        cudaFree(d_sources_all);
-        if (e != cudaSuccess) {
-            if (error.empty()) error = std::string("start-node list: ") + cudaGetErrorString(e);
-            return load_failed(h, fail(e == cudaErrorInvalidValue ? B2E_ERR_INVALID : B2E_ERR_CUDA, error));
-        }
-        h->n_src = n_src;
-        h->max_degree = (uint32_t)std::min<uint64_t>(max_degree, 0xFFFFFFFEull);
-        h->launches += 8;
-    }
-    lap("start nodes + alias table (GPU)");
-
-    // normalize_by_degree (.../node2vec_skipgram.py:94-96): the weight of v -> x divided by
-    // max(deg(x), 1), one float32 division per edge, folded into the proposal table -- no extra
-    // rejection however skewed the degrees (oracle: degree_normalised_weights)
-    std::vector<float> normalised;
-    std::vector<uint32_t> fetched_indices;
-    std::vector<int64_t> fetched_indptr;
-    if ((c.normalize_by_degree || weights) && !indptr) {  // resident graph: these options work on the host
-        fetched_indptr.resize(n + 1);
-        LOAD_TRY(cudaMemcpy(fetched_indptr.data(), h->d_indptr, (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost));
-        indptr = fetched_indptr.data();
-    }
-    if (c.normalize_by_degree) {
-        if (!indices) {  // resident graph: this rarely used option needs the ids on the host
-            fetched_indices.resize(nnz);
-            LOAD_TRY(cudaMemcpy(fetched_indices.data(), h->d_indices, nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-            indices = fetched_indices.data();
-        }
-        normalised.resize(nnz);
-        for (uint64_t e = 0; e < nnz; ++e) {
-            const uint32_t x = indices[e];
-            const float degree = (float)std::max<int64_t>(indptr[x + 1] - indptr[x], 1);
-            normalised[e] = (weights ? weights[e] : 1.0f) / degree;
-        }
-        weights = normalised.data();
-    }
-    if (weights) {
-        std::vector<uint2> edge_alias(nnz);
-        if (!build_edge_alias(indptr, weights, n, edge_alias)) {
-                return load_failed(h, fail(B2E_ERR_INVALID, "edge weights must be non-negative numbers"));
-        }
-        LOAD_TRY(cudaMalloc(&h->d_edge_alias, nnz * sizeof(uint2)));
-        LOAD_TRY(cudaMemcpyAsync(h->d_edge_alias, edge_alias.data(), nnz * sizeof(uint2), cudaMemcpyHostToDevice,
-                                 h->walk_stream));
-        LOAD_TRY(cudaStreamSynchronize(h->walk_stream));  // `edge_alias` dies here
-    }
-
-    lap("edge alias tables (weighted graphs)");
-    // Second-order walks: is the graph undirected (every edge mirrored)?  Verified here, never
-    // assumed: it allows the adjacency check in the shorter of the two rows and the folded return
-    // edge.  The row filters answer most adjacency checks with one gather (walk_kernels.cu).
-    h->undirected = false;
-    h->fold_excess = 0;
-    if (h->second_order) {
-        if (!getenv("B2E_ASSUME_DIRECTED")) {
-            LOAD_TRY(cudaMemcpyAsync(d_flags + 1, flags + 1, sizeof(int), cudaMemcpyHostToDevice, h->walk_stream));
-            LOAD_TRY(launch_symmetry_check(h->d_indptr, h->d_indices, n, nnz, d_flags + 1, h->walk_stream));
-            LOAD_TRY(cudaMemcpyAsync(flags + 1, d_flags + 1, sizeof(int), cudaMemcpyDeviceToHost, h->walk_stream));
-            LOAD_TRY(cudaStreamSynchronize(h->walk_stream));
-            h->undirected = flags[1] != 0;
-            ++h->launches;
-            lap("symmetry check");
-        }
-        uint64_t excess = 0;
-        fold_thresholds(c.return_weight, c.explore_weight, h->thr_fold, &excess);
-        if (h->undirected && !weights && !getenv("B2E_NO_FOLD")) h->fold_excess = excess;
-        if (!getenv("B2E_NO_FILTER")) {
-            const uint64_t words = row_filter_words(nnz);
-            LOAD_TRY(cudaMalloc(&h->d_filter, words * sizeof(unsigned long long)));
-            LOAD_TRY(cudaMemsetAsync(h->d_filter, 0, words * sizeof(unsigned long long), h->walk_stream));
-            LOAD_TRY(launch_row_filter_build(h->d_indptr, h->d_indices, n, h->d_filter, h->sm_count,
-                                             h->walk_stream));
-            ++h->launches;
-        }
-    }
-    lap("row filters");
-
-    LOAD_TRY(cudaMalloc(&h->d_t0, n * (uint64_t)h->row_stride * sizeof(float)));
-    LOAD_TRY(cudaMalloc(&h->d_t1, n * (uint64_t)h->row_stride * sizeof(float)));
-
-    const uint64_t per_epoch = (uint64_t)c.iterations * h->n_src;
-    // an explicit chunk_walks is honoured as given (parity tests feed host walks of that size)
-    const uint64_t cap = c.chunk_walks ? c.chunk_walks
-                                       : std::max<uint64_t>(1, std::min<uint64_t>(1ull << 20, per_epoch));
-    h->chunk_cap = cap;
-    // Walklets: a slot holds the k sub-walks of every walk, k * ceil(L / k) >= L tokens per walk
-    const uint64_t slot_tokens = walklet(c) ? (uint64_t)c.walklet_scale * sub_walk_length(c) : c.walk_length;
-    for (int s = 0; s < 2; ++s)
-        LOAD_TRY(cudaMalloc(&h->d_walks[s], cap * slot_tokens * sizeof(uint32_t)));
-    if (walklet(c)) LOAD_TRY(cudaMalloc(&h->d_walk_raw, cap * c.walk_length * sizeof(uint32_t)));
-    LOAD_TRY(cudaStreamSynchronize(h->walk_stream));
-    lap("tables + walk ring allocation");
-    return B2E_OK;
+extern "C" int b2e_load_csr_weighted(b2e_handle *h, const int64_t *indptr, const uint32_t *indices,
+                                     const float *weights, uint64_t n, uint64_t nnz) {
+    REQUIRE_HANDLE(h);
+    if (!indptr || (!indices && nnz)) return fail(B2E_ERR_INVALID, "null CSR pointer");
+    return load_graph_common(h, indptr, indices, weights, n, nnz, nullptr);
 }
 
 extern "C" uint64_t b2e_number_of_sources(const b2e_handle *h) { return h ? h->n_src : 0; }
@@ -543,15 +469,10 @@ extern "C" int b2e_set_streams(b2e_handle *h, void *walk_stream, void *train_str
     return B2E_OK;
 }
 
-static int require_graph(b2e_handle *h) {
-    if (!h->d_indptr) return fail(B2E_ERR_STATE, "b2e_load_csr must be called first");
-    return B2E_OK;
-}
-
 extern "C" int b2e_init_tables(b2e_handle *h, uint64_t seed) {
     REQUIRE_HANDLE(h);
     if (int rc = require_graph(h)) return rc;
-    CUDA_TRY(launch_init_tables(h->d_t0, h->d_t1, h->n, h->cfg.embedding_size, h->row_stride, seed,
+    CUDA_TRY(launch_init_tables(h->graph.t0.get(), h->graph.t1.get(), h->n, h->cfg.embedding_size, h->row_stride, seed,
                                 h->train_stream));
     ++h->launches;
     return B2E_OK;
@@ -560,14 +481,14 @@ extern "C" int b2e_init_tables(b2e_handle *h, uint64_t seed) {
 static int walk_into(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t n_walks,
                      uint64_t walk_id_stride, uint32_t *d_out, cudaStream_t stream) {
     WalkParams p;
-    p.indptr = h->d_indptr;
-    p.indices = h->d_indices;
-    p.edge_alias = h->d_edge_alias;
-    p.node_types = h->d_node_types;
-    p.edge_types = h->d_edge_types;
-    type_thresholds(h->d_node_types ? h->cfg.change_node_type_weight : 1.0f, p.q_node);
-    type_thresholds(h->d_edge_types ? h->cfg.change_edge_type_weight : 1.0f, p.q_edge);
-    p.sources = h->d_sources;
+    p.indptr = h->graph.csr->csr.indptr.get();
+    p.indices = h->graph.csr->csr.indices.get();
+    p.edge_alias = h->graph.edge_alias.get();
+    p.node_types = h->graph.node_types.get();
+    p.edge_types = h->graph.edge_types.get();
+    type_thresholds(h->graph.node_types.get() ? h->cfg.change_node_type_weight : 1.0f, p.q_node);
+    type_thresholds(h->graph.edge_types.get() ? h->cfg.change_edge_type_weight : 1.0f, p.q_edge);
+    p.sources = h->graph.sources.get();
     p.n_src = h->n_src;
     p.seed_lo = (uint32_t)seed;
     p.seed_hi = (uint32_t)(seed >> 32);
@@ -576,15 +497,15 @@ static int walk_into(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t
     p.walk_id_stride = walk_id_stride;
     p.walk_length = h->cfg.walk_length;
     // typed walks keep the plain envelope (their trial loop has its own Philox layout)
-    const bool typed = (h->d_node_types && p.q_node[0] != p.q_node[1]) || (h->d_edge_types && p.q_edge[0] != p.q_edge[1]);
+    const bool typed = (h->graph.node_types.get() && p.q_node[0] != p.q_node[1]) || (h->graph.edge_types.get() && p.q_edge[0] != p.q_edge[1]);
     const unsigned long long *thr = h->fold_excess && !typed ? h->thr_fold : h->thr;
     p.fold_excess = typed ? 0 : h->fold_excess;
-    p.filter = h->d_filter;
+    p.filter = h->graph.filter.get();
     p.thr_return = thr[0];
     p.thr_common = thr[1];
     p.thr_explore = thr[2];
     p.out = d_out;
-    p.counters = h->d_counters;
+    p.counters = h->d_counters.get();
     p.undirected = h->undirected ? 1u : 0u;
     p.sm_count = h->sm_count;
     CUDA_TRY(launch_walks(p, h->second_order, stream));
@@ -602,12 +523,12 @@ extern "C" int b2e_walk_chunk(b2e_handle *h, uint64_t seed, uint64_t first_walk,
     if (h->n_src == 0) return fail(B2E_ERR_INVALID, "the graph has no node with outgoing edges");
     // the slot may still be read by the SGD kernel of two chunks ago
     CUDA_TRY(cudaStreamWaitEvent(h->walk_stream, h->train_done[slot], 0));
-    uint32_t *target = walklet(h->cfg) ? h->d_walk_raw : h->d_walks[slot];
+    uint32_t *target = walklet(h->cfg) ? h->graph.walk_raw.get() : h->graph.walks[slot].get();
     if (int rc = walk_into(h, seed, first_walk, n_walks, walk_id_stride, target, h->walk_stream))
         return rc;
     if (walklet(h->cfg)) {
-        CUDA_TRY(launch_walklet_split(h->d_walk_raw, n_walks, h->cfg.walk_length, h->cfg.walklet_scale,
-                                      h->d_walks[slot], h->walk_stream));
+        CUDA_TRY(launch_walklet_split(h->graph.walk_raw.get(), n_walks, h->cfg.walk_length, h->cfg.walklet_scale,
+                                      h->graph.walks[slot].get(), h->walk_stream));
         if (n_walks) ++h->launches;
     }
     CUDA_TRY(cudaEventRecord(h->walk_done[slot], h->walk_stream));
@@ -631,14 +552,14 @@ extern "C" int b2e_adopt_walks(b2e_handle *dst, b2e_handle *src, uint32_t slot) 
     const uint64_t n_walks = src->slot_count[slot];
     if (n_walks > dst->chunk_cap) return fail(B2E_ERR_INVALID, "the chunk exceeds the capacity of the adopting handle");
     const uint32_t L = dst->cfg.walk_length;
-    const uint32_t *raw = walklet(src->cfg) ? src->d_walk_raw : src->d_walks[slot];
+    const uint32_t *raw = walklet(src->cfg) ? src->graph.walk_raw.get() : src->graph.walks[slot].get();
     CUDA_TRY(cudaStreamWaitEvent(dst->walk_stream, src->walk_done[slot], 0));
     CUDA_TRY(cudaStreamWaitEvent(dst->walk_stream, dst->train_done[slot], 0));
     if (walklet(dst->cfg)) {
-        CUDA_TRY(launch_walklet_split(raw, n_walks, L, dst->cfg.walklet_scale, dst->d_walks[slot], dst->walk_stream));
+        CUDA_TRY(launch_walklet_split(raw, n_walks, L, dst->cfg.walklet_scale, dst->graph.walks[slot].get(), dst->walk_stream));
         if (n_walks) ++dst->launches;
     } else {
-        CUDA_TRY(cudaMemcpyAsync(dst->d_walks[slot], raw, n_walks * L * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
+        CUDA_TRY(cudaMemcpyAsync(dst->graph.walks[slot].get(), raw, n_walks * L * sizeof(uint32_t), cudaMemcpyDeviceToDevice,
                                  dst->walk_stream));
     }
     CUDA_TRY(cudaEventRecord(dst->walk_done[slot], dst->walk_stream));
@@ -653,7 +574,7 @@ static int train_slot(b2e_handle *h, uint64_t seed, uint32_t slot, float learnin
     if (c.model == B2E_GLOVE)
         return fail(B2E_ERR_STATE, "a GloVe handle trains with b2e_cooccurrence + b2e_glove_train");
     TrainParams p;
-    p.walks = h->d_walks[slot];
+    p.walks = h->graph.walks[slot].get();
     p.first_walk = h->slot_first[slot];
     p.n_walks = h->slot_count[slot];
     p.walk_id_stride = h->slot_stride[slot];
@@ -673,11 +594,11 @@ static int train_slot(b2e_handle *h, uint64_t seed, uint32_t slot, float learnin
     p.downsample = c.stochastic_downsample_by_degree ? h->max_degree + 1u : 0u;
     p.scale_dot = c.scale_by_sqrt_dim ? 1u : 0u;
     p.shared_negatives = c.shared_negatives ? 1u : 0u;
-    p.alias = h->d_alias;
-    p.indptr = h->d_indptr;
-    p.t0 = h->d_t0;
-    p.t1 = h->d_t1;
-    p.counters = h->d_counters;
+    p.alias = h->graph.alias.get();
+    p.indptr = h->graph.csr->csr.indptr.get();
+    p.t0 = h->graph.t0.get();
+    p.t1 = h->graph.t1.get();
+    p.counters = h->d_counters.get();
     // Hogwild staleness: on a tiny graph thousands of concurrent walks would all train against
     // nearly the same stale rows, which slows the first epochs down (the final quality is not
     // affected: scripts/exp_concurrency.py).  Unless told otherwise keep about one walk in flight
@@ -690,7 +611,7 @@ static int train_slot(b2e_handle *h, uint64_t seed, uint32_t slot, float learnin
     // g + r * 2^48 (walk ids stay far below 2^48), the slot is laid out [r][walk][token]
     const uint32_t passes = walklet(c) ? c.walklet_scale : 1u;
     for (uint32_t r = 0; r < passes; ++r) {
-        p.walks = h->d_walks[slot] + (uint64_t)r * p.n_walks * p.walk_length;
+        p.walks = h->graph.walks[slot].get() + (uint64_t)r * p.n_walks * p.walk_length;
         p.first_walk = h->slot_first[slot] + ((uint64_t)r << 48);
         CUDA_TRY(launch_train(p, c.model, c.deterministic != 0, h->sm_count, max_warps, h->train_stream));
         if (p.n_walks) ++h->launches;
@@ -717,12 +638,12 @@ extern "C" int b2e_train_host_walks(b2e_handle *h, uint64_t seed, const uint32_t
     if (n_walks > h->chunk_cap) return fail(B2E_ERR_INVALID, "n_walks exceeds the chunk capacity");
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
-    uint32_t *target = walklet(h->cfg) ? h->d_walk_raw : h->d_walks[0];
+    uint32_t *target = walklet(h->cfg) ? h->graph.walk_raw.get() : h->graph.walks[0].get();
     CUDA_TRY(cudaMemcpyAsync(target, walks, n_walks * h->cfg.walk_length * sizeof(uint32_t),
                              cudaMemcpyHostToDevice, h->train_stream));  // ordered before the kernel
     if (walklet(h->cfg))
-        CUDA_TRY(launch_walklet_split(h->d_walk_raw, n_walks, h->cfg.walk_length, h->cfg.walklet_scale,
-                                      h->d_walks[0], h->train_stream));
+        CUDA_TRY(launch_walklet_split(h->graph.walk_raw.get(), n_walks, h->cfg.walk_length, h->cfg.walklet_scale,
+                                      h->graph.walks[0].get(), h->train_stream));
     h->slot_first[0] = first_walk;
     h->slot_count[0] = n_walks;
     h->slot_stride[0] = walk_id_stride;
@@ -739,7 +660,7 @@ extern "C" int b2e_slot_walks(b2e_handle *h, uint32_t slot, uint64_t n_walks, ui
     if (!out && n_walks) return fail(B2E_ERR_INVALID, "null output buffer");
     if (n_walks > h->slot_count[slot]) return fail(B2E_ERR_INVALID, "n_walks exceeds the walks in the slot");
     if (int rc = b2e_sync(h)) return rc;
-    CUDA_TRY(cudaMemcpyAsync(out, h->d_walks[slot], n_walks * h->cfg.walk_length * sizeof(uint32_t),
+    CUDA_TRY(cudaMemcpyAsync(out, h->graph.walks[slot].get(), n_walks * h->cfg.walk_length * sizeof(uint32_t),
                              cudaMemcpyDeviceToHost, h->train_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     return B2E_OK;
@@ -765,9 +686,9 @@ extern "C" int b2e_walks(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint
     while (done < n_walks) {
         const uint64_t count = std::min(h->chunk_cap, n_walks - done);
         if (int rc = walk_into(h, seed, first_walk + done * walk_id_stride, count, walk_id_stride,
-                               h->d_walks[0], h->walk_stream))
+                               h->graph.walks[0].get(), h->walk_stream))
             return rc;
-        CUDA_TRY(cudaMemcpyAsync(out + done * L, h->d_walks[0], count * L * sizeof(uint32_t),
+        CUDA_TRY(cudaMemcpyAsync(out + done * L, h->graph.walks[0].get(), count * L * sizeof(uint32_t),
                                  cudaMemcpyDeviceToHost, h->walk_stream));
         CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
         done += count;
@@ -778,8 +699,8 @@ extern "C" int b2e_walks(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint
 extern "C" int b2e_device_tables(b2e_handle *h, void **table0, void **table1) {
     if (!h || !table0 || !table1) return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = require_graph(h)) return rc;
-    *table0 = h->d_t0;
-    *table1 = h->d_t1;
+    *table0 = h->graph.t0.get();
+    *table1 = h->graph.t1.get();
     return B2E_OK;
 }
 
@@ -802,8 +723,8 @@ extern "C" int b2e_exchange_handles(b2e_handle *h, void *ipc_handles) {
     if (!ipc_handles) return fail(B2E_ERR_INVALID, "null argument");
     static_assert(sizeof(cudaIpcMemHandle_t) == B2E_IPC_HANDLE_BYTES, "B2E_IPC_HANDLE_BYTES");
     cudaIpcMemHandle_t *out = static_cast<cudaIpcMemHandle_t *>(ipc_handles);
-    CUDA_TRY(cudaIpcGetMemHandle(out, h->d_t0));
-    CUDA_TRY(cudaIpcGetMemHandle(out + 1, h->d_t1));
+    CUDA_TRY(cudaIpcGetMemHandle(out, h->graph.t0.get()));
+    CUDA_TRY(cudaIpcGetMemHandle(out + 1, h->graph.t1.get()));
     return B2E_OK;
 }
 
@@ -828,8 +749,8 @@ extern "C" int b2e_exchange_open(b2e_handle *h, uint32_t world, uint32_t rank, c
     h->peers_are_ipc = true;
     for (uint32_t g = 0; g < world; ++g) {
         if (g == rank) {
-            h->peer_t0[g] = h->d_t0;
-            h->peer_t1[g] = h->d_t1;
+            h->peer_t0[g] = h->graph.t0.get();
+            h->peer_t1[g] = h->graph.t1.get();
             continue;
         }
         void *t0 = nullptr, *t1 = nullptr;
@@ -857,7 +778,7 @@ extern "C" int b2e_exchange_open_local(b2e_handle *h, uint32_t world, uint32_t r
     close_peers(h);
     for (uint32_t g = 0; g < world; ++g) {
         const b2e_handle *r = g == rank ? h : replicas[g];
-        if (!r || !r->d_t0 || r->n != h->n || r->row_stride != h->row_stride)
+        if (!r || !r->graph.t0.get() || r->n != h->n || r->row_stride != h->row_stride)
             return fail(B2E_ERR_INVALID, "every replica must hold tables of the same shape");
         if (r->cfg.device != h->cfg.device) {
             int can = 0;
@@ -873,8 +794,8 @@ extern "C" int b2e_exchange_open_local(b2e_handle *h, uint32_t world, uint32_t r
     h->rank = rank;
     for (uint32_t g = 0; g < world; ++g) {
         const b2e_handle *r = g == rank ? h : replicas[g];
-        h->peer_t0[g] = r->d_t0;
-        h->peer_t1[g] = r->d_t1;
+        h->peer_t0[g] = r->graph.t0.get();
+        h->peer_t1[g] = r->graph.t1.get();
     }
     return B2E_OK;
 }
@@ -901,15 +822,13 @@ extern "C" int b2e_tables_digest(b2e_handle *h, double *sums, uint64_t *words) {
     if (int rc = require_graph(h)) return rc;
     if (!sums || !words) return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = b2e_sync(h)) return rc;
-    void *d_out = nullptr;
-    CUDA_TRY(cudaMalloc(&d_out, 56));
-    cudaError_t e = launch_tables_digest(h->d_t0, h->d_t1, h->n, h->row_stride, h->cfg.embedding_size, d_out,
-                                         h->sm_count, h->train_stream);
+    DeviceBuffer<> d_out;
+    CUDA_TRY(d_out.reserve(56));
+    CUDA_TRY(launch_tables_digest(h->graph.t0.get(), h->graph.t1.get(), h->n, h->row_stride, h->cfg.embedding_size,
+                                  d_out.get(), h->sm_count, h->train_stream));
     unsigned char host[56];
-    if (e == cudaSuccess) e = cudaMemcpyAsync(host, d_out, 56, cudaMemcpyDeviceToHost, h->train_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->train_stream);
-    cudaFree(d_out);
-    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, std::string("b2e_tables_digest: ") + cudaGetErrorString(e));
+    CUDA_TRY(cudaMemcpyAsync(host, d_out.get(), 56, cudaMemcpyDeviceToHost, h->train_stream));
+    CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     ++h->launches;
     memcpy(sums, host, 32);
     memcpy(words, host + 32, 24);
@@ -927,38 +846,35 @@ static int export_table(b2e_handle *h, const float *d_table, float *host) {
         return B2E_OK;
     }
     const uint64_t slab_rows = std::max<uint64_t>(1, (256ull << 20) / (dim * sizeof(float)));
-    float *stage[2] = {nullptr, nullptr};
-    cudaEvent_t packed[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
-    cudaError_t e = cudaSuccess;
-    for (int b = 0; b < 2 && e == cudaSuccess; ++b) {
-        e = cudaMalloc(&stage[b], std::min<uint64_t>(slab_rows, h->n) * dim * sizeof(float));
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&packed[b], cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&copied[b], cudaEventDisableTiming);
+    struct Slabs {  // two staging buffers and their events, released on every way out
+        DeviceBuffer<float> stage[2];
+        cudaEvent_t packed[2] = {nullptr, nullptr}, copied[2] = {nullptr, nullptr};
+        ~Slabs() {
+            for (cudaEvent_t event : {packed[0], packed[1], copied[0], copied[1]})
+                if (event) cudaEventDestroy(event);
+        }
+    } s;
+    for (int b = 0; b < 2; ++b) {
+        CUDA_TRY(s.stage[b].reserve(std::min<uint64_t>(slab_rows, h->n) * dim * sizeof(float)));
+        CUDA_TRY(cudaEventCreateWithFlags(&s.packed[b], cudaEventDisableTiming));
+        CUDA_TRY(cudaEventCreateWithFlags(&s.copied[b], cudaEventDisableTiming));
     }
     uint64_t slab = 0;
-    for (uint64_t row = 0; row < h->n && e == cudaSuccess; row += slab_rows, ++slab) {
+    for (uint64_t row = 0; row < h->n; row += slab_rows, ++slab) {
         const int b = (int)(slab & 1);
         const uint64_t rows = std::min(slab_rows, h->n - row);
-        if (slab >= 2) e = cudaStreamWaitEvent(h->train_stream, copied[b], 0);  // the slab buffer is free again
-        if (e == cudaSuccess)
-            e = launch_pack_rows(d_table + row * h->row_stride, rows, h->row_stride, dim, stage[b], h->sm_count,
-                                 h->train_stream);
-        if (e == cudaSuccess) e = cudaEventRecord(packed[b], h->train_stream);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(h->walk_stream, packed[b], 0);
-        if (e == cudaSuccess)
-            e = cudaMemcpyAsync(host + row * dim, stage[b], rows * dim * sizeof(float), cudaMemcpyDeviceToHost,
-                                h->walk_stream);
-        if (e == cudaSuccess) e = cudaEventRecord(copied[b], h->walk_stream);
+        if (slab >= 2) CUDA_TRY(cudaStreamWaitEvent(h->train_stream, s.copied[b], 0));  // the slab buffer is free again
+        CUDA_TRY(launch_pack_rows(d_table + row * h->row_stride, rows, h->row_stride, dim, s.stage[b].get(),
+                                  h->sm_count, h->train_stream));
+        CUDA_TRY(cudaEventRecord(s.packed[b], h->train_stream));
+        CUDA_TRY(cudaStreamWaitEvent(h->walk_stream, s.packed[b], 0));
+        CUDA_TRY(cudaMemcpyAsync(host + row * dim, s.stage[b].get(), rows * dim * sizeof(float),
+                                 cudaMemcpyDeviceToHost, h->walk_stream));
+        CUDA_TRY(cudaEventRecord(s.copied[b], h->walk_stream));
         ++h->launches;
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->walk_stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->train_stream);
-    for (int b = 0; b < 2; ++b) {
-        cudaFree(stage[b]);
-        if (packed[b]) cudaEventDestroy(packed[b]);
-        if (copied[b]) cudaEventDestroy(copied[b]);
-    }
-    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, std::string("b2e_export_tables: ") + cudaGetErrorString(e));
+    CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+    CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     return B2E_OK;
 }
 
@@ -967,8 +883,8 @@ extern "C" int b2e_export_tables(b2e_handle *h, float *table0, float *table1) {
     if (int rc = require_graph(h)) return rc;
     if (!table0 || !table1) return fail(B2E_ERR_INVALID, "null output buffer");
     if (int rc = b2e_sync(h)) return rc;
-    if (int rc = export_table(h, h->d_t0, table0)) return rc;
-    return export_table(h, h->d_t1, table1);
+    if (int rc = export_table(h, h->graph.t0.get(), table0)) return rc;
+    return export_table(h, h->graph.t1.get(), table1);
 }
 
 extern "C" int b2e_import_tables(b2e_handle *h, const float *table0, const float *table1) {
@@ -980,12 +896,12 @@ extern "C" int b2e_import_tables(b2e_handle *h, const float *table0, const float
     const size_t pitch = h->row_stride * sizeof(float);
     // the handle's streams are non-blocking: work on the legacy default stream is not ordered
     // with them, so everything here runs on the train stream and is waited for
-    CUDA_TRY(cudaMemsetAsync(h->d_t0, 0, h->n * pitch, h->train_stream));
-    CUDA_TRY(cudaMemsetAsync(h->d_t1, 0, h->n * pitch, h->train_stream));
+    CUDA_TRY(cudaMemsetAsync(h->graph.t0.get(), 0, h->n * pitch, h->train_stream));
+    CUDA_TRY(cudaMemsetAsync(h->graph.t1.get(), 0, h->n * pitch, h->train_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
-    CUDA_TRY(cudaMemcpy2DAsync(h->d_t0, pitch, table0, width, width, h->n, cudaMemcpyHostToDevice,
+    CUDA_TRY(cudaMemcpy2DAsync(h->graph.t0.get(), pitch, table0, width, width, h->n, cudaMemcpyHostToDevice,
                                h->train_stream));
-    CUDA_TRY(cudaMemcpy2DAsync(h->d_t1, pitch, table1, width, width, h->n, cudaMemcpyHostToDevice,
+    CUDA_TRY(cudaMemcpy2DAsync(h->graph.t1.get(), pitch, table1, width, width, h->n, cudaMemcpyHostToDevice,
                                h->train_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     return B2E_OK;
@@ -993,11 +909,11 @@ extern "C" int b2e_import_tables(b2e_handle *h, const float *table0, const float
 
 extern "C" int b2e_export_alias(b2e_handle *h, uint32_t *threshold, uint32_t *alias) {
     if (!h || !threshold || !alias) return fail(B2E_ERR_INVALID, "null argument");
-    if (!h->d_alias) return fail(B2E_ERR_STATE, "no alias table (uniform negatives or no graph)");
+    if (!h->graph.alias.get()) return fail(B2E_ERR_STATE, "no alias table (uniform negatives or no graph)");
     if (h->h_alias_thr.empty()) {  // built on the device: fetched on demand (parity tests)
         CUDA_TRY(cudaSetDevice(h->cfg.device));
         std::vector<uint2> packed(h->n);
-        CUDA_TRY(cudaMemcpy(packed.data(), h->d_alias, h->n * sizeof(uint2), cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(packed.data(), h->graph.alias.get(), h->n * sizeof(uint2), cudaMemcpyDeviceToHost));
         h->h_alias_thr.resize(h->n);
         h->h_alias_idx.resize(h->n);
         for (uint64_t i = 0; i < h->n; ++i) {
@@ -1015,7 +931,7 @@ extern "C" int b2e_counters_read(b2e_handle *h, b2e_counters *out) {
     if (!out) return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = b2e_sync(h)) return rc;
     DeviceCounters c;
-    CUDA_TRY(cudaMemcpyAsync(&c, h->d_counters, sizeof(c), cudaMemcpyDeviceToHost, h->train_stream));
+    CUDA_TRY(cudaMemcpyAsync(&c, h->d_counters.get(), sizeof(c), cudaMemcpyDeviceToHost, h->train_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     out->walk_steps = c.walk_steps;
     out->walk_trials = c.walk_trials;
@@ -1033,7 +949,7 @@ extern "C" int b2e_counters_reset(b2e_handle *h) {
     if (int rc = b2e_sync(h)) return rc;
     // not cudaMemset: the legacy default stream is not ordered with the non-blocking streams of
     // the handle, and a late memset would also clear the work counter of a running SGD kernel
-    CUDA_TRY(cudaMemsetAsync(h->d_counters, 0, sizeof(DeviceCounters), h->train_stream));
+    CUDA_TRY(cudaMemsetAsync(h->d_counters.get(), 0, sizeof(DeviceCounters), h->train_stream));
     CUDA_TRY(cudaStreamSynchronize(h->train_stream));
     return B2E_OK;
 }
@@ -1047,23 +963,25 @@ extern "C" int b2e_cooccurrence(b2e_handle *h, uint64_t seed, uint64_t first_wal
     if (h->n_src == 0) return fail(B2E_ERR_INVALID, "the graph has no node with outgoing edges");
     if (int rc = b2e_sync(h)) return rc;
     const b2e_config &c = h->cfg;
-    if (!accumulate) { h->glove.n_triples = 0; h->glove.finalised = false; }
+    GloveState &g = h->graph.glove;
+    if (!accumulate) { g.n_triples = 0; g.finalised = false; }
+    std::string error;
     const uint64_t step = std::min<uint64_t>(h->chunk_cap, b2e::glove_chunk_walks(c.walk_length, c.window_size));
     for (uint64_t done = 0; done < n_walks; done += step) {
         const uint64_t count = std::min(step, n_walks - done);
-        if (h->glove.n_triples + 2ull * count * c.walk_length * c.window_size >= (1ull << 31))
+        if (g.n_triples + 2ull * count * c.walk_length * c.window_size >= (1ull << 31))
             return fail(B2E_ERR_INVALID, "more than 2^31 co-occurrence entries in flight: lower walk_length, "
                                          "window_size or iterations");
         if (int rc = walk_into(h, seed, first_walk + done * walk_id_stride, count, walk_id_stride,
-                               h->d_walks[0], h->walk_stream))
+                               h->graph.walks[0].get(), h->walk_stream))
             return rc;
-        CUDA_TRY(b2e::glove_accumulate(h->glove, h->d_walks[0], count, c.walk_length, c.window_size,
-                                       h->walk_stream));
+        if (glove_accumulate(g, h->graph.walks[0].get(), count, c.walk_length, c.window_size, h->walk_stream, error))
+            return fail(B2E_ERR_CUDA, error);
         h->launches += 2;
     }
-    CUDA_TRY(b2e::glove_finalise(h->glove, h->n, h->walk_stream));
+    if (glove_finalise(g, h->n, h->walk_stream, error)) return fail(B2E_ERR_CUDA, error);
     ++h->launches;
-    if (n_triples) *n_triples = h->glove.n_triples;
+    if (n_triples) *n_triples = g.n_triples;
     return B2E_OK;
 }
 
@@ -1071,11 +989,11 @@ extern "C" int b2e_cooccurrence_export(b2e_handle *h, uint32_t *centre, uint32_t
     REQUIRE_HANDLE(h);
     if (!centre || !context || !count) return fail(B2E_ERR_INVALID, "null output buffer");
     if (int rc = b2e_sync(h)) return rc;
-    const uint64_t m = h->glove.n_triples;
+    const uint64_t m = h->graph.glove.n_triples;
     std::vector<unsigned long long> keys(m);
-    CUDA_TRY(cudaMemcpyAsync(keys.data(), h->glove.d_keys, m * sizeof(unsigned long long),
+    CUDA_TRY(cudaMemcpyAsync(keys.data(), h->graph.glove.d_keys.get(), m * sizeof(unsigned long long),
                              cudaMemcpyDeviceToHost, h->walk_stream));
-    CUDA_TRY(cudaMemcpyAsync(count, h->glove.d_counts, m * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+    CUDA_TRY(cudaMemcpyAsync(count, h->graph.glove.d_counts.get(), m * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                              h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     for (uint64_t i = 0; i < m; ++i) {
@@ -1089,16 +1007,16 @@ extern "C" int b2e_glove_train(b2e_handle *h, float learning_rate) {
     REQUIRE_HANDLE(h);
     if (int rc = require_graph(h)) return rc;
     if (h->cfg.model != B2E_GLOVE) return fail(B2E_ERR_STATE, "the handle was not created for GloVe");
-    if (!h->glove.finalised) return fail(B2E_ERR_STATE, "b2e_cooccurrence must be called first");
+    if (!h->graph.glove.finalised) return fail(B2E_ERR_STATE, "b2e_cooccurrence must be called first");
     const b2e_config &c = h->cfg;
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     // centres in flight: like SkipGram, about one per 16 nodes on small graphs (staleness)
     const uint64_t max_warps = c.max_concurrent_walks ? c.max_concurrent_walks
                                                        : std::max<uint64_t>(16, h->n / 16);
-    CUDA_TRY(b2e::glove_train(h->glove, h->n, h->row_stride, c.embedding_size, c.glove_alpha, c.clipping_value,
-                              learning_rate, h->d_t0, h->d_t1, h->d_counters, c.deterministic != 0,
+    CUDA_TRY(glove_train(h->graph.glove, h->n, h->row_stride, c.embedding_size, c.glove_alpha, c.clipping_value,
+                              learning_rate, h->graph.t0.get(), h->graph.t1.get(), h->d_counters.get(), c.deterministic != 0,
                               h->sm_count, max_warps, h->train_stream));
-    if (h->glove.n_triples) ++h->launches;
+    if (h->graph.glove.n_triples) ++h->launches;
     return B2E_OK;
 }
 
@@ -1111,19 +1029,19 @@ extern "C" int b2e_glove_train(b2e_handle *h, float learning_rate) {
 
 // the walks of a whole epoch into HBM, and their token histogram (host copy in g.histogram)
 static int glove_walk_epoch(b2e_handle *h, uint64_t seed, uint64_t first_walk, uint64_t per_epoch) {
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     const uint32_t L = h->cfg.walk_length;
     const uint64_t tokens = per_epoch * L;
     g.histogram.clear();
-    CUDA_TRY(glove_reserve((void **)&g.d_epoch_walks, &g.epoch_walks_bytes, tokens * sizeof(uint32_t)));
-    CUDA_TRY(glove_reserve((void **)&g.d_histogram, &g.histogram_bytes, h->n * sizeof(uint32_t)));
+    CUDA_TRY(g.d_epoch_walks.reserve(tokens * sizeof(uint32_t)));
+    CUDA_TRY(g.d_histogram.reserve(h->n * sizeof(uint32_t)));
     for (uint64_t done = 0; done < per_epoch; done += h->chunk_cap) {
         const uint64_t count = std::min(h->chunk_cap, per_epoch - done);
-        if (int rc = walk_into(h, seed, first_walk + done, count, 1, g.d_epoch_walks + done * L, h->walk_stream)) return rc;
+        if (int rc = walk_into(h, seed, first_walk + done, count, 1, g.d_epoch_walks.get() + done * L, h->walk_stream)) return rc;
     }
-    CUDA_TRY(glove_token_histogram(g.d_epoch_walks, tokens, g.d_histogram, h->n, h->walk_stream));
+    CUDA_TRY(glove_token_histogram(g.d_epoch_walks.get(), tokens, g.d_histogram.get(), h->n, h->walk_stream));
     std::vector<uint32_t> histogram(h->n);
-    CUDA_TRY(cudaMemcpyAsync(histogram.data(), g.d_histogram, h->n * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+    CUDA_TRY(cudaMemcpyAsync(histogram.data(), g.d_histogram.get(), h->n * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                              h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     h->launches += 2;
@@ -1136,7 +1054,7 @@ static int glove_walk_epoch(b2e_handle *h, uint64_t seed, uint64_t first_walk, u
 // may exceed it) and bucket the positions of their tokens by range (tokens of other centres are
 // skipped).
 static int glove_bucket_ranges(b2e_handle *h, uint32_t lo, uint32_t hi, uint64_t capacity_slots) {
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     const uint32_t W = h->cfg.window_size;
     std::vector<uint32_t> bounds(1, lo);
     std::vector<unsigned long long> offsets(1, 0ull);
@@ -1159,12 +1077,12 @@ static int glove_bucket_ranges(b2e_handle *h, uint32_t lo, uint32_t hi, uint64_t
     const uint32_t ranges = (uint32_t)bounds.size() - 1u;
     g.last_ranges = ranges;
     g.range_kept = false;
-    CUDA_TRY(glove_reserve((void **)&g.d_bounds, &g.bounds_bytes, bounds.size() * sizeof(uint32_t)));
-    CUDA_TRY(glove_reserve((void **)&g.d_cursor, &g.cursor_bytes, ranges * sizeof(unsigned long long)));
-    CUDA_TRY(glove_reserve((void **)&g.d_positions, &g.positions_bytes, std::max<uint64_t>(placed, 1) * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemcpyAsync(g.d_bounds, bounds.data(), bounds.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->walk_stream));
-    CUDA_TRY(cudaMemcpyAsync(g.d_cursor, offsets.data(), ranges * sizeof(unsigned long long), cudaMemcpyHostToDevice, h->walk_stream));
-    CUDA_TRY(glove_bucket_positions(g.d_epoch_walks, g.epoch_tokens, g.d_bounds, ranges, g.d_cursor, g.d_positions,
+    CUDA_TRY(g.d_bounds.reserve(bounds.size() * sizeof(uint32_t)));
+    CUDA_TRY(g.d_cursor.reserve(ranges * sizeof(unsigned long long)));
+    CUDA_TRY(g.d_positions.reserve(std::max<uint64_t>(placed, 1) * sizeof(unsigned long long)));
+    CUDA_TRY(cudaMemcpyAsync(g.d_bounds.get(), bounds.data(), bounds.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->walk_stream));
+    CUDA_TRY(cudaMemcpyAsync(g.d_cursor.get(), offsets.data(), ranges * sizeof(unsigned long long), cudaMemcpyHostToDevice, h->walk_stream));
+    CUDA_TRY(glove_bucket_positions(g.d_epoch_walks.get(), g.epoch_tokens, g.d_bounds.get(), ranges, g.d_cursor.get(), g.d_positions.get(),
                                     h->walk_stream));
     CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
     ++h->launches;
@@ -1174,23 +1092,26 @@ static int glove_bucket_ranges(b2e_handle *h, uint32_t lo, uint32_t hi, uint64_t
 }
 
 static int glove_count_range(b2e_handle *h, uint32_t r) {
-    GloveState &g = h->glove;
-    CUDA_TRY(glove_range_triples(g, g.d_epoch_walks, h->cfg.walk_length, h->cfg.window_size,
-                                 g.d_positions + g.range_offsets[r], g.range_offsets[r + 1] - g.range_offsets[r],
-                                 h->walk_stream));
+    GloveState &g = h->graph.glove;
+    std::string error;
+    if (glove_range_triples(g, g.d_epoch_walks.get(), h->cfg.walk_length, h->cfg.window_size,
+                            g.d_positions.get() + g.range_offsets[r], g.range_offsets[r + 1] - g.range_offsets[r],
+                            h->walk_stream, error))
+        return fail(B2E_ERR_CUDA, error);
     h->launches += 2;
     return B2E_OK;
 }
 
 // the largest count of the bucketed ranges (0 without triples); a single range keeps its triples
 static int glove_count_ranges(b2e_handle *h, uint32_t *largest) {
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     const uint32_t ranges = (uint32_t)g.range_bounds.size() - 1u;
     *largest = 0;
+    std::string error;
     for (uint32_t r = 0; r < ranges; ++r) {
         if (int rc = glove_count_range(h, r)) return rc;
         uint32_t local = 0;
-        CUDA_TRY(glove_max_count(g, &local, h->walk_stream));
+        if (glove_max_count(g, &local, h->walk_stream, error)) return fail(B2E_ERR_CUDA, error);
         *largest = std::max(*largest, local);
     }
     g.range_kept = ranges == 1;
@@ -1199,13 +1120,14 @@ static int glove_count_ranges(b2e_handle *h, uint32_t *largest) {
 
 // one SGD pass over the bucketed ranges in ascending order of centre, weights against x_max
 static int glove_train_ranges(b2e_handle *h, float lr, uint32_t x_max) {
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     const uint32_t ranges = (uint32_t)g.range_bounds.size() - 1u;
+    std::string error;
     for (uint32_t r = 0; r < ranges; ++r) {
         if (!g.range_kept)
             if (int rc = glove_count_range(h, r)) return rc;
         if (g.n_triples == 0) continue;
-        CUDA_TRY(glove_finalise(g, h->n, h->walk_stream));
+        if (glove_finalise(g, h->n, h->walk_stream, error)) return fail(B2E_ERR_CUDA, error);
         g.max_count = x_max;
         if (int rc = b2e_glove_train(h, lr)) return rc;
         CUDA_TRY(cudaStreamSynchronize(h->train_stream));  // the triples are replaced by the next range
@@ -1266,7 +1188,7 @@ extern "C" int b2e_glove_shard_count(b2e_handle *h, uint32_t world, uint32_t ran
     if (int rc = require_glove(h)) return rc;
     if (int rc = check_world(world, rank)) return rc;
     if (!local_max) return fail(B2E_ERR_INVALID, "null argument");
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     if (g.histogram.size() != h->n) return fail(B2E_ERR_STATE, "b2e_glove_walk_epoch must be called first");
     if (int rc = b2e_sync(h)) return rc;
     glove_owner_bounds(g.histogram, h->cfg.window_size, world, g.owner_bounds);
@@ -1279,13 +1201,13 @@ extern "C" int b2e_glove_shard_count(b2e_handle *h, uint32_t world, uint32_t ran
 extern "C" int b2e_glove_shard_train(b2e_handle *h, float learning_rate, uint32_t max_count) {
     REQUIRE_HANDLE(h);
     if (int rc = require_glove(h)) return rc;
-    GloveState &g = h->glove;
+    GloveState &g = h->graph.glove;
     if (g.owner_world == 0 || g.range_bounds.empty())
         return fail(B2E_ERR_STATE, "b2e_glove_shard_count must be called first");
     if (g.owner_world > 1) {  // the base of the merge: T1 before this epoch's training (same stream, ordered)
         const size_t bytes = h->n * (size_t)h->row_stride * sizeof(float);
-        CUDA_TRY(glove_reserve((void **)&g.d_t1_snapshot, &g.t1_snapshot_bytes, bytes));
-        CUDA_TRY(cudaMemcpyAsync(g.d_t1_snapshot, h->d_t1, bytes, cudaMemcpyDeviceToDevice, h->train_stream));
+        CUDA_TRY(g.d_t1_snapshot.reserve(bytes));
+        CUDA_TRY(cudaMemcpyAsync(g.d_t1_snapshot.get(), h->graph.t1.get(), bytes, cudaMemcpyDeviceToDevice, h->train_stream));
     }
     const int rc = glove_train_ranges(h, learning_rate, std::max(max_count, 1u));
     g.range_bounds.clear();  // trained: the next epoch counts anew
@@ -1296,11 +1218,11 @@ extern "C" int b2e_glove_merge(b2e_handle *h) {
     REQUIRE_HANDLE(h);
     if (int rc = require_glove(h)) return rc;
     if (h->world < 2) return B2E_OK;
-    GloveState &g = h->glove;
-    if (g.owner_world != h->world || !g.d_t1_snapshot)
+    GloveState &g = h->graph.glove;
+    if (g.owner_world != h->world || !g.d_t1_snapshot.get())
         return fail(B2E_ERR_STATE, "b2e_glove_shard_count and b2e_glove_shard_train with the world of the exchange "
                                    "must come first");
-    CUDA_TRY(launch_glove_merge(h->peer_t0, h->peer_t1, g.d_t1_snapshot, g.owner_bounds, h->world, h->rank, h->n,
+    CUDA_TRY(launch_glove_merge(h->peer_t0, h->peer_t1, g.d_t1_snapshot.get(), g.owner_bounds, h->world, h->rank, h->n,
                                 h->row_stride, (h->cfg.embedding_size + 3u) / 4u, h->sm_count, h->train_stream));
     ++h->launches;
     return B2E_OK;
@@ -1375,8 +1297,6 @@ extern "C" int b2e_fit(b2e_handle *h, uint64_t seed, float *table0, float *table
     return b2e_export_tables(h, table0, table1);
 }
 
-static int select_device(int device);
-
 // ---- resident graphs: built on the GPU, handed to a handle without leaving HBM ----
 // a host CSR uploaded once, to be shared by several handles (b2e_load_graph checks its contents)
 extern "C" int b2e_graph_from_csr(int device, const int64_t *indptr, const uint32_t *indices, uint64_t n,
@@ -1388,20 +1308,16 @@ extern "C" int b2e_graph_from_csr(int device, const int64_t *indptr, const uint3
     for (uint64_t v = 0; v < n; ++v)
         if (indptr[v + 1] < indptr[v]) return fail(B2E_ERR_INVALID, "indptr must be non-decreasing");
     if (int rc = select_device(device)) return rc;
-    b2e_graph *g = new (std::nothrow) b2e_graph();
+    std::unique_ptr<b2e_graph, GraphRelease> g(new (std::nothrow) b2e_graph());
     if (!g) return fail(B2E_ERR_INVALID, "out of host memory");
     g->device = device;
     g->csr.n = n;
     g->csr.nnz = nnz;
-    cudaError_t e = cudaMalloc(&g->csr.indptr, (n + 1) * sizeof(int64_t));
-    if (e == cudaSuccess) e = cudaMalloc(&g->csr.indices, std::max<uint64_t>(nnz, 1) * sizeof(uint32_t));
-    if (e == cudaSuccess) e = cudaMemcpy(g->csr.indptr, indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && nnz) e = cudaMemcpy(g->csr.indices, indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        release_graph(g);
-        return fail(B2E_ERR_CUDA, std::string("b2e_graph_from_csr: ") + cudaGetErrorString(e));
-    }
-    *out = g;
+    CUDA_TRY(g->csr.indptr.reserve((n + 1) * sizeof(int64_t)));
+    CUDA_TRY(g->csr.indices.reserve(std::max<uint64_t>(nnz, 1) * sizeof(uint32_t)));
+    CUDA_TRY(cudaMemcpy(g->csr.indptr.get(), indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
+    if (nnz) CUDA_TRY(cudaMemcpy(g->csr.indices.get(), indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    *out = g.release();
     return B2E_OK;
 }
 
@@ -1415,9 +1331,9 @@ extern "C" int b2e_graph_shape(const b2e_graph *g, uint64_t *n, uint64_t *nnz) {
 extern "C" int b2e_graph_export(const b2e_graph *g, int64_t *indptr, uint32_t *indices) {
     if (!g || !indptr || (!indices && g->csr.nnz)) return fail(B2E_ERR_INVALID, "null argument");
     CUDA_TRY(cudaSetDevice(g->device));
-    CUDA_TRY(cudaMemcpy(indptr, g->csr.indptr, (g->csr.n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(indptr, g->csr.indptr.get(), (g->csr.n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost));
     if (g->csr.nnz)
-        CUDA_TRY(cudaMemcpy(indices, g->csr.indices, g->csr.nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(indices, g->csr.indices.get(), g->csr.nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return B2E_OK;
 }
 
@@ -1439,9 +1355,9 @@ extern "C" int b2e_load_graph(b2e_handle *h, b2e_graph *g) {
     const double alpha = (double)h->cfg.negative_sampling_exponent;
     if (h->cfg.use_scale_free_distribution && alpha != 0.0 && alpha != 0.5 && alpha != 0.75 && alpha != 1.0) {
         indptr.resize(g->csr.n + 1);
-        CUDA_TRY(cudaMemcpy(indptr.data(), g->csr.indptr, indptr.size() * sizeof(int64_t), cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(indptr.data(), g->csr.indptr.get(), indptr.size() * sizeof(int64_t), cudaMemcpyDeviceToHost));
     }
-    ++g->references;  // keep it alive across free_graph() of a handle that already walks on it
+    ++g->references;  // keep it alive across drop_graph() of a handle that already walks on it
     const int rc = load_graph_common(h, indptr.empty() ? nullptr : indptr.data(), nullptr, nullptr, g->csr.n,
                                      g->csr.nnz, g);
     release_graph(g);
@@ -1449,37 +1365,47 @@ extern "C" int b2e_load_graph(b2e_handle *h, b2e_graph *g) {
 }
 
 // ---- graph ingest (csrc/graph_build.cu) ----
-static int select_device(int device) {
-    int count = 0;
-    cudaError_t e = cudaGetDeviceCount(&count);
-    if (e != cudaSuccess || count == 0)
-        return fail(B2E_ERR_CUDA, std::string("no CUDA device available (there is no CPU fallback): ") +
-                                      cudaGetErrorString(e));
-    if (device < 0 || device >= count) return fail(B2E_ERR_INVALID, "device ordinal out of range");
-    CUDA_TRY(cudaSetDevice(device));
+// the status of an ingest call: cudaErrorInvalidValue marks bad input, named in `error`
+static int ingest_status(cudaError_t e, const std::string &error) {
+    if (e == cudaErrorInvalidValue) return fail(B2E_ERR_INVALID, error);
+    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, error);
     return B2E_OK;
 }
 
 static int deliver_graph(int device, cudaError_t e, const std::string &error, ResidentCsr &csr, b2e_graph **out) {
-    if (e == cudaErrorInvalidValue) return fail(B2E_ERR_INVALID, error);
-    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, error);
+    if (int rc = ingest_status(e, error)) return rc;
     b2e_graph *g = new (std::nothrow) b2e_graph();
-    if (!g) {
-        cudaFree(csr.indptr);
-        cudaFree(csr.indices);
-        return fail(B2E_ERR_INVALID, "out of host memory");
-    }
-    g->csr = csr;
+    if (!g) return fail(B2E_ERR_INVALID, "out of host memory");
+    g->csr = std::move(csr);
     g->device = device;
     *out = g;
     return B2E_OK;
 }
 
-extern "C" int b2e_graph_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
-                                    uint64_t n_nodes, int symmetrise, b2e_graph **out) {
-    if (!out || (n_edges && (!src || !dst))) return fail(B2E_ERR_INVALID, "null argument");
+// the checks b2e_graph_from_edges and b2e_csr_from_edges share, after their own output arguments
+static int check_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_edges, uint64_t n_nodes) {
+    if (n_edges && (!src || !dst)) return fail(B2E_ERR_INVALID, "null argument");
     if (n_nodes == 0 || n_nodes >= 0xFFFFFF00ull)
         return fail(B2E_ERR_INVALID, "the number of nodes must be in [1, 0xFFFFFF00)");
+    return B2E_OK;
+}
+
+// the checks b2e_graph_synthetic and b2e_synthetic_csr share, after their own output arguments
+static int check_synthetic(int kind, uint64_t n_nodes, uint32_t scale, uint64_t n_edges) {
+    if (kind != 0 && kind != 1) return fail(B2E_ERR_INVALID, "kind must be 0 (Erdos-Renyi) or 1 (R-MAT)");
+    if (n_nodes < 2 || n_nodes >= 0xFFFFFF00ull)
+        return fail(B2E_ERR_INVALID, "the number of nodes must be in [2, 0xFFFFFF00)");
+    if (kind == 1 && (scale == 0 || scale > 32 || (scale < 32 && n_nodes > (1ull << scale))))
+        return fail(B2E_ERR_INVALID, "R-MAT needs 1 <= scale <= 32 and n_nodes <= 2^scale");
+    if ((double)n_edges > 0.5 * (double)n_nodes * (double)(n_nodes - 1) * 0.5)
+        return fail(B2E_ERR_INVALID, "Too many edges requested.");
+    return B2E_OK;
+}
+
+extern "C" int b2e_graph_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
+                                    uint64_t n_nodes, int symmetrise, b2e_graph **out) {
+    if (!out) return fail(B2E_ERR_INVALID, "null argument");
+    if (int rc = check_edges(src, dst, n_edges, n_nodes)) return rc;
     if (int rc = select_device(device)) return rc;
     std::string error;
     ResidentCsr csr;
@@ -1491,13 +1417,7 @@ extern "C" int b2e_graph_from_edges(int device, const uint32_t *src, const uint3
 extern "C" int b2e_graph_synthetic(int device, int kind, uint64_t n_nodes, uint32_t scale, uint64_t n_edges,
                                    uint64_t seed, uint64_t t_a, uint64_t t_ab, uint64_t t_abc, b2e_graph **out) {
     if (!out) return fail(B2E_ERR_INVALID, "null argument");
-    if (kind != 0 && kind != 1) return fail(B2E_ERR_INVALID, "kind must be 0 (Erdos-Renyi) or 1 (R-MAT)");
-    if (n_nodes < 2 || n_nodes >= 0xFFFFFF00ull)
-        return fail(B2E_ERR_INVALID, "the number of nodes must be in [2, 0xFFFFFF00)");
-    if (kind == 1 && (scale == 0 || scale > 32 || (scale < 32 && n_nodes > (1ull << scale))))
-        return fail(B2E_ERR_INVALID, "R-MAT needs 1 <= scale <= 32 and n_nodes <= 2^scale");
-    if ((double)n_edges > 0.5 * (double)n_nodes * (double)(n_nodes - 1) * 0.5)
-        return fail(B2E_ERR_INVALID, "Too many edges requested.");
+    if (int rc = check_synthetic(kind, n_nodes, scale, n_edges)) return rc;
     if (int rc = select_device(device)) return rc;
     std::string error;
     ResidentCsr csr;
@@ -1510,17 +1430,13 @@ extern "C" int b2e_graph_synthetic(int device, int kind, uint64_t n_nodes, uint3
 extern "C" int b2e_csr_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
                                   uint64_t n_nodes, int symmetrise, int64_t *indptr, uint32_t *indices,
                                   uint64_t indices_capacity, uint64_t *nnz) {
-    if (!indptr || !nnz || (n_edges && (!src || !dst || !indices)))
-        return fail(B2E_ERR_INVALID, "null argument");
-    if (n_nodes == 0 || n_nodes >= 0xFFFFFF00ull)
-        return fail(B2E_ERR_INVALID, "the number of nodes must be in [1, 0xFFFFFF00)");
+    if (!indptr || !nnz || (n_edges && !indices)) return fail(B2E_ERR_INVALID, "null argument");
+    if (int rc = check_edges(src, dst, n_edges, n_nodes)) return rc;
     if (int rc = select_device(device)) return rc;
     std::string error;
     cudaError_t e = csr_from_edges(src, dst, n_edges, n_nodes, symmetrise, indptr, indices,
                                    indices_capacity, nnz, error);
-    if (e == cudaErrorInvalidValue) return fail(B2E_ERR_INVALID, error);
-    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, error);
-    return B2E_OK;
+    return ingest_status(e, error);
 }
 
 extern "C" int b2e_synthetic_csr(int device, int kind, uint64_t n_nodes, uint32_t scale, uint64_t n_edges,
@@ -1528,19 +1444,11 @@ extern "C" int b2e_synthetic_csr(int device, int kind, uint64_t n_nodes, uint32_
                                  int64_t *indptr, uint32_t *indices, uint64_t indices_capacity,
                                  uint64_t *nnz) {
     if (!indptr || !indices || !nnz) return fail(B2E_ERR_INVALID, "null argument");
-    if (kind != 0 && kind != 1) return fail(B2E_ERR_INVALID, "kind must be 0 (Erdos-Renyi) or 1 (R-MAT)");
-    if (n_nodes < 2 || n_nodes >= 0xFFFFFF00ull)
-        return fail(B2E_ERR_INVALID, "the number of nodes must be in [2, 0xFFFFFF00)");
-    if (kind == 1 && (scale == 0 || scale > 32 || (scale < 32 && n_nodes > (1ull << scale))))
-        return fail(B2E_ERR_INVALID, "R-MAT needs 1 <= scale <= 32 and n_nodes <= 2^scale");
-    if ((double)n_edges > 0.5 * (double)n_nodes * (double)(n_nodes - 1) * 0.5)
-        return fail(B2E_ERR_INVALID, "Too many edges requested.");
+    if (int rc = check_synthetic(kind, n_nodes, scale, n_edges)) return rc;
     if (indices_capacity < 2 * n_edges) return fail(B2E_ERR_INVALID, "indices_capacity must be >= 2 * n_edges");
     if (int rc = select_device(device)) return rc;
     std::string error;
     cudaError_t e = synthetic_csr(kind, n_nodes, scale, n_edges, seed, t_a, t_ab, t_abc, indptr, indices,
                                   indices_capacity, nnz, error);
-    if (e == cudaErrorInvalidValue) return fail(B2E_ERR_INVALID, error);
-    if (e != cudaSuccess) return fail(B2E_ERR_CUDA, error);
-    return B2E_OK;
+    return ingest_status(e, error);
 }

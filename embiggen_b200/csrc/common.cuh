@@ -89,54 +89,6 @@ struct TrainParams {
 };
 
 cudaError_t launch_walks(const WalkParams &p, bool second_order, cudaStream_t stream);
-// GloVe (glove.cu): the co-occurrence triples of an epoch, sorted by (centre << 32 | context)
-struct GloveState {
-    unsigned long long *d_keys = nullptr;
-    uint32_t *d_counts = nullptr;
-    uint64_t *d_rowptr = nullptr;
-    uint64_t n_triples = 0;
-    uint32_t max_count = 1;
-    bool finalised = false;
-    size_t keys_bytes = 0, counts_bytes = 0, rowptr_bytes = 0;
-    unsigned long long *d_scratch_keys = nullptr, *d_merge_keys = nullptr;
-    uint32_t *d_merge_counts = nullptr;
-    void *d_temp = nullptr, *d_scalar = nullptr;
-    size_t scratch_keys_bytes = 0, merge_keys_bytes = 0, merge_counts_bytes = 0, temp_bytes = 0, scalar_bytes = 0;
-    // co-occurrence by centre range: the walks of an epoch, their token positions bucketed by range
-    uint32_t *d_epoch_walks = nullptr, *d_histogram = nullptr, *d_bounds = nullptr;
-    unsigned long long *d_positions = nullptr, *d_cursor = nullptr;
-    size_t epoch_walks_bytes = 0, histogram_bytes = 0, bounds_bytes = 0, positions_bytes = 0, cursor_bytes = 0;
-    uint32_t last_ranges = 0;  // how many centre ranges the last epoch took (1 = one piece)
-    uint64_t epoch_tokens = 0;                    // tokens of the walked epoch (d_epoch_walks)
-    std::vector<uint32_t> histogram;              // tokens per node of the walked epoch (host copy)
-    std::vector<uint32_t> range_bounds;           // range r: range_bounds[r] <= centre < range_bounds[r + 1]
-    std::vector<unsigned long long> range_offsets;  // bucketed occurrences before range r
-    bool range_kept = false;                      // one range: its triples are resident, counted once
-    // sharded epoch (several GPUs): rank r owns the centres [owner_bounds[r], owner_bounds[r + 1])
-    uint32_t owner_world = 0, owner_bounds[B2E_MAX_WORLD + 1] = {0};
-    float *d_t1_snapshot = nullptr;  // T1 as it stood before this epoch's training (the merge's base)
-    size_t t1_snapshot_bytes = 0;
-};
-uint64_t glove_chunk_walks(uint32_t walk_length, uint32_t window);
-cudaError_t glove_accumulate(GloveState &g, const uint32_t *d_walks, uint64_t n_walks, uint32_t walk_length,
-                             uint32_t window, cudaStream_t stream);
-cudaError_t glove_finalise(GloveState &g, uint64_t n, cudaStream_t stream);
-cudaError_t glove_train(const GloveState &g, uint64_t n, uint32_t row_stride, uint32_t embedding_size,
-                        float alpha, float clip, float lr, float *t0, float *t1, DeviceCounters *counters,
-                        bool deterministic, int sm_count, uint64_t max_warps, cudaStream_t stream);
-// co-occurrence by centre range (glove.cu): histogram of the epoch's tokens, occurrences bucketed
-// by range, the triples of one range
-cudaError_t glove_token_histogram(const uint32_t *d_walks, uint64_t tokens, uint32_t *d_histogram, uint64_t n,
-                                  cudaStream_t stream);
-cudaError_t glove_bucket_positions(const uint32_t *d_walks, uint64_t tokens, const uint32_t *d_bounds, uint32_t ranges,
-                                   unsigned long long *d_cursor, unsigned long long *d_positions,
-                                   cudaStream_t stream);
-cudaError_t glove_range_triples(GloveState &g, const uint32_t *d_walks, uint32_t L, uint32_t W,
-                                const unsigned long long *d_positions, uint64_t count, cudaStream_t stream);
-cudaError_t glove_reserve(void **ptr, size_t *have, size_t want);
-cudaError_t glove_max_count(GloveState &g, uint32_t *max_count, cudaStream_t stream);
-void glove_free(GloveState &g);
-
 cudaError_t launch_walklet_split(const uint32_t *raw, uint64_t n_walks, uint32_t walk_length, uint32_t scale,
                                  uint32_t *out, cudaStream_t stream);
 cudaError_t launch_symmetry_check(const int64_t *indptr, const uint32_t *indices, uint64_t n,
@@ -175,62 +127,4 @@ bool shared_negatives_supported(const TrainParams &p);
 cudaError_t launch_train_pipe(const TrainParams &p, uint32_t model, bool deterministic, int sm_count,
                               uint64_t max_warps, cudaStream_t stream);
 
-// a CSR that stays in HBM (b2e_graph): built by graph_build.cu, handed to a handle without a copy
-struct ResidentCsr {
-    int64_t *indptr = nullptr;
-    uint32_t *indices = nullptr;
-    uint64_t n = 0, nnz = 0;
-};
-// `resident` != nullptr: the device arrays move into it and the host buffers are not touched
-cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_edges, uint64_t n,
-                           int symmetrise, int64_t *indptr, uint32_t *indices, uint64_t capacity,
-                           uint64_t *nnz_out, std::string &error, ResidentCsr *resident = nullptr);
-cudaError_t synthetic_csr(int kind, uint64_t n, uint32_t scale, uint64_t m, uint64_t seed,
-                          unsigned long long t_a, unsigned long long t_ab, unsigned long long t_abc,
-                          int64_t *indptr, uint32_t *indices, uint64_t capacity, uint64_t *nnz_out,
-                          std::string &error, ResidentCsr *resident = nullptr);
-
 }  // namespace b2e
-
-struct b2e_graph {
-    b2e::ResidentCsr csr;
-    int device = 0;
-    int references = 1;  // the caller's object + every handle that walks on it
-};
-
-struct b2e_handle {
-    b2e_config cfg;
-    b2e_graph *shared_graph = nullptr;  // d_indptr / d_indices belong to it (b2e_load_graph)
-    int sm_count = 0;
-    uint64_t n = 0, nnz = 0, n_src = 0;
-    uint32_t row_stride = 0;
-    int64_t *d_indptr = nullptr;
-    uint32_t *d_indices = nullptr;
-    uint2 *d_edge_alias = nullptr;
-    uint32_t *d_node_types = nullptr, *d_edge_types = nullptr;
-    b2e::GloveState glove;
-    uint32_t *d_walk_raw = nullptr;  // Walklets: the chunk as walked, before it is split by stride
-    uint32_t max_degree = 0;
-    uint32_t *d_sources = nullptr;
-    unsigned long long *d_filter = nullptr;  // row filters of the adjacency check (second-order walks)
-    uint64_t fold_excess = 0;                // see WalkParams
-    unsigned long long thr_fold[3] = {0, 0, 0};
-    uint2 *d_alias = nullptr;
-    float *d_t0 = nullptr, *d_t1 = nullptr;
-    uint32_t *d_walks[2] = {nullptr, nullptr};
-    uint64_t chunk_cap = 0;
-    uint64_t slot_first[2] = {0, 0}, slot_count[2] = {0, 0}, slot_stride[2] = {1, 1};
-    cudaEvent_t walk_done[2] = {nullptr, nullptr}, train_done[2] = {nullptr, nullptr};
-    cudaStream_t walk_stream = nullptr, train_stream = nullptr;
-    bool own_streams = false;
-    b2e::DeviceCounters *d_counters = nullptr;
-    unsigned long long thr[3] = {0, 0, 0};
-    bool second_order = false;
-    bool undirected = false;
-    uint64_t launches = 0;
-    std::vector<uint32_t> h_alias_thr, h_alias_idx;
-    // the exchange step: replicas of the tables on the other GPUs of the node
-    uint32_t world = 1, rank = 0;
-    float *peer_t0[B2E_MAX_WORLD] = {nullptr}, *peer_t1[B2E_MAX_WORLD] = {nullptr};
-    bool peers_are_ipc = false;
-};

@@ -21,7 +21,7 @@
 #include <string>
 #include <vector>
 
-#include "common.cuh"
+#include "host.cuh"
 
 namespace b2e {
 
@@ -486,56 +486,43 @@ using namespace b2e;
 
 struct b2e_features {
     int device = 0;
-    float *d = nullptr;
+    DeviceBuffer<float> owned;  // the table of b2e_features_create; empty for a view of a handle's table
+    const float *d = nullptr;
     uint64_t n = 0, pitch = 0;
     uint32_t dim = 0;
-    bool owned = true;
 };
-
-int b2e_set_error(int status, const std::string &message);  // b2e_api.cu
-
-#define EP_TRY(call)                                                                          \
-    do {                                                                                      \
-        cudaError_t e_ = (call);                                                              \
-        if (e_ != cudaSuccess)                                                                \
-            return b2e_set_error(B2E_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
-    } while (0)
 
 static int build_methods(const uint32_t *ids, uint32_t count, uint32_t dim, const uint32_t *metrics,
                          uint32_t n_metrics, MethodList &out) {
     if (count > MAX_METHODS || n_metrics > MAX_METRICS || (count && !ids) || (n_metrics && !metrics))
-        return b2e_set_error(B2E_ERR_INVALID, "at most 12 edge embedding methods and 5 edge features");
+        return fail(B2E_ERR_INVALID, "at most 12 edge embedding methods and 5 edge features");
     if (count + n_metrics == 0)
-        return b2e_set_error(B2E_ERR_INVALID, "at least one edge embedding method or edge feature is required");
+        return fail(B2E_ERR_INVALID, "at least one edge embedding method or edge feature is required");
     out.n = count;
     out.n_metrics = n_metrics;
     out.size = 0;
     for (uint32_t k = 0; k < count; ++k) {
-        if (ids[k] > B2E_EDGE_COSINE_SIMILARITY) return b2e_set_error(B2E_ERR_INVALID, "unknown edge embedding method");
+        if (ids[k] > B2E_EDGE_COSINE_SIMILARITY) return fail(B2E_ERR_INVALID, "unknown edge embedding method");
         out.id[k] = ids[k];
         out.offset[k] = out.size;
         out.size += method_width(ids[k], dim);
     }
     for (uint32_t k = 0; k < n_metrics; ++k) {
         if (metrics[k] > B2E_EDGE_FEATURE_PREFERENTIAL_ATTACHMENT)
-            return b2e_set_error(B2E_ERR_INVALID, "unknown edge feature");
+            return fail(B2E_ERR_INVALID, "unknown edge feature");
         out.metric_id[k] = metrics[k];
         out.metric_offset[k] = out.size;
         out.size += metrics[k] == B2E_EDGE_FEATURE_DEGREE ? 2u : 1u;
     }
     if ((out.size + 1) * 2 * sizeof(float) > 200 * 1024)
-        return b2e_set_error(B2E_ERR_INVALID, "edge embedding too wide for the perceptron kernels");
+        return fail(B2E_ERR_INVALID, "edge embedding too wide for the perceptron kernels");
     return B2E_OK;
 }
 
-
-
-struct DeviceArray {
-    void *p = nullptr;
-    ~DeviceArray() { cudaFree(p); }
-    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, std::max<size_t>(bytes, 16)); }
-    template <typename T> T *as() { return static_cast<T *>(p); }
-};
+// every upload holds at least 16 bytes
+template <typename T> static cudaError_t alloc(DeviceBuffer<T> &buffer, size_t bytes) {
+    return buffer.reserve(std::max<size_t>(bytes, 16));
+}
 
 // the support graph of the topological features, uploaded for the duration of a call
 // ids in range and rows strictly ascending (walk_kernels.cu: csr_check_kernel): the common-neighbour
@@ -543,106 +530,98 @@ struct DeviceArray {
 static int check_csr_contents(const int64_t *h_indptr, const int64_t *d_indptr, const uint32_t *d_indices,
                               uint64_t n) {
     for (uint64_t v = 0; v < n; ++v)
-        if (h_indptr[v + 1] < h_indptr[v]) return b2e_set_error(B2E_ERR_INVALID, "indptr must be non-decreasing");
-    int *d_flags = nullptr, flags = 0;
-    EP_TRY(cudaMalloc(&d_flags, sizeof(int)));
-    cudaError_t e = cudaMemset(d_flags, 0, sizeof(int));
-    if (e == cudaSuccess) e = launch_csr_check(d_indptr, d_indices, n, d_flags, 148, 0);
-    if (e == cudaSuccess) e = cudaMemcpy(&flags, d_flags, sizeof(int), cudaMemcpyDeviceToHost);
-    cudaFree(d_flags);
-    EP_TRY(e);
-    if (flags & 1) return b2e_set_error(B2E_ERR_INVALID, "a destination node id is out of range");
+        if (h_indptr[v + 1] < h_indptr[v]) return fail(B2E_ERR_INVALID, "indptr must be non-decreasing");
+    DeviceBuffer<int> d_flags;
+    int flags = 0;
+    CUDA_TRY(d_flags.reserve(sizeof(int)));
+    CUDA_TRY(cudaMemset(d_flags.get(), 0, sizeof(int)));
+    CUDA_TRY(launch_csr_check(d_indptr, d_indices, n, d_flags.get(), 148, 0));
+    CUDA_TRY(cudaMemcpy(&flags, d_flags.get(), sizeof(int), cudaMemcpyDeviceToHost));
+    if (flags & 1) return fail(B2E_ERR_INVALID, "a destination node id is out of range");
     if (flags & 2)
-        return b2e_set_error(B2E_ERR_INVALID, "neighbour lists must be sorted strictly ascending within each row");
+        return fail(B2E_ERR_INVALID, "neighbour lists must be sorted strictly ascending within each row");
     return B2E_OK;
 }
 
 struct DeviceGraph {
-    DeviceArray indptr, indices;
+    DeviceBuffer<int64_t> indptr;
+    DeviceBuffer<uint32_t> indices;
     GraphView view = {nullptr, nullptr, 0.f};
     int upload(const int64_t *h_indptr, const uint32_t *h_indices, uint64_t n, uint64_t nnz) {
         if (!h_indptr || (!h_indices && nnz) || h_indptr[0] != 0 || (uint64_t)h_indptr[n] != nnz)
-            return b2e_set_error(B2E_ERR_INVALID, "the edge features need the support graph's CSR");
+            return fail(B2E_ERR_INVALID, "the edge features need the support graph's CSR");
         int64_t max_degree = 1;
         for (uint64_t v = 0; v < n; ++v) max_degree = std::max(max_degree, h_indptr[v + 1] - h_indptr[v]);
-        EP_TRY(indptr.alloc((n + 1) * sizeof(int64_t)));
-        EP_TRY(indices.alloc(nnz * sizeof(uint32_t)));
-        EP_TRY(cudaMemcpy(indptr.p, h_indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
-        EP_TRY(cudaMemcpy(indices.p, h_indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
-        if (int rc = check_csr_contents(h_indptr, indptr.as<int64_t>(), indices.as<uint32_t>(), n)) return rc;
-        view.indptr = indptr.as<int64_t>();
-        view.indices = indices.as<uint32_t>();
+        CUDA_TRY(alloc(indptr, (n + 1) * sizeof(int64_t)));
+        CUDA_TRY(alloc(indices, nnz * sizeof(uint32_t)));
+        CUDA_TRY(cudaMemcpy(indptr.get(), h_indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
+        CUDA_TRY(cudaMemcpy(indices.get(), h_indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        if (int rc = check_csr_contents(h_indptr, indptr.get(), indices.get(), n)) return rc;
+        view.indptr = indptr.get();
+        view.indices = indices.get();
         view.inv_max_degree = 1.0f / (float)max_degree;
         return B2E_OK;
     }
 };
 
-static int select_device(const b2e_features *f) {
-    if (f) EP_TRY(cudaSetDevice(f->device));
+static int use_features_device(const b2e_features *f) {
+    if (f) CUDA_TRY(cudaSetDevice(f->device));
     return B2E_OK;
 }
 
 extern "C" int b2e_features_create(int device, const float *host, uint64_t n, uint32_t dim, b2e_features **out) {
-    if (!host || !out || n == 0 || dim == 0) return b2e_set_error(B2E_ERR_INVALID, "null or empty node features");
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0)
-        return b2e_set_error(B2E_ERR_CUDA, "no CUDA device available (there is no CPU fallback)");
-    if (device < 0 || device >= count) return b2e_set_error(B2E_ERR_INVALID, "device ordinal out of range");
-    EP_TRY(cudaSetDevice(device));
-    b2e_features *f = new b2e_features();
+    if (!host || !out || n == 0 || dim == 0) return fail(B2E_ERR_INVALID, "null or empty node features");
+    if (int rc = select_device(device)) return rc;
+    std::unique_ptr<b2e_features> f(new b2e_features());
     f->device = device;
     f->n = n;
     f->dim = dim;
     f->pitch = dim;
-    cudaError_t e = cudaMalloc(&f->d, n * (uint64_t)dim * sizeof(float));
-    if (e == cudaSuccess) e = cudaMemcpy(f->d, host, n * (uint64_t)dim * sizeof(float), cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) {
-        cudaFree(f->d);
-        delete f;
-        return b2e_set_error(B2E_ERR_CUDA, std::string("node features: ") + cudaGetErrorString(e));
-    }
-    *out = f;
+    CUDA_TRY(f->owned.reserve(n * (uint64_t)dim * sizeof(float)));
+    CUDA_TRY(cudaMemcpy(f->owned.get(), host, n * (uint64_t)dim * sizeof(float), cudaMemcpyHostToDevice));
+    f->d = f->owned.get();
+    *out = f.release();
     return B2E_OK;
 }
 
 extern "C" int b2e_features_from_handle(b2e_handle *h, int table, b2e_features **out) {
-    if (!h || !out || table < 0 || table > 1) return b2e_set_error(B2E_ERR_INVALID, "bad argument");
-    if (!h->d_t0) return b2e_set_error(B2E_ERR_STATE, "the handle holds no tables yet");
+    if (!h || !out || table < 0 || table > 1) return fail(B2E_ERR_INVALID, "bad argument");
+    if (!h->graph.t0.get()) return fail(B2E_ERR_STATE, "the handle holds no tables yet");
     if (int rc = b2e_sync(h)) return rc;
     b2e_features *f = new b2e_features();
     f->device = h->cfg.device;
-    f->d = table ? h->d_t1 : h->d_t0;
+    f->d = table ? h->graph.t1.get() : h->graph.t0.get();
     f->n = h->n;
     f->dim = h->cfg.embedding_size;
     f->pitch = h->row_stride;
-    f->owned = false;  // a view: valid while the handle lives and keeps its graph
+    // a view: valid while the handle lives and keeps its graph
     *out = f;
     return B2E_OK;
 }
 
 extern "C" void b2e_features_destroy(b2e_features *f) {
     if (!f) return;
-    if (f->owned) { cudaSetDevice(f->device); cudaFree(f->d); }
+    if (f->owned.get()) cudaSetDevice(f->device);
     delete f;
 }
 
 extern "C" int b2e_edge_embedding_size(uint32_t dim, const uint32_t *methods, uint32_t n_methods,
                                        const uint32_t *edge_features, uint32_t n_edge_features, uint32_t *size) {
     MethodList list;
-    if (!size) return b2e_set_error(B2E_ERR_INVALID, "null argument");
+    if (!size) return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = build_methods(methods, n_methods, dim, edge_features, n_edge_features, list)) return rc;
     *size = list.size;
     return B2E_OK;
 }
 
 static int upload_edges(uint64_t n, const uint32_t *src, const uint32_t *dst, uint64_t m,
-                        DeviceArray &d_src, DeviceArray &d_dst) {
+                        DeviceBuffer<uint32_t> &d_src, DeviceBuffer<uint32_t> &d_dst) {
     for (uint64_t e = 0; e < m; ++e)
-        if (src[e] >= n || dst[e] >= n) return b2e_set_error(B2E_ERR_INVALID, "a node id is out of range");
-    EP_TRY(d_src.alloc(m * sizeof(uint32_t)));
-    EP_TRY(d_dst.alloc(m * sizeof(uint32_t)));
-    EP_TRY(cudaMemcpy(d_src.p, src, m * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    EP_TRY(cudaMemcpy(d_dst.p, dst, m * sizeof(uint32_t), cudaMemcpyHostToDevice));
+        if (src[e] >= n || dst[e] >= n) return fail(B2E_ERR_INVALID, "a node id is out of range");
+    CUDA_TRY(alloc(d_src, m * sizeof(uint32_t)));
+    CUDA_TRY(alloc(d_dst, m * sizeof(uint32_t)));
+    CUDA_TRY(cudaMemcpy(d_src.get(), src, m * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(d_dst.get(), dst, m * sizeof(uint32_t), cudaMemcpyHostToDevice));
     return B2E_OK;
 }
 
@@ -652,23 +631,24 @@ static unsigned warp_grid(uint64_t warps_wanted) {
 
 extern "C" int b2e_edge_embedding(const b2e_features *f, const uint32_t *src, const uint32_t *dst, uint64_t m,
                                   const uint32_t *methods, uint32_t n_methods, float *out) {
-    if (!f || (m && (!src || !dst || !out))) return b2e_set_error(B2E_ERR_INVALID, "null argument");
+    if (!f || (m && (!src || !dst || !out))) return fail(B2E_ERR_INVALID, "null argument");
     MethodList list;
-    if (n_methods == 0) return b2e_set_error(B2E_ERR_INVALID, "at least one edge embedding method is required");
+    if (n_methods == 0) return fail(B2E_ERR_INVALID, "at least one edge embedding method is required");
     if (int rc = build_methods(methods, n_methods, f->dim, nullptr, 0, list)) return rc;
     if (m == 0) return B2E_OK;
-    EP_TRY(cudaSetDevice(f->device));
-    DeviceArray d_src, d_dst, d_out;
+    CUDA_TRY(cudaSetDevice(f->device));
+    DeviceBuffer<uint32_t> d_src, d_dst;
+    DeviceBuffer<float> d_out;
     if (int rc = upload_edges(f->n, src, dst, m, d_src, d_dst)) return rc;
     // the materialised embedding is produced in slabs so that it never needs more than 1 GiB
     const uint64_t slab = std::max<uint64_t>(1, (1ull << 28) / list.size);
-    EP_TRY(d_out.alloc(std::min(slab, m) * list.size * sizeof(float)));
+    CUDA_TRY(alloc(d_out, std::min(slab, m) * list.size * sizeof(float)));
     for (uint64_t done = 0; done < m; done += slab) {
         const uint64_t count = std::min(slab, m - done);
-        edge_embedding_kernel<<<warp_grid(count), 256>>>(f->d, f->pitch, f->dim, d_src.as<uint32_t>() + done,
-                                                        d_dst.as<uint32_t>() + done, count, list, d_out.as<float>());
-        EP_TRY(cudaGetLastError());
-        EP_TRY(cudaMemcpy(out + done * list.size, d_out.p, count * list.size * sizeof(float), cudaMemcpyDeviceToHost));
+        edge_embedding_kernel<<<warp_grid(count), 256>>>(f->d, f->pitch, f->dim, d_src.get() + done,
+                                                        d_dst.get() + done, count, list, d_out.get());
+        CUDA_TRY(cudaGetLastError());
+        CUDA_TRY(cudaMemcpy(out + done * list.size, d_out.get(), count * list.size * sizeof(float), cudaMemcpyDeviceToHost));
     }
     return B2E_OK;
 }
@@ -676,21 +656,22 @@ extern "C" int b2e_edge_embedding(const b2e_features *f, const uint32_t *src, co
 extern "C" int b2e_edge_metrics(int device, const int64_t *indptr, const uint32_t *indices, uint64_t n, uint64_t nnz,
                                 const uint32_t *src, const uint32_t *dst, uint64_t m, const uint32_t *edge_features,
                                 uint32_t n_edge_features, float *out) {
-    if (m && (!src || !dst || !out)) return b2e_set_error(B2E_ERR_INVALID, "null argument");
+    if (m && (!src || !dst || !out)) return fail(B2E_ERR_INVALID, "null argument");
     MethodList list;
-    if (n_edge_features == 0) return b2e_set_error(B2E_ERR_INVALID, "at least one edge feature is required");
+    if (n_edge_features == 0) return fail(B2E_ERR_INVALID, "at least one edge feature is required");
     if (int rc = build_methods(nullptr, 0, 0, edge_features, n_edge_features, list)) return rc;
     if (m == 0) return B2E_OK;
-    EP_TRY(cudaSetDevice(device));
+    CUDA_TRY(cudaSetDevice(device));
     DeviceGraph graph;
     if (int rc = graph.upload(indptr, indices, n, nnz)) return rc;
-    DeviceArray d_src, d_dst, d_out;
+    DeviceBuffer<uint32_t> d_src, d_dst;
+    DeviceBuffer<float> d_out;
     if (int rc = upload_edges(n, src, dst, m, d_src, d_dst)) return rc;
-    EP_TRY(d_out.alloc(m * list.size * sizeof(float)));
-    edge_metrics_kernel<<<warp_grid(m), 256>>>(graph.view, d_src.as<uint32_t>(), d_dst.as<uint32_t>(), m, list,
-                                               d_out.as<float>());
-    EP_TRY(cudaGetLastError());
-    EP_TRY(cudaMemcpy(out, d_out.p, m * list.size * sizeof(float), cudaMemcpyDeviceToHost));
+    CUDA_TRY(alloc(d_out, m * list.size * sizeof(float)));
+    edge_metrics_kernel<<<warp_grid(m), 256>>>(graph.view, d_src.get(), d_dst.get(), m, list,
+                                               d_out.get());
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpy(out, d_out.get(), m * list.size * sizeof(float), cudaMemcpyDeviceToHost));
     return B2E_OK;
 }
 
@@ -698,82 +679,86 @@ extern "C" int b2e_perceptron_predict(const b2e_features *f, const int64_t *indp
                                       uint64_t n, uint64_t nnz, const uint32_t *src, const uint32_t *dst, uint64_t m,
                                       const uint32_t *methods, uint32_t n_methods, const uint32_t *edge_features,
                                       uint32_t n_edge_features, const float *params, float *scores) {
-    if (!params || (m && (!src || !dst || !scores))) return b2e_set_error(B2E_ERR_INVALID, "null argument");
-    if (n_methods && !f) return b2e_set_error(B2E_ERR_INVALID, "edge embeddings need node features");
+    if (!params || (m && (!src || !dst || !scores))) return fail(B2E_ERR_INVALID, "null argument");
+    if (n_methods && !f) return fail(B2E_ERR_INVALID, "edge embeddings need node features");
     if (f && n_edge_features && n != f->n)
-        return b2e_set_error(B2E_ERR_INVALID, "the graph and the node features disagree on the number of nodes");
+        return fail(B2E_ERR_INVALID, "the graph and the node features disagree on the number of nodes");
     MethodList list;
     if (int rc = build_methods(methods, n_methods, f ? f->dim : 0, edge_features, n_edge_features, list)) return rc;
     if (m == 0) return B2E_OK;
-    if (int rc = select_device(f)) return rc;
+    if (int rc = use_features_device(f)) return rc;
     DeviceGraph graph;
     if (n_edge_features)
         if (int rc = graph.upload(indptr, indices, n, nnz)) return rc;
-    DeviceArray d_src, d_dst, d_params, d_scores;
+    DeviceBuffer<uint32_t> d_src, d_dst;
+    DeviceBuffer<float> d_params, d_scores;
     if (int rc = upload_edges(f ? f->n : n, src, dst, m, d_src, d_dst)) return rc;
-    EP_TRY(d_params.alloc((list.size + 1) * sizeof(float)));
-    EP_TRY(d_scores.alloc(m * sizeof(float)));
-    EP_TRY(cudaMemcpy(d_params.p, params, (list.size + 1) * sizeof(float), cudaMemcpyHostToDevice));
+    CUDA_TRY(alloc(d_params, (list.size + 1) * sizeof(float)));
+    CUDA_TRY(alloc(d_scores, m * sizeof(float)));
+    CUDA_TRY(cudaMemcpy(d_params.get(), params, (list.size + 1) * sizeof(float), cudaMemcpyHostToDevice));
     const size_t smem = (list.size + 1) * sizeof(float);
-    EP_TRY(cudaFuncSetAttribute(perceptron_predict_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CUDA_TRY(cudaFuncSetAttribute(perceptron_predict_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     perceptron_predict_kernel<<<warp_grid(m), 256, smem>>>(f ? f->d : nullptr, f ? f->pitch : 0, f ? f->dim : 0,
-                                                           d_src.as<uint32_t>(), d_dst.as<uint32_t>(), m, list,
-                                                           graph.view, d_params.as<float>(), d_scores.as<float>());
-    EP_TRY(cudaGetLastError());
-    EP_TRY(cudaMemcpy(scores, d_scores.p, m * sizeof(float), cudaMemcpyDeviceToHost));
+                                                           d_src.get(), d_dst.get(), m, list,
+                                                           graph.view, d_params.get(), d_scores.get());
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaMemcpy(scores, d_scores.get(), m * sizeof(float), cudaMemcpyDeviceToHost));
     return B2E_OK;
 }
 
 extern "C" int b2e_perceptron_fit(const b2e_features *f, const int64_t *indptr, const uint32_t *indices, uint64_t n,
                                   uint64_t nnz, const b2e_perceptron_config *cfg, uint64_t seed, float *params_out,
                                   float *epoch_loss) {
-    if (!indptr || !indices || !cfg || !params_out) return b2e_set_error(B2E_ERR_INVALID, "null argument");
+    if (!indptr || !indices || !cfg || !params_out) return fail(B2E_ERR_INVALID, "null argument");
     if (cfg->struct_size != sizeof(b2e_perceptron_config))
-        return b2e_set_error(B2E_ERR_INVALID, "b2e_perceptron_config size mismatch (ABI)");
-    if (cfg->n_methods && !f) return b2e_set_error(B2E_ERR_INVALID, "edge embeddings need node features");
-    if (f && n != f->n) return b2e_set_error(B2E_ERR_INVALID, "the graph and the node features disagree on the number of nodes");
+        return fail(B2E_ERR_INVALID, "b2e_perceptron_config size mismatch (ABI)");
+    if (cfg->n_methods && !f) return fail(B2E_ERR_INVALID, "edge embeddings need node features");
+    if (f && n != f->n) return fail(B2E_ERR_INVALID, "the graph and the node features disagree on the number of nodes");
     if (nnz == 0 || indptr[0] != 0 || (uint64_t)indptr[n] != nnz)
-        return b2e_set_error(B2E_ERR_INVALID, "the graph has no edges");
-    if (cfg->number_of_edges_per_mini_batch == 0) return b2e_set_error(B2E_ERR_INVALID, "empty mini-batch");
+        return fail(B2E_ERR_INVALID, "the graph has no edges");
+    if (cfg->number_of_edges_per_mini_batch == 0) return fail(B2E_ERR_INVALID, "empty mini-batch");
     if (!(cfg->first_order_decay_factor >= 0.f && cfg->first_order_decay_factor < 1.f) ||
         !(cfg->second_order_decay_factor >= 0.f && cfg->second_order_decay_factor < 1.f))
-        return b2e_set_error(B2E_ERR_INVALID, "decay factors must be in [0, 1)");
+        return fail(B2E_ERR_INVALID, "decay factors must be in [0, 1)");
     MethodList list;
     if (int rc = build_methods(cfg->methods, cfg->n_methods, f ? f->dim : 0, cfg->edge_features,
                                cfg->n_edge_features, list))
         return rc;
-    if (int rc = select_device(f)) return rc;
+    if (int rc = use_features_device(f)) return rc;
     int64_t max_degree = 1;
     for (uint64_t v = 0; v < n; ++v) max_degree = std::max(max_degree, indptr[v + 1] - indptr[v]);
     const uint32_t count = list.size + 1;
-    DeviceArray d_indptr, d_indices, d_edge_src, d_params, d_m, d_v, d_grad, d_loss;
-    EP_TRY(d_indptr.alloc((n + 1) * sizeof(int64_t)));
-    EP_TRY(d_indices.alloc(nnz * sizeof(uint32_t)));
-    EP_TRY(d_edge_src.alloc(nnz * sizeof(uint32_t)));
-    EP_TRY(d_params.alloc(count * sizeof(float)));
-    EP_TRY(d_m.alloc(count * sizeof(float)));
-    EP_TRY(d_v.alloc(count * sizeof(float)));
-    EP_TRY(d_grad.alloc(count * sizeof(float)));
-    EP_TRY(d_loss.alloc(2 * sizeof(double)));
-    EP_TRY(cudaMemcpy(d_indptr.p, indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
-    EP_TRY(cudaMemcpy(d_indices.p, indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    if (int rc = check_csr_contents(indptr, d_indptr.as<int64_t>(), d_indices.as<uint32_t>(), n)) return rc;
-    EP_TRY(cudaMemset(d_m.p, 0, count * sizeof(float)));
-    EP_TRY(cudaMemset(d_v.p, 0, count * sizeof(float)));
-    EP_TRY(cudaMemset(d_grad.p, 0, count * sizeof(float)));
-    edge_sources_kernel<<<warp_grid(n), 256>>>(d_indptr.as<int64_t>(), n, d_edge_src.as<uint32_t>());
-    perceptron_init_kernel<<<(count + 255) / 256, 256>>>(d_params.as<float>(), list.size, (uint32_t)seed,
+    DeviceBuffer<int64_t> d_indptr;
+    DeviceBuffer<uint32_t> d_indices, d_edge_src;
+    DeviceBuffer<float> d_params, d_m, d_v, d_grad;
+    DeviceBuffer<double> d_loss;
+    CUDA_TRY(alloc(d_indptr, (n + 1) * sizeof(int64_t)));
+    CUDA_TRY(alloc(d_indices, nnz * sizeof(uint32_t)));
+    CUDA_TRY(alloc(d_edge_src, nnz * sizeof(uint32_t)));
+    CUDA_TRY(alloc(d_params, count * sizeof(float)));
+    CUDA_TRY(alloc(d_m, count * sizeof(float)));
+    CUDA_TRY(alloc(d_v, count * sizeof(float)));
+    CUDA_TRY(alloc(d_grad, count * sizeof(float)));
+    CUDA_TRY(alloc(d_loss, 2 * sizeof(double)));
+    CUDA_TRY(cudaMemcpy(d_indptr.get(), indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
+    CUDA_TRY(cudaMemcpy(d_indices.get(), indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    if (int rc = check_csr_contents(indptr, d_indptr.get(), d_indices.get(), n)) return rc;
+    CUDA_TRY(cudaMemset(d_m.get(), 0, count * sizeof(float)));
+    CUDA_TRY(cudaMemset(d_v.get(), 0, count * sizeof(float)));
+    CUDA_TRY(cudaMemset(d_grad.get(), 0, count * sizeof(float)));
+    edge_sources_kernel<<<warp_grid(n), 256>>>(d_indptr.get(), n, d_edge_src.get());
+    perceptron_init_kernel<<<(count + 255) / 256, 256>>>(d_params.get(), list.size, (uint32_t)seed,
                                                          (uint32_t)(seed >> 32));
-    EP_TRY(cudaGetLastError());
+    CUDA_TRY(cudaGetLastError());
 
     StepParams p;
     p.features = f ? f->d : nullptr;
     p.pitch = f ? f->pitch : 0;
     p.dim = f ? f->dim : 0;
     p.inv_max_degree = 1.0f / (float)max_degree;
-    p.indptr = d_indptr.as<int64_t>();
-    p.indices = d_indices.as<uint32_t>();
-    p.edge_src = d_edge_src.as<uint32_t>();
+    p.indptr = d_indptr.get();
+    p.indices = d_indices.get();
+    p.edge_src = d_edge_src.get();
     p.n = (uint32_t)n;
     p.nnz = nnz;
     p.seed_lo = (uint32_t)seed;
@@ -781,32 +766,32 @@ extern "C" int b2e_perceptron_fit(const b2e_features *f, const int64_t *indptr, 
     p.batch = cfg->number_of_edges_per_mini_batch;
     p.scale_free = cfg->use_scale_free_distribution ? 1u : 0u;
     p.avoid_false_negatives = cfg->avoid_false_negatives ? 1u : 0u;
-    p.params = d_params.as<float>();
-    p.grad = d_grad.as<float>();
-    p.loss = d_loss.as<double>();
+    p.params = d_params.get();
+    p.grad = d_grad.get();
+    p.loss = d_loss.get();
     const size_t smem = 2 * (size_t)count * sizeof(float);
-    EP_TRY(cudaFuncSetAttribute(perceptron_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+    CUDA_TRY(cudaFuncSetAttribute(perceptron_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     const uint64_t steps_per_epoch = std::max<uint64_t>(1, nnz / p.batch);
     const double beta1 = cfg->first_order_decay_factor, beta2 = cfg->second_order_decay_factor;
     uint64_t step = 0;
     for (uint32_t epoch = 0; epoch < cfg->number_of_epochs; ++epoch) {
-        EP_TRY(cudaMemsetAsync(d_loss.p, 0, 2 * sizeof(double)));
+        CUDA_TRY(cudaMemsetAsync(d_loss.get(), 0, 2 * sizeof(double)));
         for (uint64_t s = 0; s < steps_per_epoch; ++s) {
             ++step;
             p.step = (uint32_t)step;
             perceptron_step_kernel<<<warp_grid(p.batch), 256, smem>>>(p, list);
             const float lr_s = (float)((double)cfg->learning_rate * std::sqrt(1.0 - std::pow(beta2, (double)step)) /
                                        (1.0 - std::pow(beta1, (double)step)));
-            adam_kernel<<<(count + 255) / 256, 256>>>(d_params.as<float>(), d_m.as<float>(), d_v.as<float>(),
-                                                      d_grad.as<float>(), count, (float)beta1, (float)beta2, lr_s);
+            adam_kernel<<<(count + 255) / 256, 256>>>(d_params.get(), d_m.get(), d_v.get(),
+                                                      d_grad.get(), count, (float)beta1, (float)beta2, lr_s);
         }
-        EP_TRY(cudaGetLastError());
+        CUDA_TRY(cudaGetLastError());
         if (epoch_loss) {
             double host[2];
-            EP_TRY(cudaMemcpy(host, d_loss.p, sizeof(host), cudaMemcpyDeviceToHost));
+            CUDA_TRY(cudaMemcpy(host, d_loss.get(), sizeof(host), cudaMemcpyDeviceToHost));
             epoch_loss[epoch] = host[1] > 0 ? (float)(host[0] / host[1]) : 0.f;
         }
     }
-    EP_TRY(cudaMemcpy(params_out, d_params.p, count * sizeof(float), cudaMemcpyDeviceToHost));
+    CUDA_TRY(cudaMemcpy(params_out, d_params.get(), count * sizeof(float), cudaMemcpyDeviceToHost));
     return B2E_OK;
 }

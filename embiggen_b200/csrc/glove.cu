@@ -25,6 +25,7 @@
 
 #include <algorithm>
 
+#include "host.cuh"
 #include "sgns_device.cuh"
 
 namespace b2e {
@@ -279,22 +280,6 @@ static cudaError_t launch_glove_one(const GloveParams &p, uint64_t n_triples, bo
     return cudaGetLastError();
 }
 
-#define GLOVE_TRY(call)                            \
-    do {                                           \
-        cudaError_t e_ = (call);                   \
-        if (e_ != cudaSuccess) return e_;          \
-    } while (0)
-
-static cudaError_t grow(void **ptr, size_t *have, size_t want) {
-    if (want <= *have) return cudaSuccess;
-    cudaFree(*ptr);
-    *ptr = nullptr;
-    *have = 0;
-    cudaError_t e = cudaMalloc(ptr, want);
-    if (e == cudaSuccess) *have = want;
-    return e;
-}
-
 // walks per co-occurrence chunk: at most 2^27 key slots (1 GiB of keys, sorted out of place)
 uint64_t glove_chunk_walks(uint32_t walk_length, uint32_t window) {
     const uint64_t slots_per_walk = 2ull * walk_length * window;
@@ -303,53 +288,53 @@ uint64_t glove_chunk_walks(uint32_t walk_length, uint32_t window) {
 
 // Adds the co-occurrences of `n_walks` device-resident walks to the state (merged by key).
 cudaError_t glove_accumulate(GloveState &g, const uint32_t *d_walks, uint64_t n_walks, uint32_t L,
-                             uint32_t W, cudaStream_t stream) {
+                             uint32_t W, cudaStream_t stream, std::string &error) {
     typedef unsigned long long u64;
     const uint64_t slots = 2ull * n_walks * L * W;
     if (slots == 0) return cudaSuccess;
-    GLOVE_TRY(grow((void **)&g.d_scratch_keys, &g.scratch_keys_bytes, 2 * slots * sizeof(u64)));
-    u64 *raw = g.d_scratch_keys, *sorted = g.d_scratch_keys + slots;
+    CUDA_CHECK(g.d_scratch_keys.reserve(2 * slots * sizeof(u64)));
+    u64 *raw = g.d_scratch_keys.get(), *sorted = g.d_scratch_keys.get() + slots;
     const uint64_t grid = std::min<uint64_t>((slots / 2 + 255) / 256, 148ull * 32);
     cooc_keys_kernel<<<(unsigned)grid, 256, 0, stream>>>(d_walks, n_walks, L, W, raw);
-    GLOVE_TRY(cudaGetLastError());
+    CUDA_CHECK(cudaGetLastError());
 
     size_t need = 0, bytes = 0;
-    GLOVE_TRY(cub::DeviceRadixSort::SortKeys(nullptr, bytes, raw, sorted, slots, 0, 64, stream));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, raw, sorted, slots, 0, 64, stream));
     need = bytes;
     // run-length encode into the tail of the merge buffers (sized below)
     const uint64_t merged_cap = g.n_triples + slots;
-    GLOVE_TRY(grow((void **)&g.d_merge_keys, &g.merge_keys_bytes, 2 * merged_cap * sizeof(u64)));
-    GLOVE_TRY(grow((void **)&g.d_merge_counts, &g.merge_counts_bytes, 2 * merged_cap * sizeof(uint32_t)));
-    GLOVE_TRY(grow((void **)&g.d_scalar, &g.scalar_bytes, 16));
-    u64 *cat_keys = g.d_merge_keys, *out_keys = g.d_merge_keys + merged_cap;
-    uint32_t *cat_counts = g.d_merge_counts, *out_counts = g.d_merge_counts + merged_cap;
-    uint64_t *d_runs = reinterpret_cast<uint64_t *>(g.d_scalar);
-    GLOVE_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, bytes, sorted, cat_keys + g.n_triples,
+    CUDA_CHECK(g.d_merge_keys.reserve(2 * merged_cap * sizeof(u64)));
+    CUDA_CHECK(g.d_merge_counts.reserve(2 * merged_cap * sizeof(uint32_t)));
+    CUDA_CHECK(g.d_scalar.reserve(16));
+    u64 *cat_keys = g.d_merge_keys.get(), *out_keys = g.d_merge_keys.get() + merged_cap;
+    uint32_t *cat_counts = g.d_merge_counts.get(), *out_counts = g.d_merge_counts.get() + merged_cap;
+    uint64_t *d_runs = reinterpret_cast<uint64_t *>(g.d_scalar.get());
+    CUDA_CHECK(cub::DeviceRunLengthEncode::Encode(nullptr, bytes, sorted, cat_keys + g.n_triples,
                                                  cat_counts + g.n_triples, d_runs, slots, stream));
     need = std::max(need, bytes);
     // merging two sorted lists is one linear pass (sorting the concatenation would be eight)
-    GLOVE_TRY(cub::DeviceMerge::MergePairs(nullptr, bytes, g.d_keys, g.d_counts, (int64_t)g.n_triples,
+    CUDA_CHECK(cub::DeviceMerge::MergePairs(nullptr, bytes, g.d_keys.get(), g.d_counts.get(), (int64_t)g.n_triples,
                                            cat_keys + g.n_triples, cat_counts + g.n_triples, (int64_t)slots,
                                            out_keys, out_counts, ::cuda::std::less<>{}, stream));
     need = std::max(need, bytes);
-    GLOVE_TRY(cub::DeviceReduce::ReduceByKey(nullptr, bytes, out_keys, cat_keys, out_counts, cat_counts, d_runs,
+    CUDA_CHECK(cub::DeviceReduce::ReduceByKey(nullptr, bytes, out_keys, cat_keys, out_counts, cat_counts, d_runs,
                                              cub::Sum(), merged_cap, stream));
     need = std::max(need, bytes);
-    GLOVE_TRY(grow(&g.d_temp, &g.temp_bytes, need));
+    CUDA_CHECK(g.d_temp.reserve(need));
 
-    bytes = g.temp_bytes;
-    GLOVE_TRY(cub::DeviceRadixSort::SortKeys(g.d_temp, bytes, raw, sorted, slots, 0, 64, stream));
+    bytes = g.d_temp.bytes();
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(g.d_temp.get(), bytes, raw, sorted, slots, 0, 64, stream));
     // the chunk's (key, count) list goes behind the room of the triples gathered so far
-    bytes = g.temp_bytes;
-    GLOVE_TRY(cub::DeviceRunLengthEncode::Encode(g.d_temp, bytes, sorted, cat_keys + g.n_triples,
+    bytes = g.d_temp.bytes();
+    CUDA_CHECK(cub::DeviceRunLengthEncode::Encode(g.d_temp.get(), bytes, sorted, cat_keys + g.n_triples,
                                                  cat_counts + g.n_triples, d_runs, slots, stream));
     uint64_t runs = 0;
-    GLOVE_TRY(cudaMemcpyAsync(&runs, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
-    GLOVE_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaMemcpyAsync(&runs, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     if (runs) {  // the all-ones key, if present, is the last run
         u64 last = 0;
-        GLOVE_TRY(cudaMemcpyAsync(&last, cat_keys + g.n_triples + runs - 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-        GLOVE_TRY(cudaStreamSynchronize(stream));
+        CUDA_CHECK(cudaMemcpyAsync(&last, cat_keys + g.n_triples + runs - 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
+        CUDA_CHECK(cudaStreamSynchronize(stream));
         if (last == COOC_INVALID) --runs;
     }
     if (runs == 0) return cudaSuccess;  // nothing new: the resident triples stand
@@ -358,42 +343,42 @@ cudaError_t glove_accumulate(GloveState &g, const uint32_t *d_walks, uint64_t n_
     const uint32_t *result_counts = cat_counts;
     if (g.n_triples) {  // both lists are sorted: merge, then add the counts of equal keys
         total = g.n_triples + runs;
-        bytes = g.temp_bytes;
-        GLOVE_TRY(cub::DeviceMerge::MergePairs(g.d_temp, bytes, g.d_keys, g.d_counts, (int64_t)g.n_triples,
+        bytes = g.d_temp.bytes();
+        CUDA_CHECK(cub::DeviceMerge::MergePairs(g.d_temp.get(), bytes, g.d_keys.get(), g.d_counts.get(), (int64_t)g.n_triples,
                                                cat_keys + g.n_triples, cat_counts + g.n_triples, (int64_t)runs,
                                                out_keys, out_counts, ::cuda::std::less<>{}, stream));
-        bytes = g.temp_bytes;
-        GLOVE_TRY(cub::DeviceReduce::ReduceByKey(g.d_temp, bytes, out_keys, cat_keys, out_counts, cat_counts,
+        bytes = g.d_temp.bytes();
+        CUDA_CHECK(cub::DeviceReduce::ReduceByKey(g.d_temp.get(), bytes, out_keys, cat_keys, out_counts, cat_counts,
                                                  d_runs, cub::Sum(), total, stream));
-        GLOVE_TRY(cudaMemcpyAsync(&total, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
-        GLOVE_TRY(cudaStreamSynchronize(stream));
+        CUDA_CHECK(cudaMemcpyAsync(&total, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        CUDA_CHECK(cudaStreamSynchronize(stream));
     }
-    GLOVE_TRY(grow((void **)&g.d_keys, &g.keys_bytes, total * sizeof(u64)));
-    GLOVE_TRY(grow((void **)&g.d_counts, &g.counts_bytes, total * sizeof(uint32_t)));
-    GLOVE_TRY(cudaMemcpyAsync(g.d_keys, result_keys, total * sizeof(u64), cudaMemcpyDeviceToDevice, stream));
-    GLOVE_TRY(cudaMemcpyAsync(g.d_counts, result_counts, total * sizeof(uint32_t), cudaMemcpyDeviceToDevice, stream));
+    CUDA_CHECK(g.d_keys.reserve(total * sizeof(u64)));
+    CUDA_CHECK(g.d_counts.reserve(total * sizeof(uint32_t)));
+    CUDA_CHECK(cudaMemcpyAsync(g.d_keys.get(), result_keys, total * sizeof(u64), cudaMemcpyDeviceToDevice, stream));
+    CUDA_CHECK(cudaMemcpyAsync(g.d_counts.get(), result_counts, total * sizeof(uint32_t), cudaMemcpyDeviceToDevice, stream));
     g.n_triples = total;
     g.finalised = false;
     return cudaSuccess;
 }
 
 // row offsets by centre and the largest count: needed before training
-cudaError_t glove_finalise(GloveState &g, uint64_t n, cudaStream_t stream) {
-    GLOVE_TRY(grow((void **)&g.d_rowptr, &g.rowptr_bytes, (n + 1) * sizeof(uint64_t)));
-    cooc_rowptr_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, stream>>>(g.d_keys, g.n_triples, n, g.d_rowptr);
-    GLOVE_TRY(cudaGetLastError());
+cudaError_t glove_finalise(GloveState &g, uint64_t n, cudaStream_t stream, std::string &error) {
+    CUDA_CHECK(g.d_rowptr.reserve((n + 1) * sizeof(uint64_t)));
+    cooc_rowptr_kernel<<<(unsigned)((n + 1 + 255) / 256), 256, 0, stream>>>(g.d_keys.get(), g.n_triples, n, g.d_rowptr.get());
+    CUDA_CHECK(cudaGetLastError());
     g.max_count = 1;
     if (g.n_triples) {
-        GLOVE_TRY(grow((void **)&g.d_scalar, &g.scalar_bytes, 16));
-        uint32_t *d_max = reinterpret_cast<uint32_t *>(g.d_scalar);
+        CUDA_CHECK(g.d_scalar.reserve(16));
+        uint32_t *d_max = reinterpret_cast<uint32_t *>(g.d_scalar.get());
         size_t bytes = 0;
-        GLOVE_TRY(cub::DeviceReduce::Max(nullptr, bytes, g.d_counts, d_max, g.n_triples, stream));
-        GLOVE_TRY(grow(&g.d_temp, &g.temp_bytes, bytes));
-        bytes = g.temp_bytes;
-        GLOVE_TRY(cub::DeviceReduce::Max(g.d_temp, bytes, g.d_counts, d_max, g.n_triples, stream));
-        GLOVE_TRY(cudaMemcpyAsync(&g.max_count, d_max, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+        CUDA_CHECK(cub::DeviceReduce::Max(nullptr, bytes, g.d_counts.get(), d_max, g.n_triples, stream));
+        CUDA_CHECK(g.d_temp.reserve(bytes));
+        bytes = g.d_temp.bytes();
+        CUDA_CHECK(cub::DeviceReduce::Max(g.d_temp.get(), bytes, g.d_counts.get(), d_max, g.n_triples, stream));
+        CUDA_CHECK(cudaMemcpyAsync(&g.max_count, d_max, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
     }
-    GLOVE_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     g.finalised = true;
     return cudaSuccess;
 }
@@ -403,9 +388,9 @@ cudaError_t glove_train(const GloveState &g, uint64_t n, uint32_t row_stride, ui
                         bool deterministic, int sm_count, uint64_t max_warps, cudaStream_t stream) {
     if (g.n_triples == 0) return cudaSuccess;
     GloveParams p;
-    p.keys = g.d_keys;
-    p.counts = g.d_counts;
-    p.rowptr = g.d_rowptr;
+    p.keys = g.d_keys.get();
+    p.counts = g.d_counts.get();
+    p.rowptr = g.d_rowptr.get();
     p.n = n;
     p.row_stride = row_stride;
     p.chunks = (embedding_size + 3u) / 4u;
@@ -488,8 +473,8 @@ __global__ void __launch_bounds__(256) range_keys_kernel(const uint32_t *__restr
 
 cudaError_t glove_token_histogram(const uint32_t *d_walks, uint64_t tokens, uint32_t *d_histogram, uint64_t n,
                                   cudaStream_t stream) {
-    GLOVE_TRY(cudaMemsetAsync(d_histogram, 0, n * sizeof(uint32_t), stream));
-    if (tokens == 0) return cudaSuccess;
+    const cudaError_t e = cudaMemsetAsync(d_histogram, 0, n * sizeof(uint32_t), stream);
+    if (e != cudaSuccess || tokens == 0) return e;
     token_histogram_kernel<<<148 * 16, 256, 0, stream>>>(d_walks, tokens, d_histogram);
     return cudaGetLastError();
 }
@@ -505,67 +490,59 @@ cudaError_t glove_bucket_positions(const uint32_t *d_walks, uint64_t tokens, con
 // The co-occurrence triples of one centre range replace the resident ones (g.n_triples, sorted
 // by (centre, context)); `count` occurrences, 2 W key slots each.
 cudaError_t glove_range_triples(GloveState &g, const uint32_t *d_walks, uint32_t L, uint32_t W,
-                                const unsigned long long *d_positions, uint64_t count, cudaStream_t stream) {
+                                const unsigned long long *d_positions, uint64_t count, cudaStream_t stream,
+                                std::string &error) {
     typedef unsigned long long u64;
     g.n_triples = 0;
     g.finalised = false;
     const uint64_t slots = count * 2ull * W;
     if (slots == 0) return cudaSuccess;
-    GLOVE_TRY(grow((void **)&g.d_scratch_keys, &g.scratch_keys_bytes, 2 * slots * sizeof(u64)));
-    u64 *raw = g.d_scratch_keys, *sorted = g.d_scratch_keys + slots;
+    CUDA_CHECK(g.d_scratch_keys.reserve(2 * slots * sizeof(u64)));
+    u64 *raw = g.d_scratch_keys.get(), *sorted = g.d_scratch_keys.get() + slots;
     const uint64_t grid = std::min<uint64_t>((slots + 255) / 256, 148ull * 32);
     range_keys_kernel<<<(unsigned)grid, 256, 0, stream>>>(d_walks, L, W, d_positions, count, raw);
-    GLOVE_TRY(cudaGetLastError());
-    GLOVE_TRY(grow((void **)&g.d_keys, &g.keys_bytes, slots * sizeof(u64)));
-    GLOVE_TRY(grow((void **)&g.d_counts, &g.counts_bytes, slots * sizeof(uint32_t)));
-    GLOVE_TRY(grow((void **)&g.d_scalar, &g.scalar_bytes, 16));
-    uint64_t *d_runs = reinterpret_cast<uint64_t *>(g.d_scalar);
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(g.d_keys.reserve(slots * sizeof(u64)));
+    CUDA_CHECK(g.d_counts.reserve(slots * sizeof(uint32_t)));
+    CUDA_CHECK(g.d_scalar.reserve(16));
+    uint64_t *d_runs = reinterpret_cast<uint64_t *>(g.d_scalar.get());
     size_t bytes = 0, need = 0;
-    GLOVE_TRY(cub::DeviceRadixSort::SortKeys(nullptr, bytes, raw, sorted, slots, 0, 64, stream));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, raw, sorted, slots, 0, 64, stream));
     need = bytes;
-    GLOVE_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, bytes, sorted, g.d_keys, g.d_counts, d_runs, slots, stream));
+    CUDA_CHECK(cub::DeviceRunLengthEncode::Encode(nullptr, bytes, sorted, g.d_keys.get(), g.d_counts.get(), d_runs, slots, stream));
     need = std::max(need, bytes);
-    GLOVE_TRY(grow(&g.d_temp, &g.temp_bytes, need));
-    bytes = g.temp_bytes;
-    GLOVE_TRY(cub::DeviceRadixSort::SortKeys(g.d_temp, bytes, raw, sorted, slots, 0, 64, stream));
-    bytes = g.temp_bytes;
-    GLOVE_TRY(cub::DeviceRunLengthEncode::Encode(g.d_temp, bytes, sorted, g.d_keys, g.d_counts, d_runs, slots, stream));
+    CUDA_CHECK(g.d_temp.reserve(need));
+    bytes = g.d_temp.bytes();
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(g.d_temp.get(), bytes, raw, sorted, slots, 0, 64, stream));
+    bytes = g.d_temp.bytes();
+    CUDA_CHECK(cub::DeviceRunLengthEncode::Encode(g.d_temp.get(), bytes, sorted, g.d_keys.get(), g.d_counts.get(), d_runs, slots, stream));
     uint64_t runs = 0;
-    GLOVE_TRY(cudaMemcpyAsync(&runs, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
-    GLOVE_TRY(cudaStreamSynchronize(stream));
+    CUDA_CHECK(cudaMemcpyAsync(&runs, d_runs, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
     if (runs) {  // the all-ones key, if present, is the last run
         u64 last = 0;
-        GLOVE_TRY(cudaMemcpyAsync(&last, g.d_keys + runs - 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-        GLOVE_TRY(cudaStreamSynchronize(stream));
+        CUDA_CHECK(cudaMemcpyAsync(&last, g.d_keys.get() + runs - 1, sizeof(u64), cudaMemcpyDeviceToHost, stream));
+        CUDA_CHECK(cudaStreamSynchronize(stream));
         if (last == COOC_INVALID) --runs;
     }
     g.n_triples = runs;
     return cudaSuccess;
 }
 
-cudaError_t glove_reserve(void **ptr, size_t *have, size_t want) { return grow(ptr, have, want); }
-
 // largest count of the resident triples (0 when there are none)
-cudaError_t glove_max_count(GloveState &g, uint32_t *max_count, cudaStream_t stream) {
+cudaError_t glove_max_count(GloveState &g, uint32_t *max_count, cudaStream_t stream, std::string &error) {
     *max_count = 0;
     if (g.n_triples == 0) return cudaSuccess;
-    GLOVE_TRY(grow((void **)&g.d_scalar, &g.scalar_bytes, 16));
-    uint32_t *d_max = reinterpret_cast<uint32_t *>(g.d_scalar);
+    CUDA_CHECK(g.d_scalar.reserve(16));
+    uint32_t *d_max = reinterpret_cast<uint32_t *>(g.d_scalar.get());
     size_t bytes = 0;
-    GLOVE_TRY(cub::DeviceReduce::Max(nullptr, bytes, g.d_counts, d_max, g.n_triples, stream));
-    GLOVE_TRY(grow(&g.d_temp, &g.temp_bytes, bytes));
-    bytes = g.temp_bytes;
-    GLOVE_TRY(cub::DeviceReduce::Max(g.d_temp, bytes, g.d_counts, d_max, g.n_triples, stream));
-    GLOVE_TRY(cudaMemcpyAsync(max_count, d_max, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
-    return cudaStreamSynchronize(stream);
-}
-
-void glove_free(GloveState &g) {
-    cudaFree(g.d_keys); cudaFree(g.d_counts); cudaFree(g.d_rowptr); cudaFree(g.d_scratch_keys);
-    cudaFree(g.d_merge_keys); cudaFree(g.d_merge_counts); cudaFree(g.d_temp); cudaFree(g.d_scalar);
-    cudaFree(g.d_epoch_walks); cudaFree(g.d_histogram); cudaFree(g.d_bounds); cudaFree(g.d_positions);
-    cudaFree(g.d_cursor); cudaFree(g.d_t1_snapshot);
-    g = GloveState();
+    CUDA_CHECK(cub::DeviceReduce::Max(nullptr, bytes, g.d_counts.get(), d_max, g.n_triples, stream));
+    CUDA_CHECK(g.d_temp.reserve(bytes));
+    bytes = g.d_temp.bytes();
+    CUDA_CHECK(cub::DeviceReduce::Max(g.d_temp.get(), bytes, g.d_counts.get(), d_max, g.n_triples, stream));
+    CUDA_CHECK(cudaMemcpyAsync(max_count, d_max, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
+    return cudaSuccess;
 }
 
 }  // namespace b2e

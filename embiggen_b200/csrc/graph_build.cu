@@ -16,34 +16,13 @@
 #include <algorithm>
 #include <string>
 
-#include "common.cuh"
+#include "host.cuh"
 
 namespace b2e {
 
 constexpr uint32_t TAG_ER = 0x10u;    // graph.py: erdos_renyi
 constexpr uint32_t TAG_RMAT = 0x11u;  // graph.py: rmat
 constexpr unsigned long long INVALID_KEY = ~0ull;
-
-struct DeviceBuffer {
-    void *ptr = nullptr;
-    size_t bytes = 0;
-    ~DeviceBuffer() { cudaFree(ptr); }
-    cudaError_t reserve(size_t want) {
-        if (want <= bytes) return cudaSuccess;
-        cudaFree(ptr);
-        ptr = nullptr;
-        bytes = 0;
-        cudaError_t e = cudaMalloc(&ptr, want);
-        if (e == cudaSuccess) bytes = want;
-        return e;
-    }
-    void release() {
-        cudaFree(ptr);
-        ptr = nullptr;
-        bytes = 0;
-    }
-    template <typename T> T *as() { return static_cast<T *>(ptr); }
-};
 
 // candidate undirected edge of draw `idx`: key = (min << 32) | max, INVALID_KEY if rejected
 __global__ void __launch_bounds__(256) draw_edges_kernel(int kind, uint64_t n, uint32_t scale,
@@ -123,88 +102,77 @@ __global__ void __launch_bounds__(256) csr_from_keys_kernel(const unsigned long 
 
 static inline unsigned blocks_for(uint64_t count) { return (unsigned)((count + 255) / 256); }
 
-#define GB_TRY(expr)                                                          \
-    do {                                                                      \
-        cudaError_t _e = (expr);                                              \
-        if (_e != cudaSuccess) {                                              \
-            error = std::string(#expr) + ": " + cudaGetErrorString(_e);       \
-            return _e;                                                        \
-        }                                                                     \
-    } while (0)
-
 // stable radix sort of (keys, values) by key; results land in keys_out / values_out
-static cudaError_t sort_pairs(DeviceBuffer &temp, const unsigned long long *keys_in,
+static cudaError_t sort_pairs(DeviceBuffer<> &temp, const unsigned long long *keys_in,
                               unsigned long long *keys_out, const unsigned long long *values_in,
                               unsigned long long *values_out, uint64_t count, std::string &error) {
     size_t bytes = 0;
-    GB_TRY(cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys_in, keys_out, values_in, values_out, count));
-    GB_TRY(temp.reserve(bytes));
-    GB_TRY(cub::DeviceRadixSort::SortPairs(temp.ptr, bytes, keys_in, keys_out, values_in, values_out, count));
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, keys_in, keys_out, values_in, values_out, count));
+    CUDA_CHECK(temp.reserve(bytes));
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairs(temp.get(), bytes, keys_in, keys_out, values_in, values_out, count));
     return cudaSuccess;
 }
 
-static cudaError_t sort_keys(DeviceBuffer &temp, const unsigned long long *keys_in,
+static cudaError_t sort_keys(DeviceBuffer<> &temp, const unsigned long long *keys_in,
                              unsigned long long *keys_out, uint64_t count, std::string &error) {
     size_t bytes = 0;
-    GB_TRY(cub::DeviceRadixSort::SortKeys(nullptr, bytes, keys_in, keys_out, count));
-    GB_TRY(temp.reserve(bytes));
-    GB_TRY(cub::DeviceRadixSort::SortKeys(temp.ptr, bytes, keys_in, keys_out, count));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, keys_in, keys_out, count));
+    CUDA_CHECK(temp.reserve(bytes));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(temp.get(), bytes, keys_in, keys_out, count));
     return cudaSuccess;
 }
 
 // directed keys (any order) -> CSR in device buffers.  `scratch` is the alternate buffer of the
 // radix sort (no third copy).  With `dedup` the keys may repeat and contain INVALID_KEY.
-static cudaError_t keys_to_csr(DeviceBuffer &temp, unsigned long long *keys, unsigned long long *scratch,
-                               uint64_t count, uint64_t n, bool dedup, DeviceBuffer &d_indptr,
-                               DeviceBuffer &d_indices, uint64_t *nnz_out, std::string &error) {
+static cudaError_t keys_to_csr(DeviceBuffer<> &temp, unsigned long long *keys, unsigned long long *scratch,
+                               uint64_t count, uint64_t n, bool dedup, DeviceBuffer<int64_t> &d_indptr,
+                               DeviceBuffer<uint32_t> &d_indices, uint64_t *nnz_out, std::string &error) {
     cub::DoubleBuffer<unsigned long long> buffers(keys, scratch);
     size_t bytes = 0;
-    GB_TRY(cub::DeviceRadixSort::SortKeys(nullptr, bytes, buffers, count));
-    GB_TRY(temp.reserve(bytes));
-    GB_TRY(cub::DeviceRadixSort::SortKeys(temp.ptr, bytes, buffers, count));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, buffers, count));
+    CUDA_CHECK(temp.reserve(bytes));
+    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(temp.get(), bytes, buffers, count));
     unsigned long long *sorted = buffers.Current(), *other = buffers.Alternate();
     uint64_t nnz = count;
     if (dedup) {
-        DeviceBuffer selected;
-        GB_TRY(selected.reserve(sizeof(unsigned long long)));
-        GB_TRY(cub::DeviceSelect::Unique(nullptr, bytes, sorted, other, selected.as<unsigned long long>(), count));
-        GB_TRY(temp.reserve(bytes));
-        GB_TRY(cub::DeviceSelect::Unique(temp.ptr, bytes, sorted, other, selected.as<unsigned long long>(), count));
+        DeviceBuffer<unsigned long long> selected;
+        CUDA_CHECK(selected.reserve(sizeof(unsigned long long)));
+        CUDA_CHECK(cub::DeviceSelect::Unique(nullptr, bytes, sorted, other, selected.get(), count));
+        CUDA_CHECK(temp.reserve(bytes));
+        CUDA_CHECK(cub::DeviceSelect::Unique(temp.get(), bytes, sorted, other, selected.get(), count));
         unsigned long long unique = 0, last = 0;
-        GB_TRY(cudaMemcpy(&unique, selected.ptr, sizeof(unique), cudaMemcpyDeviceToHost));
-        if (unique) GB_TRY(cudaMemcpy(&last, other + unique - 1, sizeof(last), cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(&unique, selected.get(), sizeof(unique), cudaMemcpyDeviceToHost));
+        if (unique) CUDA_CHECK(cudaMemcpy(&last, other + unique - 1, sizeof(last), cudaMemcpyDeviceToHost));
         nnz = unique - ((unique && last == INVALID_KEY) ? 1 : 0);
         sorted = other;
     }
     *nnz_out = nnz;
-    GB_TRY(d_indices.reserve(std::max<uint64_t>(nnz, 1) * sizeof(uint32_t)));
-    GB_TRY(d_indptr.reserve((n + 1) * sizeof(long long)));
+    CUDA_CHECK(d_indices.reserve(std::max<uint64_t>(nnz, 1) * sizeof(uint32_t)));
+    CUDA_CHECK(d_indptr.reserve((n + 1) * sizeof(long long)));
     csr_from_keys_kernel<<<blocks_for(std::max<uint64_t>(nnz, n + 1)), 256>>>(
-        sorted, nnz, n, d_indices.as<uint32_t>(), d_indptr.as<long long>());
-    GB_TRY(cudaGetLastError());
-    GB_TRY(cudaDeviceSynchronize());
+        sorted, nnz, n, d_indices.get(), reinterpret_cast<long long *>(d_indptr.get()));
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaDeviceSynchronize());
     return cudaSuccess;
 }
 
 // hand the device arrays over: to host buffers, or (out != nullptr) to a resident b2e_graph
-static cudaError_t deliver(DeviceBuffer &d_indptr, DeviceBuffer &d_indices, uint64_t n, uint64_t nnz,
+static cudaError_t deliver(DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<uint32_t> &d_indices, uint64_t n, uint64_t nnz,
                            int64_t *indptr, uint32_t *indices, uint64_t capacity, ResidentCsr *out,
                            std::string &error) {
     if (out) {
-        out->indptr = d_indptr.as<int64_t>();
-        out->indices = d_indices.as<uint32_t>();
+        out->indptr = std::move(d_indptr);
+        out->indices = std::move(d_indices);
         out->n = n;
         out->nnz = nnz;
-        d_indptr.ptr = d_indices.ptr = nullptr;  // ownership moves
-        d_indptr.bytes = d_indices.bytes = 0;
         return cudaSuccess;
     }
     if (nnz > capacity) {
         error = "indices buffer too small for the de-duplicated graph";
         return cudaErrorInvalidValue;
     }
-    GB_TRY(cudaMemcpy(indptr, d_indptr.ptr, (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost));
-    if (nnz) GB_TRY(cudaMemcpy(indices, d_indices.ptr, nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(indptr, d_indptr.get(), (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost));
+    if (nnz) CUDA_CHECK(cudaMemcpy(indices, d_indices.get(), nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return cudaSuccess;
 }
 
@@ -212,31 +180,35 @@ cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_
                            int symmetrise, int64_t *indptr, uint32_t *indices, uint64_t capacity,
                            uint64_t *nnz_out, std::string &error, ResidentCsr *resident) {
     const uint64_t count = n_edges * (symmetrise ? 2 : 1);
-    DeviceBuffer d_src, d_dst, keys, scratch, temp, flag;
-    GB_TRY(d_src.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(uint32_t)));
-    GB_TRY(d_dst.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(uint32_t)));
-    GB_TRY(keys.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
-    GB_TRY(scratch.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
-    GB_TRY(flag.reserve(sizeof(int)));
-    GB_TRY(cudaMemset(flag.ptr, 0, sizeof(int)));
-    GB_TRY(cudaMemcpy(d_src.ptr, src, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
-    GB_TRY(cudaMemcpy(d_dst.ptr, dst, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    DeviceBuffer<uint32_t> d_src, d_dst;
+    DeviceBuffer<unsigned long long> keys, scratch;
+    DeviceBuffer<> temp;
+    DeviceBuffer<int> flag;
+    CUDA_CHECK(d_src.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(uint32_t)));
+    CUDA_CHECK(d_dst.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(uint32_t)));
+    CUDA_CHECK(keys.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
+    CUDA_CHECK(scratch.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
+    CUDA_CHECK(flag.reserve(sizeof(int)));
+    CUDA_CHECK(cudaMemset(flag.get(), 0, sizeof(int)));
+    CUDA_CHECK(cudaMemcpy(d_src.get(), src, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    CUDA_CHECK(cudaMemcpy(d_dst.get(), dst, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
     if (n_edges) {
-        edge_keys_kernel<<<blocks_for(n_edges), 256>>>(d_src.as<uint32_t>(), d_dst.as<uint32_t>(), n_edges, n,
-                                                       symmetrise, keys.as<unsigned long long>(),
-                                                       flag.as<int>());
-        GB_TRY(cudaGetLastError());
+        edge_keys_kernel<<<blocks_for(n_edges), 256>>>(d_src.get(), d_dst.get(), n_edges, n,
+                                                       symmetrise, keys.get(),
+                                                       flag.get());
+        CUDA_CHECK(cudaGetLastError());
     }
     int out_of_range = 0;
-    GB_TRY(cudaMemcpy(&out_of_range, flag.ptr, sizeof(int), cudaMemcpyDeviceToHost));
+    CUDA_CHECK(cudaMemcpy(&out_of_range, flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
     if (out_of_range) {
         error = "an edge endpoint is not below the number of nodes";
         return cudaErrorInvalidValue;
     }
-    d_src.release();
-    d_dst.release();
-    DeviceBuffer d_indptr, d_indices;
-    GB_TRY(keys_to_csr(temp, keys.as<unsigned long long>(), scratch.as<unsigned long long>(), count, n, true,
+    d_src.reset();
+    d_dst.reset();
+    DeviceBuffer<int64_t> d_indptr;
+    DeviceBuffer<uint32_t> d_indices;
+    CUDA_CHECK(keys_to_csr(temp, keys.get(), scratch.get(), count, n, true,
                        d_indptr, d_indices, nnz_out, error));
     return deliver(d_indptr, d_indices, n, *nnz_out, indptr, indices, capacity, resident, error);
 }
@@ -257,12 +229,12 @@ __global__ void __launch_bounds__(256) new_key_flags_kernel(const unsigned long 
 }
 
 template <typename T>
-static cudaError_t select_flagged(DeviceBuffer &temp, const T *in, const unsigned char *flags, T *out,
+static cudaError_t select_flagged(DeviceBuffer<> &temp, const T *in, const unsigned char *flags, T *out,
                                   unsigned long long *d_count, uint64_t count, std::string &error) {
     size_t bytes = 0;
-    GB_TRY(cub::DeviceSelect::Flagged(nullptr, bytes, in, flags, out, d_count, count));
-    GB_TRY(temp.reserve(bytes));
-    GB_TRY(cub::DeviceSelect::Flagged(temp.ptr, bytes, in, flags, out, d_count, count));
+    CUDA_CHECK(cub::DeviceSelect::Flagged(nullptr, bytes, in, flags, out, d_count, count));
+    CUDA_CHECK(temp.reserve(bytes));
+    CUDA_CHECK(cub::DeviceSelect::Flagged(temp.get(), bytes, in, flags, out, d_count, count));
     return cudaSuccess;
 }
 
@@ -278,11 +250,13 @@ cudaError_t synthetic_csr(int kind, uint64_t n, uint32_t scale, uint64_t m, uint
                           std::string &error, ResidentCsr *resident) {
     typedef unsigned long long u64;
     const uint64_t batch_max = 1ull << 29;
-    DeviceBuffer pool[2], keys_in, ids_in, keys_sorted, ids_sorted, keys_unique, ids_unique, keys_new,
-        ids_new, flags, temp, d_count;
-    GB_TRY(d_count.reserve(sizeof(u64)));
-    GB_TRY(pool[0].reserve(std::max<uint64_t>(m, 1) * sizeof(u64)));
-    GB_TRY(pool[1].reserve(std::max<uint64_t>(m, 1) * sizeof(u64)));
+    DeviceBuffer<u64> pool[2], keys_in, ids_in, keys_sorted, ids_sorted, keys_unique, ids_unique, keys_new,
+        ids_new, d_count;
+    DeviceBuffer<unsigned char> flags;
+    DeviceBuffer<> temp;
+    CUDA_CHECK(d_count.reserve(sizeof(u64)));
+    CUDA_CHECK(pool[0].reserve(std::max<uint64_t>(m, 1) * sizeof(u64)));
+    CUDA_CHECK(pool[1].reserve(std::max<uint64_t>(m, 1) * sizeof(u64)));
     int cur = 0;
     uint64_t have = 0, drawn = 0;
     for (int round = 0; have < m; ++round) {
@@ -291,76 +265,74 @@ cudaError_t synthetic_csr(int kind, uint64_t n, uint32_t scale, uint64_t m, uint
             return cudaErrorInvalidValue;
         }
         const uint64_t want = std::min<uint64_t>(batch_max, (uint64_t)((double)(m - have) * 1.3) + 1024);
-        for (DeviceBuffer *buffer : {&keys_in, &ids_in, &keys_sorted, &ids_sorted, &keys_unique, &ids_unique,
-                                     &keys_new, &ids_new})
-            GB_TRY(buffer->reserve(want * sizeof(u64)));
-        GB_TRY(flags.reserve(want));
+        for (DeviceBuffer<u64> *buffer : {&keys_in, &ids_in, &keys_sorted, &ids_sorted, &keys_unique, &ids_unique,
+                                          &keys_new, &ids_new})
+            CUDA_CHECK(buffer->reserve(want * sizeof(u64)));
+        CUDA_CHECK(flags.reserve(want));
         draw_edges_kernel<<<blocks_for(want), 256>>>(kind, n, scale, (uint32_t)seed, (uint32_t)(seed >> 32),
-                                                     t_a, t_ab, t_abc, drawn, want, keys_in.as<u64>(),
-                                                     ids_in.as<u64>());
-        GB_TRY(cudaGetLastError());
+                                                     t_a, t_ab, t_abc, drawn, want, keys_in.get(),
+                                                     ids_in.get());
+        CUDA_CHECK(cudaGetLastError());
         drawn += want;
         // stable sort by key: equal keys stay in ascending draw order, so "first" = earliest draw
-        GB_TRY(sort_pairs(temp, keys_in.as<u64>(), keys_sorted.as<u64>(), ids_in.as<u64>(),
-                          ids_sorted.as<u64>(), want, error));
+        CUDA_CHECK(sort_pairs(temp, keys_in.get(), keys_sorted.get(), ids_in.get(),
+                          ids_sorted.get(), want, error));
         size_t bytes = 0;
-        GB_TRY(cub::DeviceSelect::UniqueByKey(nullptr, bytes, keys_sorted.as<u64>(), ids_sorted.as<u64>(),
-                                              keys_unique.as<u64>(), ids_unique.as<u64>(), d_count.as<u64>(),
+        CUDA_CHECK(cub::DeviceSelect::UniqueByKey(nullptr, bytes, keys_sorted.get(), ids_sorted.get(),
+                                              keys_unique.get(), ids_unique.get(), d_count.get(),
                                               want));
-        GB_TRY(temp.reserve(bytes));
-        GB_TRY(cub::DeviceSelect::UniqueByKey(temp.ptr, bytes, keys_sorted.as<u64>(), ids_sorted.as<u64>(),
-                                              keys_unique.as<u64>(), ids_unique.as<u64>(), d_count.as<u64>(),
+        CUDA_CHECK(temp.reserve(bytes));
+        CUDA_CHECK(cub::DeviceSelect::UniqueByKey(temp.get(), bytes, keys_sorted.get(), ids_sorted.get(),
+                                              keys_unique.get(), ids_unique.get(), d_count.get(),
                                               want));
         u64 unique = 0;
-        GB_TRY(cudaMemcpy(&unique, d_count.ptr, sizeof(unique), cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(&unique, d_count.get(), sizeof(unique), cudaMemcpyDeviceToHost));
         if (unique == 0) continue;
-        new_key_flags_kernel<<<blocks_for(unique), 256>>>(keys_unique.as<u64>(), unique, pool[cur].as<u64>(),
-                                                          have, flags.as<unsigned char>());
-        GB_TRY(cudaGetLastError());
-        GB_TRY(select_flagged(temp, keys_unique.as<u64>(), flags.as<unsigned char>(), keys_new.as<u64>(),
-                              d_count.as<u64>(), unique, error));
-        GB_TRY(select_flagged(temp, ids_unique.as<u64>(), flags.as<unsigned char>(), ids_new.as<u64>(),
-                              d_count.as<u64>(), unique, error));
+        new_key_flags_kernel<<<blocks_for(unique), 256>>>(keys_unique.get(), unique, pool[cur].get(),
+                                                          have, flags.get());
+        CUDA_CHECK(cudaGetLastError());
+        CUDA_CHECK(select_flagged(temp, keys_unique.get(), flags.get(), keys_new.get(),
+                              d_count.get(), unique, error));
+        CUDA_CHECK(select_flagged(temp, ids_unique.get(), flags.get(), ids_new.get(),
+                              d_count.get(), unique, error));
         u64 fresh = 0;
-        GB_TRY(cudaMemcpy(&fresh, d_count.ptr, sizeof(fresh), cudaMemcpyDeviceToHost));
+        CUDA_CHECK(cudaMemcpy(&fresh, d_count.get(), sizeof(fresh), cudaMemcpyDeviceToHost));
         if (fresh == 0) continue;
         if (have + fresh > m) {  // the last batch overshoots: keep its m - have earliest draws
             const uint64_t keep = m - have;
-            GB_TRY(sort_pairs(temp, ids_new.as<u64>(), ids_sorted.as<u64>(), keys_new.as<u64>(),
-                              keys_sorted.as<u64>(), fresh, error));
-            GB_TRY(sort_keys(temp, keys_sorted.as<u64>(), keys_new.as<u64>(), keep, error));
+            CUDA_CHECK(sort_pairs(temp, ids_new.get(), ids_sorted.get(), keys_new.get(),
+                              keys_sorted.get(), fresh, error));
+            CUDA_CHECK(sort_keys(temp, keys_sorted.get(), keys_new.get(), keep, error));
             fresh = keep;
         }
-        GB_TRY(cub::DeviceMerge::MergeKeys(nullptr, bytes, pool[cur].as<u64>(), (int64_t)have,
-                                           keys_new.as<u64>(), (int64_t)fresh, pool[cur ^ 1].as<u64>()));
-        GB_TRY(temp.reserve(bytes));
-        GB_TRY(cub::DeviceMerge::MergeKeys(temp.ptr, bytes, pool[cur].as<u64>(), (int64_t)have,
-                                           keys_new.as<u64>(), (int64_t)fresh, pool[cur ^ 1].as<u64>()));
+        CUDA_CHECK(cub::DeviceMerge::MergeKeys(nullptr, bytes, pool[cur].get(), (int64_t)have,
+                                           keys_new.get(), (int64_t)fresh, pool[cur ^ 1].get()));
+        CUDA_CHECK(temp.reserve(bytes));
+        CUDA_CHECK(cub::DeviceMerge::MergeKeys(temp.get(), bytes, pool[cur].get(), (int64_t)have,
+                                           keys_new.get(), (int64_t)fresh, pool[cur ^ 1].get()));
         cur ^= 1;
         have += fresh;
     }
-    for (DeviceBuffer *buffer : {&keys_in, &ids_in, &keys_sorted, &ids_sorted, &keys_unique, &ids_unique,
-                                 &keys_new, &ids_new, &flags, &pool[cur ^ 1]}) {
-        cudaFree(buffer->ptr);
-        buffer->ptr = nullptr;
-        buffer->bytes = 0;
-    }
+    for (DeviceBuffer<u64> *buffer : {&keys_in, &ids_in, &keys_sorted, &ids_sorted, &keys_unique, &ids_unique,
+                                      &keys_new, &ids_new})
+        buffer->reset();
+    flags.reset();
+    pool[cur ^ 1].reset();
     // both directions, sorted -> CSR
-    DeviceBuffer directed, alternate;
-    GB_TRY(directed.reserve(2 * have * sizeof(u64)));
-    mirror_keys_kernel<<<blocks_for(have), 256>>>(pool[cur].as<u64>(), have, directed.as<u64>());
-    GB_TRY(cudaGetLastError());
-    GB_TRY(cudaDeviceSynchronize());
-    cudaFree(pool[cur].ptr);
-    pool[cur].ptr = nullptr;
-    pool[cur].bytes = 0;
-    GB_TRY(alternate.reserve(2 * have * sizeof(u64)));
-    DeviceBuffer d_indptr, d_indices;
-    GB_TRY(keys_to_csr(temp, directed.as<u64>(), alternate.as<u64>(), 2 * have, n, false, d_indptr, d_indices,
+    DeviceBuffer<u64> directed, alternate;
+    CUDA_CHECK(directed.reserve(2 * have * sizeof(u64)));
+    mirror_keys_kernel<<<blocks_for(have), 256>>>(pool[cur].get(), have, directed.get());
+    CUDA_CHECK(cudaGetLastError());
+    CUDA_CHECK(cudaDeviceSynchronize());
+    pool[cur].reset();
+    CUDA_CHECK(alternate.reserve(2 * have * sizeof(u64)));
+    DeviceBuffer<int64_t> d_indptr;
+    DeviceBuffer<uint32_t> d_indices;
+    CUDA_CHECK(keys_to_csr(temp, directed.get(), alternate.get(), 2 * have, n, false, d_indptr, d_indices,
                        nnz_out, error));
-    directed.release();
-    alternate.release();
-    temp.release();
+    directed.reset();
+    alternate.reset();
+    temp.reset();
     return deliver(d_indptr, d_indices, n, *nnz_out, indptr, indices, capacity, resident, error);
 }
 

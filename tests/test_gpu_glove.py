@@ -61,7 +61,7 @@ def test_glove_deterministic_bit_exact(small_ppi, D, alpha):
     assert np.isclose(counters["loss_sum"], stats["loss_sum"], rtol=1e-4)
 
 
-def test_glove_fit_tracks_the_oracle(small_ppi):
+def test_glove_fit_tracks_the_oracle(small_ppi, rmat_graph):
     kw = dict(embedding_size=32, epochs=8, walk_length=64, window_size=4, learning_rate=0.05,
               learning_rate_decay=0.9)
     _, _, expected = oracle.glove_fit(small_ppi.indptr, small_ppi.indices, 5, alpha=0.75,
@@ -80,11 +80,17 @@ def test_glove_fit_tracks_the_oracle(small_ppi):
     # deterministic launch: the same tables as the oracle, whole path
     t0, t1, _ = oracle.glove_fit(small_ppi.indptr, small_ppi.indices, 5, alpha=0.75,
                                  return_weight=0.25, explore_weight=4.0, **dict(kw, epochs=2))
-    with Engine("GloVe", return_weight=0.25, explore_weight=4.0, iterations=1, deterministic=True,
-                **dict(kw, epochs=2)) as engine:
+    deterministic = dict(kw, epochs=2, return_weight=0.25, explore_weight=4.0, iterations=1, deterministic=True)
+    with Engine("GloVe", **deterministic) as engine:
         engine.load_csr(small_ppi.indptr, small_ppi.indices)
         c, x, _ = engine.fit(5)
-    assert np.array_equal(c, t0[:, :32]) and np.array_equal(x, t1[:, :32])
+        assert np.array_equal(c, t0[:, :32]) and np.array_equal(x, t1[:, :32])
+        engine.load_csr(rmat_graph.indptr, rmat_graph.indices)  # the first graph's GloVe state goes with it
+        reloaded = engine.fit(5)[:2]
+    with Engine("GloVe", **deterministic) as engine:
+        engine.load_csr(rmat_graph.indptr, rmat_graph.indices)
+        fresh = engine.fit(5)[:2]
+    assert all(np.array_equal(a, b) for a, b in zip(reloaded, fresh))
 
 
 def test_glove_embedders(small_ppi):

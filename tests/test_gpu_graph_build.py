@@ -89,10 +89,25 @@ def test_resident_graph_equals_host_graph_and_walks_identically(small_ppi):
     assert same_graph(small_ppi, device_graph_from_edges(src, small_ppi.indices, 1064).to_host())
     # walks on the resident CSR == walks on the uploaded CSR == the oracle's
     want, _ = oracle.walks(expected.indptr, expected.indices, 3, 0, 3000, 40, 2.0, 0.5)
-    with Engine("SkipGram", walk_length=40, return_weight=2.0, explore_weight=0.5) as engine:
-        engine.load_graph(resident)
-        resident.close()  # reference counted: the engine keeps the arrays alive
+    kw = dict(walk_length=40, return_weight=2.0, explore_weight=0.5)
+    with Engine("SkipGram", **kw) as engine:
+        engine.load_csr(expected.indptr, expected.indices)  # a host graph, then the resident one
         assert np.array_equal(engine.walks(3, 0, 3000), want)
+        engine.load_graph(resident)
+        assert np.array_equal(engine.walks(3, 0, 3000), want)
+        malformed = expected.indices.copy()
+        malformed[0] = 4000  # an id out of range: found on the device, after the resident graph was let go
+        with pytest.raises(ValueError):
+            engine.load_csr(expected.indptr, malformed)
+        with pytest.raises(RuntimeError):
+            engine.walks(3, 0, 3000)  # a failed load leaves the engine without a graph
+        engine.load_graph(resident)
+        assert np.array_equal(engine.walks(3, 0, 3000), want)
+        with Engine("SkipGram", **kw) as other:  # two engines on one resident graph
+            other.load_graph(resident)
+            resident.close()  # reference counted: the engines keep the arrays alive
+            assert np.array_equal(other.walks(3, 0, 3000), want)
+        assert np.array_equal(engine.walks(3, 0, 3000), want)  # `other` let go, this one walks on
         engine.load_csr(expected.indptr, expected.indices)  # and a host graph can replace it
         assert np.array_equal(engine.walks(3, 0, 3000), want)
 
