@@ -135,6 +135,7 @@ SIGNATURES = {
     "b2e_export_tables": (ctypes.c_int, [_H, ctypes.c_void_p, ctypes.c_void_p]),
     "b2e_import_tables": (ctypes.c_int, [_H, ctypes.c_void_p, ctypes.c_void_p]),
     "b2e_export_alias": (ctypes.c_int, [_H, ctypes.c_void_p, ctypes.c_void_p]),
+    "b2e_export_edge_alias": (ctypes.c_int, [_H, ctypes.c_void_p]),
     "b2e_counters_read": (ctypes.c_int, [_H, _P(B2ECounters)]),
     "b2e_counters_reset": (ctypes.c_int, [_H]),
     "b2e_launch_count": (_U64, [_H]),
@@ -153,15 +154,24 @@ SIGNATURES = {
                                               ctypes.c_void_p, ctypes.c_void_p]),
     "b2e_graph_from_edges": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, _U64, _U64,
                                             ctypes.c_int, _P(_H)]),
+    "b2e_graph_from_edges_weighted": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                     ctypes.c_void_p, _U64, _U64, ctypes.c_int, _P(_H)]),
     "b2e_graph_synthetic": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, _U64, _U32, _U64, _U64, _U64, _U64,
                                            _U64, _P(_H)]),
     "b2e_graph_from_csr": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, _U64, _U64, _P(_H)]),
+    "b2e_graph_from_csr_weighted": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                   ctypes.c_void_p, _U64, _U64, _P(_H)]),
     "b2e_graph_shape": (ctypes.c_int, [_H, _P(_U64), _P(_U64)]),
     "b2e_graph_export": (ctypes.c_int, [_H, ctypes.c_void_p, ctypes.c_void_p]),
+    "b2e_graph_weighted": (ctypes.c_int, [_H]),
+    "b2e_graph_export_weights": (ctypes.c_int, [_H, ctypes.c_void_p]),
     "b2e_graph_destroy": (None, [_H]),
     "b2e_load_graph": (ctypes.c_int, [_H, _H]),
     "b2e_csr_from_edges": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, _U64, _U64,
                                           ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, _U64, _P(_U64)]),
+    "b2e_csr_from_edges_weighted": (ctypes.c_int, [ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                                   ctypes.c_void_p, _U64, _U64, ctypes.c_int, ctypes.c_void_p,
+                                                   ctypes.c_void_p, ctypes.c_void_p, _U64, _P(_U64)]),
     "b2e_synthetic_csr": (ctypes.c_int, [ctypes.c_int, ctypes.c_int, _U64, _U32, _U64, _U64, _U64, _U64,
                                          _U64, ctypes.c_void_p, ctypes.c_void_p, _U64, _P(_U64)]),
 }

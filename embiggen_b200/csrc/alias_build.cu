@@ -309,4 +309,145 @@ cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indpt
     return cudaSuccess;
 }
 
+
+// ---- per-row alias tables of a weighted graph (the proposal of weighted walks) ----
+// The normative construction is oracle/walks.c: orc_edge_alias, reproduced bit for bit: per row of
+// d edges, total = the left-to-right double sum of its weights, heaviest = the first index of the
+// strict maximum, scaled_i = w_i d / total (1 when total is 0), small / large = LIFO stacks filled
+// in ascending edge order, thr = min(floor(scaled 2^32), 2^32 - 1), leftovers {2^32 - 1, self}
+// except a zero-weight leftover, {0, heaviest}.  The double operations are the _rn intrinsics so
+// that nothing is contracted into an FMA.  LIFO Vose is sequential within a row, so one thread
+// builds one row; the threads take the rows longest first (the longest row is the critical path).
+// Each row keeps its open scaled_i in its own 8-byte output slot, which becomes {thr, alias} when
+// entry i closes, and both stacks in one two-ended array of 4 B per edge at the row's offset:
+// small grows up from the front, large down from the back (|small| + |large| <= d).
+
+__global__ void __launch_bounds__(256) row_degree_kernel(const int64_t *__restrict__ indptr, uint64_t n,
+                                                         uint32_t *__restrict__ degree, uint32_t *__restrict__ row) {
+    const uint64_t v = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= n) return;
+    degree[v] = (uint32_t)(indptr[v + 1] - indptr[v]);
+    row[v] = (uint32_t)v;
+}
+
+// a table slot: low word thr, high word alias (the layout of uint2 {x = thr, y = alias})
+__device__ __forceinline__ unsigned long long edge_entry(uint32_t thr, uint32_t alias) {
+    return ((unsigned long long)alias << 32) | thr;
+}
+
+__global__ void __launch_bounds__(128) edge_alias_kernel(const int64_t *__restrict__ indptr,
+                                                         const uint32_t *__restrict__ order, uint64_t n,
+                                                         const float *__restrict__ weights,
+                                                         unsigned long long *__restrict__ table,
+                                                         uint32_t *__restrict__ stacks, int *flags) {
+    const uint64_t t = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n) return;
+    const uint32_t v = order[t];
+    const int64_t begin = indptr[v];
+    const uint64_t d = (uint64_t)(indptr[v + 1] - begin);
+    if (d == 0) return;
+    const float *w = weights + begin;
+    unsigned long long *slot = table + begin;
+    uint32_t *stack = stacks + begin;
+    double total = 0.0;
+    uint64_t heaviest = 0;
+    float w_heaviest = w[0];
+    for (uint64_t i = 0; i < d; ++i) {
+        const float wi = w[i];
+        if (!(wi >= 0.0f)) {  // negative or NaN
+            atomicOr(flags, 1);
+            return;
+        }
+        total = __dadd_rn(total, (double)wi);
+        if (wi > w_heaviest) {
+            heaviest = i;
+            w_heaviest = wi;
+        }
+    }
+    const double dd = (double)d;
+    uint64_t ns = 0, nl = 0;  // small: stack[0, ns); large: stack[d - nl, d), top at stack[d - nl]
+    for (uint64_t i = 0; i < d; ++i) {
+        const double scaled = total > 0.0 ? __ddiv_rn(__dmul_rn((double)w[i], dd), total) : 1.0;
+        slot[i] = (unsigned long long)__double_as_longlong(scaled);
+        if (scaled < 1.0) stack[ns++] = (uint32_t)i; else stack[d - 1 - nl++] = (uint32_t)i;
+    }
+    while (ns > 0 && nl > 0) {
+        const uint32_t s = stack[--ns];
+        const uint32_t l = stack[d - nl];
+        --nl;
+        const double scaled_s = __longlong_as_double((long long)slot[s]);
+        const double thr = floor(__dmul_rn(scaled_s, 4294967296.0));
+        slot[s] = edge_entry(thr >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)thr, l);
+        const double scaled_l = __dsub_rn(__dadd_rn(__longlong_as_double((long long)slot[l]), scaled_s), 1.0);
+        slot[l] = (unsigned long long)__double_as_longlong(scaled_l);
+        if (scaled_l < 1.0) stack[ns++] = l; else stack[d - 1 - nl++] = l;
+    }
+    for (uint64_t k = 0; k < ns; ++k) {  // leftovers of weight zero are never proposed
+        const uint32_t s = stack[k];
+        slot[s] = total > 0.0 && w[s] == 0.0f ? edge_entry(0u, (uint32_t)heaviest) : edge_entry(0xFFFFFFFFu, s);
+    }
+    for (uint64_t k = 0; k < nl; ++k) {
+        const uint32_t l = stack[d - 1 - k];
+        slot[l] = edge_entry(0xFFFFFFFFu, l);
+    }
+}
+
+// normalize_by_degree (oracle: degree_normalised_weights): one IEEE float division per edge
+__global__ void __launch_bounds__(256) degree_normalise_kernel(const int64_t *__restrict__ indptr,
+                                                               const uint32_t *__restrict__ indices,
+                                                               const float *__restrict__ weights, uint64_t nnz,
+                                                               float *__restrict__ out) {
+    const uint64_t e = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= nnz) return;
+    const uint32_t x = indices[e];
+    const long long degree = (long long)(indptr[x + 1] - indptr[x]);
+    out[e] = __fdiv_rn(weights ? weights[e] : 1.0f, (float)(degree > 1 ? degree : 1));
+}
+
+cudaError_t launch_degree_normalise(const int64_t *d_indptr, const uint32_t *d_indices, const float *d_weights,
+                                    uint64_t nnz, float *d_out, cudaStream_t stream) {
+    if (nnz == 0) return cudaSuccess;
+    degree_normalise_kernel<<<grid_for(nnz), 256, 0, stream>>>(d_indptr, d_indices, d_weights, nnz, d_out);
+    return cudaGetLastError();
+}
+
+// Device memory beyond the table (8 B per edge): 4 B per edge of stacks and 16 B per node for the
+// degree-sorted row order.
+cudaError_t build_edge_alias(const int64_t *d_indptr, const float *d_weights, uint64_t n, uint64_t nnz,
+                             uint2 *d_table, uint64_t *longest_row, cudaStream_t stream, std::string &error) {
+    DeviceBuffer<uint32_t> degree, degree_sorted, row, order, stacks;
+    DeviceBuffer<int> flags;
+    DeviceBuffer<> temp;
+    CUDA_CHECK(degree.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(degree_sorted.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(row.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(order.reserve(n * sizeof(uint32_t)));
+    CUDA_CHECK(stacks.reserve(std::max<uint64_t>(nnz, 1) * sizeof(uint32_t)));
+    CUDA_CHECK(flags.reserve(sizeof(int)));
+    CUDA_CHECK(cudaMemsetAsync(flags.get(), 0, sizeof(int), stream));
+    row_degree_kernel<<<grid_for(n), 256, 0, stream>>>(d_indptr, n, degree.get(), row.get());
+    CUDA_CHECK(cudaGetLastError());
+    size_t bytes = 0;
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(nullptr, bytes, degree.get(), degree_sorted.get(), row.get(),
+                                                         order.get(), n, 0, 32, stream));
+    CUDA_CHECK(temp.reserve(std::max<size_t>(bytes, 1)));
+    CUDA_CHECK(cub::DeviceRadixSort::SortPairsDescending(temp.get(), bytes, degree.get(), degree_sorted.get(),
+                                                         row.get(), order.get(), n, 0, 32, stream));
+    edge_alias_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(
+        d_indptr, order.get(), n, d_weights, reinterpret_cast<unsigned long long *>(d_table), stacks.get(),
+        flags.get());
+    CUDA_CHECK(cudaGetLastError());
+    int bad = 0;
+    uint32_t longest = 0;
+    CUDA_CHECK(cudaMemcpyAsync(&bad, flags.get(), sizeof(int), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaMemcpyAsync(&longest, degree_sorted.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_CHECK(cudaStreamSynchronize(stream));
+    if (bad) {
+        error = "edge weights must be non-negative numbers";
+        return cudaErrorInvalidValue;
+    }
+    *longest_row = longest;
+    return cudaSuccess;
+}
+
 }  // namespace b2e

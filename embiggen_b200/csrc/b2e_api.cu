@@ -185,45 +185,6 @@ extern "C" void b2e_destroy(b2e_handle *h) {
     delete h;
 }
 
-// per-row Vose alias tables of a weighted graph, {thr, alias index inside the row} per edge;
-// normative construction: oracle/walks.c (orc_edge_alias), reproduced bit for bit
-static bool build_edge_alias(const int64_t *indptr, const float *weights, uint64_t n, std::vector<uint2> &table) {
-    std::vector<double> scaled;
-    std::vector<uint32_t> small, large;
-    for (uint64_t v = 0; v < n; ++v) {
-        const int64_t begin = indptr[v];
-        const uint64_t d = (uint64_t)(indptr[v + 1] - begin);
-        uint2 *row = table.data() + begin;
-        double total = 0.0;
-        uint64_t heaviest = 0;
-        for (uint64_t i = 0; i < d; ++i) {
-            const float w = weights[begin + i];
-            if (!(w >= 0.0f)) return false;
-            total += (double)w;
-            if (w > weights[begin + heaviest]) heaviest = i;
-        }
-        scaled.resize(d);
-        small.clear();
-        large.clear();
-        for (uint64_t i = 0; i < d; ++i) {
-            scaled[i] = total > 0.0 ? (double)weights[begin + i] * (double)d / total : 1.0;
-            row[i] = make_uint2(0xFFFFFFFFu, (uint32_t)i);
-            if (scaled[i] < 1.0) small.push_back((uint32_t)i); else large.push_back((uint32_t)i);
-        }
-        while (!small.empty() && !large.empty()) {
-            const uint32_t s = small.back(); small.pop_back();
-            const uint32_t l = large.back(); large.pop_back();
-            const double t = floor(scaled[s] * 4294967296.0);
-            row[s] = make_uint2(t >= 4294967295.0 ? 0xFFFFFFFFu : (uint32_t)t, l);
-            scaled[l] = (scaled[l] + scaled[s]) - 1.0;
-            if (scaled[l] < 1.0) small.push_back(l); else large.push_back(l);
-        }
-        for (const uint32_t s : small)  // leftovers of weight zero are never proposed
-            if (total > 0.0 && weights[begin + s] == 0.0f) row[s] = make_uint2(0u, (uint32_t)heaviest);
-    }
-    return true;
-}
-
 extern "C" int b2e_load_types(b2e_handle *h, const uint32_t *node_types, const uint32_t *edge_types) {
     REQUIRE_HANDLE(h);
     if (int rc = require_graph(h)) return rc;
@@ -319,42 +280,40 @@ static int build_graph(b2e_handle *h, const int64_t *indptr, const uint32_t *ind
     }
     lap("start nodes + alias table (GPU)");
 
-    // normalize_by_degree (.../node2vec_skipgram.py:94-96): the weight of v -> x divided by
-    // max(deg(x), 1), one float32 division per edge, folded into the proposal table -- no extra
-    // rejection however skewed the degrees (oracle: degree_normalised_weights)
-    std::vector<float> normalised;
-    std::vector<uint32_t> fetched_indices;
-    std::vector<int64_t> fetched_indptr;
-    if ((c.normalize_by_degree || weights) && !indptr) {  // resident graph: these options work on the host
-        fetched_indptr.resize(n + 1);
-        CUDA_TRY(cudaMemcpy(fetched_indptr.data(), d_indptr, (n + 1) * sizeof(int64_t), cudaMemcpyDeviceToHost));
-        indptr = fetched_indptr.data();
+    // Edge weights: the per-row alias tables of the proposal, built on the device (alias_build.cu)
+    // from the resident graph's own weights or from host weights uploaded once (4 B per edge,
+    // freed once the table is built).  normalize_by_degree (.../node2vec_skipgram.py:94-96) divides the
+    // weight of v -> x by max(deg(x), 1), one float32 division per edge on the device, folded into
+    // the proposal table -- no extra rejection however skewed the degrees (oracle:
+    // degree_normalised_weights).
+    const float *d_weights = g.csr->csr.weights.get();
+    DeviceBuffer<float> uploaded, normalised;
+    if (weights) {
+        CUDA_TRY(uploaded.reserve(nnz * sizeof(float)));
+        CUDA_TRY(cudaMemcpyAsync(uploaded.get(), weights, nnz * sizeof(float), cudaMemcpyHostToDevice, h->walk_stream));
+        d_weights = uploaded.get();
+        lap("edge weight upload");
     }
     if (c.normalize_by_degree) {
-        if (!indices) {  // resident graph: this rarely used option needs the ids on the host
-            fetched_indices.resize(nnz);
-            CUDA_TRY(cudaMemcpy(fetched_indices.data(), d_indices, nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
-            indices = fetched_indices.data();
-        }
-        normalised.resize(nnz);
-        for (uint64_t e = 0; e < nnz; ++e) {
-            const uint32_t x = indices[e];
-            const float degree = (float)std::max<int64_t>(indptr[x + 1] - indptr[x], 1);
-            normalised[e] = (weights ? weights[e] : 1.0f) / degree;
-        }
-        weights = normalised.data();
+        CUDA_TRY(normalised.reserve(nnz * sizeof(float)));
+        CUDA_TRY(launch_degree_normalise(d_indptr, d_indices, d_weights, nnz, normalised.get(), h->walk_stream));
+        ++h->launches;
+        d_weights = normalised.get();
+        lap("degree normalisation (GPU)");
     }
-    if (weights) {
-        std::vector<uint2> edge_alias(nnz);
-        if (!build_edge_alias(indptr, weights, n, edge_alias))
-            return fail(B2E_ERR_INVALID, "edge weights must be non-negative numbers");
+    if (d_weights) {
         CUDA_TRY(g.edge_alias.reserve(nnz * sizeof(uint2)));
-        CUDA_TRY(cudaMemcpyAsync(g.edge_alias.get(), edge_alias.data(), nnz * sizeof(uint2), cudaMemcpyHostToDevice,
-                                 h->walk_stream));
-        CUDA_TRY(cudaStreamSynchronize(h->walk_stream));  // `edge_alias` dies here
+        std::string error;
+        uint64_t longest_row = 0;
+        const cudaError_t e = build_edge_alias(d_indptr, d_weights, n, nnz, g.edge_alias.get(), &longest_row,
+                                               h->walk_stream, error);
+        if (e != cudaSuccess) return fail(e == cudaErrorInvalidValue ? B2E_ERR_INVALID : B2E_ERR_CUDA, error);
+        h->launches += 3;
+        lap(("edge alias tables (GPU, longest row " + std::to_string(longest_row) + ")").c_str());
     }
-
-    lap("edge alias tables (weighted graphs)");
+    const bool weighted = d_weights != nullptr;
+    uploaded.reset();  // the table is built: a host load's weights and the normalised ones go
+    normalised.reset();
     // Second-order walks: is the graph undirected (every edge mirrored)?  Verified here, never
     // assumed: it allows the adjacency check in the shorter of the two rows and the folded return
     // edge.  The row filters answer most adjacency checks with one gather (walk_kernels.cu).
@@ -372,7 +331,7 @@ static int build_graph(b2e_handle *h, const int64_t *indptr, const uint32_t *ind
         }
         uint64_t excess = 0;
         fold_thresholds(c.return_weight, c.explore_weight, h->thr_fold, &excess);
-        if (h->undirected && !weights && !getenv("B2E_NO_FOLD")) h->fold_excess = excess;
+        if (h->undirected && !weighted && !getenv("B2E_NO_FOLD")) h->fold_excess = excess;
         if (!getenv("B2E_NO_FILTER")) {
             const uint64_t words = row_filter_words(nnz);
             CUDA_TRY(g.filter.reserve(words * sizeof(unsigned long long)));
@@ -926,6 +885,15 @@ extern "C" int b2e_export_alias(b2e_handle *h, uint32_t *threshold, uint32_t *al
     return B2E_OK;
 }
 
+extern "C" int b2e_export_edge_alias(b2e_handle *h, uint32_t *table) {
+    REQUIRE_HANDLE(h);
+    if (!table) return fail(B2E_ERR_INVALID, "null argument");
+    if (!h->graph.edge_alias.get()) return fail(B2E_ERR_STATE, "no edge alias table (unweighted graph or no graph)");
+    CUDA_TRY(cudaStreamSynchronize(h->walk_stream));
+    CUDA_TRY(cudaMemcpy(table, h->graph.edge_alias.get(), h->nnz * sizeof(uint2), cudaMemcpyDeviceToHost));
+    return B2E_OK;
+}
+
 extern "C" int b2e_counters_read(b2e_handle *h, b2e_counters *out) {
     REQUIRE_HANDLE(h);
     if (!out) return fail(B2E_ERR_INVALID, "null argument");
@@ -1301,12 +1269,20 @@ extern "C" int b2e_fit(b2e_handle *h, uint64_t seed, float *table0, float *table
 // a host CSR uploaded once, to be shared by several handles (b2e_load_graph checks its contents)
 extern "C" int b2e_graph_from_csr(int device, const int64_t *indptr, const uint32_t *indices, uint64_t n,
                                   uint64_t nnz, b2e_graph **out) {
+    return b2e_graph_from_csr_weighted(device, indptr, indices, nullptr, n, nnz, out);
+}
+
+extern "C" int b2e_graph_from_csr_weighted(int device, const int64_t *indptr, const uint32_t *indices,
+                                           const float *weights, uint64_t n, uint64_t nnz, b2e_graph **out) {
     if (!out || !indptr || (!indices && nnz)) return fail(B2E_ERR_INVALID, "null argument");
     if (n == 0 || n >= 0xFFFFFF00ull) return fail(B2E_ERR_INVALID, "the number of nodes must be in [1, 0xFFFFFF00)");
     if (indptr[0] != 0 || (uint64_t)indptr[n] != nnz)
         return fail(B2E_ERR_INVALID, "indptr must start at 0 and end at nnz");
     for (uint64_t v = 0; v < n; ++v)
         if (indptr[v + 1] < indptr[v]) return fail(B2E_ERR_INVALID, "indptr must be non-decreasing");
+    if (weights)
+        for (uint64_t e = 0; e < nnz; ++e)
+            if (!(weights[e] >= 0.0f)) return fail(B2E_ERR_INVALID, "edge weights must be non-negative numbers");
     if (int rc = select_device(device)) return rc;
     std::unique_ptr<b2e_graph, GraphRelease> g(new (std::nothrow) b2e_graph());
     if (!g) return fail(B2E_ERR_INVALID, "out of host memory");
@@ -1317,6 +1293,10 @@ extern "C" int b2e_graph_from_csr(int device, const int64_t *indptr, const uint3
     CUDA_TRY(g->csr.indices.reserve(std::max<uint64_t>(nnz, 1) * sizeof(uint32_t)));
     CUDA_TRY(cudaMemcpy(g->csr.indptr.get(), indptr, (n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice));
     if (nnz) CUDA_TRY(cudaMemcpy(g->csr.indices.get(), indices, nnz * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    if (weights) {
+        CUDA_TRY(g->csr.weights.reserve(std::max<uint64_t>(nnz, 1) * sizeof(float)));
+        if (nnz) CUDA_TRY(cudaMemcpy(g->csr.weights.get(), weights, nnz * sizeof(float), cudaMemcpyHostToDevice));
+    }
     *out = g.release();
     return B2E_OK;
 }
@@ -1337,6 +1317,17 @@ extern "C" int b2e_graph_export(const b2e_graph *g, int64_t *indptr, uint32_t *i
     return B2E_OK;
 }
 
+extern "C" int b2e_graph_weighted(const b2e_graph *g) { return g && g->csr.weights.get() ? 1 : 0; }
+
+extern "C" int b2e_graph_export_weights(const b2e_graph *g, float *weights) {
+    if (!g || (!weights && g->csr.nnz)) return fail(B2E_ERR_INVALID, "null argument");
+    if (!g->csr.weights.get()) return fail(B2E_ERR_STATE, "the graph has no edge weights");
+    CUDA_TRY(cudaSetDevice(g->device));
+    if (g->csr.nnz)
+        CUDA_TRY(cudaMemcpy(weights, g->csr.weights.get(), g->csr.nnz * sizeof(float), cudaMemcpyDeviceToHost));
+    return B2E_OK;
+}
+
 extern "C" void b2e_graph_destroy(b2e_graph *g) {
     if (!g) return;
     cudaSetDevice(g->device);
@@ -1349,8 +1340,9 @@ extern "C" int b2e_load_graph(b2e_handle *h, b2e_graph *g) {
     if (g->device != h->cfg.device) return fail(B2E_ERR_INVALID, "the graph lives on another device than the handle");
     if (g->csr.n == 0) return fail(B2E_ERR_INVALID, "The provided graph is empty.");
     if (g->csr.nnz == 0) return fail(B2E_ERR_INVALID, "The provided graph does not have edges.");
-    // nothing comes back to the host: start nodes, alias table, filters are all built from the
-    // resident arrays (an exponent without an exact form fetches the offsets, see alias_build.cu)
+    // nothing comes back to the host: start nodes, alias table, edge alias tables (a weighted
+    // graph, normalize_by_degree), filters are all built from the resident arrays (an exponent
+    // without an exact form fetches the offsets, see alias_build.cu)
     std::vector<int64_t> indptr;
     const double alpha = (double)h->cfg.negative_sampling_exponent;
     if (h->cfg.use_scale_free_distribution && alpha != 0.0 && alpha != 0.5 && alpha != 0.75 && alpha != 1.0) {
@@ -1404,13 +1396,20 @@ static int check_synthetic(int kind, uint64_t n_nodes, uint32_t scale, uint64_t 
 
 extern "C" int b2e_graph_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
                                     uint64_t n_nodes, int symmetrise, b2e_graph **out) {
+    return b2e_graph_from_edges_weighted(device, src, dst, nullptr, n_edges, n_nodes, symmetrise, out);
+}
+
+extern "C" int b2e_graph_from_edges_weighted(int device, const uint32_t *src, const uint32_t *dst,
+                                             const float *weights, uint64_t n_edges, uint64_t n_nodes, int symmetrise,
+                                             b2e_graph **out) {
     if (!out) return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = check_edges(src, dst, n_edges, n_nodes)) return rc;
     if (int rc = select_device(device)) return rc;
     std::string error;
     ResidentCsr csr;
     uint64_t nnz = 0;
-    cudaError_t e = csr_from_edges(src, dst, n_edges, n_nodes, symmetrise, nullptr, nullptr, 0, &nnz, error, &csr);
+    cudaError_t e = csr_from_edges(src, dst, weights, n_edges, n_nodes, symmetrise, nullptr, nullptr, nullptr, 0, &nnz,
+                                   error, &csr);
     return deliver_graph(device, e, error, csr, out);
 }
 
@@ -1430,11 +1429,20 @@ extern "C" int b2e_graph_synthetic(int device, int kind, uint64_t n_nodes, uint3
 extern "C" int b2e_csr_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
                                   uint64_t n_nodes, int symmetrise, int64_t *indptr, uint32_t *indices,
                                   uint64_t indices_capacity, uint64_t *nnz) {
-    if (!indptr || !nnz || (n_edges && !indices)) return fail(B2E_ERR_INVALID, "null argument");
+    return b2e_csr_from_edges_weighted(device, src, dst, nullptr, n_edges, n_nodes, symmetrise, indptr, indices,
+                                       nullptr, indices_capacity, nnz);
+}
+
+extern "C" int b2e_csr_from_edges_weighted(int device, const uint32_t *src, const uint32_t *dst,
+                                           const float *weights, uint64_t n_edges, uint64_t n_nodes, int symmetrise,
+                                           int64_t *indptr, uint32_t *indices, float *out_weights,
+                                           uint64_t indices_capacity, uint64_t *nnz) {
+    if (!indptr || !nnz || (n_edges && !indices) || (n_edges && weights && !out_weights))
+        return fail(B2E_ERR_INVALID, "null argument");
     if (int rc = check_edges(src, dst, n_edges, n_nodes)) return rc;
     if (int rc = select_device(device)) return rc;
     std::string error;
-    cudaError_t e = csr_from_edges(src, dst, n_edges, n_nodes, symmetrise, indptr, indices,
+    cudaError_t e = csr_from_edges(src, dst, weights, n_edges, n_nodes, symmetrise, indptr, indices, out_weights,
                                    indices_capacity, nnz, error);
     return ingest_status(e, error);
 }

@@ -101,6 +101,13 @@ cudaError_t check_indptr_device(const int64_t *d_indptr, uint64_t n, uint64_t nn
 cudaError_t build_node_tables(const int64_t *d_indptr, const int64_t *host_indptr, uint64_t n, double alpha,
                               uint32_t *d_sources, uint64_t *n_src_out, uint64_t *max_degree_out, uint2 *d_table,
                               cudaStream_t stream, std::string &error);
+// alias_build.cu: the per-row alias tables of a weighted graph, {thr, alias index inside the row} per
+// edge, bit-identical to oracle/walks.c (orc_edge_alias); *longest_row: the largest degree
+cudaError_t build_edge_alias(const int64_t *d_indptr, const float *d_weights, uint64_t n, uint64_t nnz,
+                             uint2 *d_table, uint64_t *longest_row, cudaStream_t stream, std::string &error);
+// normalize_by_degree: out[e] = (weights ? weights[e] : 1) / max(deg(indices[e]), 1), in float32
+cudaError_t launch_degree_normalise(const int64_t *d_indptr, const uint32_t *d_indices, const float *d_weights,
+                                    uint64_t nnz, float *d_out, cudaStream_t stream);
 uint64_t row_filter_words(uint64_t nnz);
 cudaError_t launch_row_filter_build(const int64_t *indptr, const uint32_t *indices, uint64_t n,
                                     unsigned long long *filter, int sm_count, cudaStream_t stream);

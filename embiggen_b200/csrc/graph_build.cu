@@ -61,17 +61,27 @@ __global__ void __launch_bounds__(256) draw_edges_kernel(int kind, uint64_t n, u
     ids[k] = idx;
 }
 
-// (src, dst) host-style edge list -> directed keys (src << 32) | dst, self-loops dropped
+// (src, dst) host-style edge list -> directed keys (src << 32) | dst, self-loops dropped; originals
+// at [0, count), mirrors at [count, 2 count).  With `weights` every key carries its edge's weight in
+// `values` (same layout), and flags |= 2 marks a negative or NaN input weight (flags |= 1: an
+// endpoint out of range)
 __global__ void __launch_bounds__(256) edge_keys_kernel(const uint32_t *src, const uint32_t *dst,
-                                                        uint64_t count, uint64_t n, int symmetrise,
-                                                        unsigned long long *keys, int *out_of_range) {
+                                                        const float *weights, uint64_t count, uint64_t n,
+                                                        int symmetrise, unsigned long long *keys,
+                                                        float *values, int *flags) {
     const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= count) return;
     const uint64_t s = src[k], d = dst[k];
-    if (s >= n || d >= n) *out_of_range = 1;
+    if (s >= n || d >= n) atomicOr(flags, 1);
     const bool ok = s != d && s < n && d < n;
     keys[k] = ok ? ((s << 32) | d) : INVALID_KEY;
     if (symmetrise) keys[count + k] = ok ? ((d << 32) | s) : INVALID_KEY;
+    if (weights) {
+        const float w = weights[k];
+        if (!(w >= 0.0f)) atomicOr(flags, 2);
+        values[k] = w;
+        if (symmetrise) values[count + k] = w;
+    }
 }
 
 __global__ void __launch_bounds__(256) mirror_keys_kernel(const unsigned long long *undirected,
@@ -123,23 +133,45 @@ static cudaError_t sort_keys(DeviceBuffer<> &temp, const unsigned long long *key
 }
 
 // directed keys (any order) -> CSR in device buffers.  `scratch` is the alternate buffer of the
-// radix sort (no third copy).  With `dedup` the keys may repeat and contain INVALID_KEY.
+// radix sort (no third copy).  With `dedup` the keys may repeat and contain INVALID_KEY.  With
+// `values` (and their alternate `value_scratch`) every key carries a weight: the sort is stable,
+// so the first element of a run of equal keys carries the weight of the key's first occurrence,
+// and that is the weight the de-duplicated edge keeps (d_weights, nnz entries).
 static cudaError_t keys_to_csr(DeviceBuffer<> &temp, unsigned long long *keys, unsigned long long *scratch,
                                uint64_t count, uint64_t n, bool dedup, DeviceBuffer<int64_t> &d_indptr,
-                               DeviceBuffer<uint32_t> &d_indices, uint64_t *nnz_out, std::string &error) {
+                               DeviceBuffer<uint32_t> &d_indices, uint64_t *nnz_out, std::string &error,
+                               float *values = nullptr, float *value_scratch = nullptr,
+                               DeviceBuffer<float> *d_weights = nullptr) {
     cub::DoubleBuffer<unsigned long long> buffers(keys, scratch);
+    cub::DoubleBuffer<float> weights(values, value_scratch);
     size_t bytes = 0;
-    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, buffers, count));
-    CUDA_CHECK(temp.reserve(bytes));
-    CUDA_CHECK(cub::DeviceRadixSort::SortKeys(temp.get(), bytes, buffers, count));
+    if (values) {
+        CUDA_CHECK(cub::DeviceRadixSort::SortPairs(nullptr, bytes, buffers, weights, count));
+        CUDA_CHECK(temp.reserve(bytes));
+        CUDA_CHECK(cub::DeviceRadixSort::SortPairs(temp.get(), bytes, buffers, weights, count));
+    } else {
+        CUDA_CHECK(cub::DeviceRadixSort::SortKeys(nullptr, bytes, buffers, count));
+        CUDA_CHECK(temp.reserve(bytes));
+        CUDA_CHECK(cub::DeviceRadixSort::SortKeys(temp.get(), bytes, buffers, count));
+    }
     unsigned long long *sorted = buffers.Current(), *other = buffers.Alternate();
+    float *sorted_values = weights.Current();
     uint64_t nnz = count;
     if (dedup) {
         DeviceBuffer<unsigned long long> selected;
         CUDA_CHECK(selected.reserve(sizeof(unsigned long long)));
-        CUDA_CHECK(cub::DeviceSelect::Unique(nullptr, bytes, sorted, other, selected.get(), count));
-        CUDA_CHECK(temp.reserve(bytes));
-        CUDA_CHECK(cub::DeviceSelect::Unique(temp.get(), bytes, sorted, other, selected.get(), count));
+        if (values) {  // UniqueByKey keeps the first element of every run
+            CUDA_CHECK(cub::DeviceSelect::UniqueByKey(nullptr, bytes, sorted, sorted_values, other,
+                                                      weights.Alternate(), selected.get(), count));
+            CUDA_CHECK(temp.reserve(bytes));
+            CUDA_CHECK(cub::DeviceSelect::UniqueByKey(temp.get(), bytes, sorted, sorted_values, other,
+                                                      weights.Alternate(), selected.get(), count));
+            sorted_values = weights.Alternate();
+        } else {
+            CUDA_CHECK(cub::DeviceSelect::Unique(nullptr, bytes, sorted, other, selected.get(), count));
+            CUDA_CHECK(temp.reserve(bytes));
+            CUDA_CHECK(cub::DeviceSelect::Unique(temp.get(), bytes, sorted, other, selected.get(), count));
+        }
         unsigned long long unique = 0, last = 0;
         CUDA_CHECK(cudaMemcpy(&unique, selected.get(), sizeof(unique), cudaMemcpyDeviceToHost));
         if (unique) CUDA_CHECK(cudaMemcpy(&last, other + unique - 1, sizeof(last), cudaMemcpyDeviceToHost));
@@ -152,17 +184,24 @@ static cudaError_t keys_to_csr(DeviceBuffer<> &temp, unsigned long long *keys, u
     csr_from_keys_kernel<<<blocks_for(std::max<uint64_t>(nnz, n + 1)), 256>>>(
         sorted, nnz, n, d_indices.get(), reinterpret_cast<long long *>(d_indptr.get()));
     CUDA_CHECK(cudaGetLastError());
+    if (values) {
+        CUDA_CHECK(d_weights->reserve(std::max<uint64_t>(nnz, 1) * sizeof(float)));
+        if (nnz) CUDA_CHECK(cudaMemcpy(d_weights->get(), sorted_values, nnz * sizeof(float), cudaMemcpyDeviceToDevice));
+    }
     CUDA_CHECK(cudaDeviceSynchronize());
     return cudaSuccess;
 }
 
-// hand the device arrays over: to host buffers, or (out != nullptr) to a resident b2e_graph
-static cudaError_t deliver(DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<uint32_t> &d_indices, uint64_t n, uint64_t nnz,
-                           int64_t *indptr, uint32_t *indices, uint64_t capacity, ResidentCsr *out,
+// hand the device arrays over: to host buffers, or (out != nullptr) to a resident b2e_graph.
+// `d_weights` is empty for an unweighted graph (then `weights` is not touched).
+static cudaError_t deliver(DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<uint32_t> &d_indices,
+                           DeviceBuffer<float> &d_weights, uint64_t n, uint64_t nnz, int64_t *indptr,
+                           uint32_t *indices, float *weights, uint64_t capacity, ResidentCsr *out,
                            std::string &error) {
     if (out) {
         out->indptr = std::move(d_indptr);
         out->indices = std::move(d_indices);
+        out->weights = std::move(d_weights);
         out->n = n;
         out->nnz = nnz;
         return cudaSuccess;
@@ -173,14 +212,20 @@ static cudaError_t deliver(DeviceBuffer<int64_t> &d_indptr, DeviceBuffer<uint32_
     }
     CUDA_CHECK(cudaMemcpy(indptr, d_indptr.get(), (n + 1) * sizeof(long long), cudaMemcpyDeviceToHost));
     if (nnz) CUDA_CHECK(cudaMemcpy(indices, d_indices.get(), nnz * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    if (nnz && weights && d_weights.get())
+        CUDA_CHECK(cudaMemcpy(weights, d_weights.get(), nnz * sizeof(float), cudaMemcpyDeviceToHost));
     return cudaSuccess;
 }
 
-cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_edges, uint64_t n,
-                           int symmetrise, int64_t *indptr, uint32_t *indices, uint64_t capacity,
-                           uint64_t *nnz_out, std::string &error, ResidentCsr *resident) {
+// Peak device memory per input edge, symmetrised: 8 B of endpoints, 32 B of keys (two buffers of
+// two directed keys), plus for a weighted list 4 B of input weights and 16 B of sorted values (two
+// buffers of two floats); afterwards the CSR (8 B, 8 B more with weights) while the keys still live.
+cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, const float *weights, uint64_t n_edges,
+                           uint64_t n, int symmetrise, int64_t *indptr, uint32_t *indices, float *out_weights,
+                           uint64_t capacity, uint64_t *nnz_out, std::string &error, ResidentCsr *resident) {
     const uint64_t count = n_edges * (symmetrise ? 2 : 1);
     DeviceBuffer<uint32_t> d_src, d_dst;
+    DeviceBuffer<float> d_in, values, value_scratch;
     DeviceBuffer<unsigned long long> keys, scratch;
     DeviceBuffer<> temp;
     DeviceBuffer<int> flag;
@@ -188,29 +233,41 @@ cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_
     CUDA_CHECK(d_dst.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(uint32_t)));
     CUDA_CHECK(keys.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
     CUDA_CHECK(scratch.reserve(std::max<uint64_t>(count, 1) * sizeof(unsigned long long)));
+    if (weights) {
+        CUDA_CHECK(d_in.reserve(std::max<uint64_t>(n_edges, 1) * sizeof(float)));
+        CUDA_CHECK(values.reserve(std::max<uint64_t>(count, 1) * sizeof(float)));
+        CUDA_CHECK(value_scratch.reserve(std::max<uint64_t>(count, 1) * sizeof(float)));
+        CUDA_CHECK(cudaMemcpy(d_in.get(), weights, n_edges * sizeof(float), cudaMemcpyHostToDevice));
+    }
     CUDA_CHECK(flag.reserve(sizeof(int)));
     CUDA_CHECK(cudaMemset(flag.get(), 0, sizeof(int)));
     CUDA_CHECK(cudaMemcpy(d_src.get(), src, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
     CUDA_CHECK(cudaMemcpy(d_dst.get(), dst, n_edges * sizeof(uint32_t), cudaMemcpyHostToDevice));
     if (n_edges) {
-        edge_keys_kernel<<<blocks_for(n_edges), 256>>>(d_src.get(), d_dst.get(), n_edges, n,
-                                                       symmetrise, keys.get(),
-                                                       flag.get());
+        edge_keys_kernel<<<blocks_for(n_edges), 256>>>(d_src.get(), d_dst.get(), d_in.get(), n_edges, n,
+                                                       symmetrise, keys.get(), values.get(), flag.get());
         CUDA_CHECK(cudaGetLastError());
     }
-    int out_of_range = 0;
-    CUDA_CHECK(cudaMemcpy(&out_of_range, flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
-    if (out_of_range) {
+    int flags = 0;
+    CUDA_CHECK(cudaMemcpy(&flags, flag.get(), sizeof(int), cudaMemcpyDeviceToHost));
+    if (flags & 1) {
         error = "an edge endpoint is not below the number of nodes";
+        return cudaErrorInvalidValue;
+    }
+    if (flags & 2) {
+        error = "edge weights must be non-negative numbers";
         return cudaErrorInvalidValue;
     }
     d_src.reset();
     d_dst.reset();
+    d_in.reset();
     DeviceBuffer<int64_t> d_indptr;
     DeviceBuffer<uint32_t> d_indices;
-    CUDA_CHECK(keys_to_csr(temp, keys.get(), scratch.get(), count, n, true,
-                       d_indptr, d_indices, nnz_out, error));
-    return deliver(d_indptr, d_indices, n, *nnz_out, indptr, indices, capacity, resident, error);
+    DeviceBuffer<float> d_weights;
+    CUDA_CHECK(keys_to_csr(temp, keys.get(), scratch.get(), count, n, true, d_indptr, d_indices, nnz_out, error,
+                           values.get(), value_scratch.get(), &d_weights));
+    return deliver(d_indptr, d_indices, d_weights, n, *nnz_out, indptr, indices, out_weights, capacity, resident,
+                   error);
 }
 
 // flags[j] = 1 when keys[j] is a real key that the sorted pool does not hold yet
@@ -328,12 +385,14 @@ cudaError_t synthetic_csr(int kind, uint64_t n, uint32_t scale, uint64_t m, uint
     CUDA_CHECK(alternate.reserve(2 * have * sizeof(u64)));
     DeviceBuffer<int64_t> d_indptr;
     DeviceBuffer<uint32_t> d_indices;
+    DeviceBuffer<float> no_weights;
     CUDA_CHECK(keys_to_csr(temp, directed.get(), alternate.get(), 2 * have, n, false, d_indptr, d_indices,
                        nnz_out, error));
     directed.reset();
     alternate.reset();
     temp.reset();
-    return deliver(d_indptr, d_indices, n, *nnz_out, indptr, indices, capacity, resident, error);
+    return deliver(d_indptr, d_indices, no_weights, n, *nnz_out, indptr, indices, nullptr, capacity, resident,
+                   error);
 }
 
 }  // namespace b2e

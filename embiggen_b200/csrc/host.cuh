@@ -137,12 +137,16 @@ cudaError_t glove_max_count(GloveState &g, uint32_t *max_count, cudaStream_t str
 struct ResidentCsr {
     DeviceBuffer<int64_t> indptr;
     DeviceBuffer<uint32_t> indices;
+    DeviceBuffer<float> weights;  // one per edge, never negative; empty for an unweighted graph
     uint64_t n = 0, nnz = 0;
 };
-// `resident` != nullptr: the device arrays move into it and the host buffers are not touched
-cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, uint64_t n_edges, uint64_t n,
-                           int symmetrise, int64_t *indptr, uint32_t *indices, uint64_t capacity,
-                           uint64_t *nnz_out, std::string &error, ResidentCsr *resident = nullptr);
+// `resident` != nullptr: the device arrays move into it and the host buffers are not touched.
+// `weights` (nullable, one per input edge) makes a weighted graph; `out_weights` receives its nnz
+// weights when the CSR goes to host buffers.
+cudaError_t csr_from_edges(const uint32_t *src, const uint32_t *dst, const float *weights, uint64_t n_edges,
+                           uint64_t n, int symmetrise, int64_t *indptr, uint32_t *indices, float *out_weights,
+                           uint64_t capacity, uint64_t *nnz_out, std::string &error,
+                           ResidentCsr *resident = nullptr);
 cudaError_t synthetic_csr(int kind, uint64_t n, uint32_t scale, uint64_t m, uint64_t seed,
                           unsigned long long t_a, unsigned long long t_ab, unsigned long long t_abc,
                           int64_t *indptr, uint32_t *indices, uint64_t capacity, uint64_t *nnz_out,

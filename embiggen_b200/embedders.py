@@ -511,8 +511,10 @@ class WalkletsB200(Node2VecB200):
     def _fit_transform(self, graph, return_dataframe: bool = True) -> EmbeddingResult:
         """All scales in ONE pass over the walks: the graph is uploaded once and shared, every
         chunk is walked once (by the engine of scale 1) and adopted by the engines of the other
-        scales, each of which owns its pair of tables (engine.fit_scales).  Weighted and typed
-        graphs, other dtypes than f32 and torch.distributed runs take the scale-by-scale path."""
+        scales, each of which owns its pair of tables (engine.fit_scales).  A resident graph
+        (graph_gpu.DeviceGraph) takes this path weighted or not: every scale builds its edge alias
+        tables from the resident weights.  Weighted host graphs, typed graphs, other dtypes than
+        f32 and torch.distributed runs take the scale-by-scale path."""
         from .engine import fit_scales
         from .graph_gpu import device_graph_from_csr
         window_size = self._model_kwargs["window_size"]

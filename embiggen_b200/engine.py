@@ -183,7 +183,7 @@ class Engine:
 
     def load_graph(self, graph) -> None:
         """K1 without the copy: walk on a :class:`embiggen_b200.graph_gpu.DeviceGraph` (a CSR that
-        was built on this GPU and never left HBM)."""
+        was built on this GPU and never left HBM); a weighted one walks by its weights."""
         check(self._lib.b2e_load_graph(self._handle, graph._handle))
         self.n = graph.get_number_of_nodes()
         self.nnz = graph.get_number_of_directed_edges()
@@ -359,6 +359,13 @@ class Engine:
         thr, alias = np.empty(self.n, dtype=np.uint32), np.empty(self.n, dtype=np.uint32)
         check(self._lib.b2e_export_alias(self._handle, thr.ctypes.data, alias.ctypes.data))
         return thr, alias
+
+    def export_edge_alias(self) -> np.ndarray:
+        """The per-row alias tables of a weighted load, shape (nnz, 2): {thr, alias index inside the
+        row}, the layout of ``oracle.edge_alias``."""
+        table = np.empty((max(self.nnz, 1), 2), dtype=np.uint32)
+        check(self._lib.b2e_export_edge_alias(self._handle, table.ctypes.data))
+        return table[: self.nnz]
 
     def counters(self) -> dict:
         out = B2ECounters()

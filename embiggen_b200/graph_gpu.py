@@ -6,6 +6,10 @@ out of a plain edge list; ``erdos_renyi_gpu`` / ``rmat_gpu`` generate the synthe
 BASELINE.json shapes and return the same graphs as the numpy generators of
 :mod:`embiggen_b200.graph` (same Philox stream, same "first m distinct edges in draw order"
 rule), which is how the 200 M-edge configurations become practical.
+
+Edge weights go through both: ``weights=`` (one float32 per input edge, never negative) gives the
+weighted CSR of :func:`embiggen_b200.graph.csr_from_edges`, bit for bit, and a weighted
+:class:`DeviceGraph` walks by weight without its weights ever leaving HBM.
 """
 import ctypes
 from typing import Optional
@@ -17,21 +21,35 @@ from ._lib import check
 from .graph import CSRGraph
 
 
-def csr_from_edges_gpu(src, dst, n: int, symmetrise: bool = True, node_names=None,
-                       name: str = "graph", device: int = 0) -> CSRGraph:
+def _edge_list(src, dst, weights):
     src = np.ascontiguousarray(src, dtype=np.uint32)
     dst = np.ascontiguousarray(dst, dtype=np.uint32)
     if src.shape != dst.shape or src.ndim != 1:
         raise ValueError("src and dst must be 1-d arrays of the same length.")
+    if weights is not None:
+        weights = np.ascontiguousarray(weights, dtype=np.float32)
+        if weights.shape != src.shape:
+            raise ValueError("weights must have one entry per edge.")
+    return src, dst, weights
+
+
+def csr_from_edges_gpu(src, dst, n: int, symmetrise: bool = True, node_names=None,
+                       name: str = "graph", device: int = 0, weights=None) -> CSRGraph:
+    """Sorted, de-duplicated, self-loop-free CSR, equal to :func:`embiggen_b200.graph.csr_from_edges`
+    (with ``weights``: a duplicated edge keeps the weight of its first occurrence; a negative or
+    NaN weight raises ValueError)."""
+    src, dst, weights = _edge_list(src, dst, weights)
     capacity = max(1, src.shape[0] * (2 if symmetrise else 1))
     indptr = np.empty(n + 1, dtype=np.int64)
     indices = np.empty(capacity, dtype=np.uint32)
+    out_weights = None if weights is None else np.empty(capacity, dtype=np.float32)
     nnz = ctypes.c_uint64()
-    check(_lib.load().b2e_csr_from_edges(device, src.ctypes.data, dst.ctypes.data, src.shape[0], n,
-                                         int(symmetrise), indptr.ctypes.data, indices.ctypes.data,
-                                         capacity, ctypes.byref(nnz)))
+    check(_lib.load().b2e_csr_from_edges_weighted(
+        device, src.ctypes.data, dst.ctypes.data, None if weights is None else weights.ctypes.data, src.shape[0], n,
+        int(symmetrise), indptr.ctypes.data, indices.ctypes.data,
+        None if out_weights is None else out_weights.ctypes.data, capacity, ctypes.byref(nnz)))
     return CSRGraph(indptr, indices[: nnz.value].copy(), node_names=node_names, name=name,
-                    directed=not symmetrise)
+                    directed=not symmetrise, weights=None if weights is None else out_weights[: nnz.value].copy())
 
 
 class DeviceGraph:
@@ -50,6 +68,7 @@ class DeviceGraph:
         n, nnz = ctypes.c_uint64(), ctypes.c_uint64()
         check(self._lib.b2e_graph_shape(self._handle, ctypes.byref(n), ctypes.byref(nnz)))
         self._n, self._nnz = int(n.value), int(nnz.value)
+        self._weighted = bool(self._lib.b2e_graph_weighted(self._handle))
         self._host: Optional[CSRGraph] = None
 
     def close(self) -> None:
@@ -68,7 +87,9 @@ class DeviceGraph:
             indptr = np.empty(self._n + 1, dtype=np.int64)
             indices = np.empty(max(self._nnz, 1), dtype=np.uint32)
             check(self._lib.b2e_graph_export(self._handle, indptr.ctypes.data, indices.ctypes.data))
-            self._host = CSRGraph(indptr, indices[: self._nnz], name=self._name, directed=self._directed)
+            weights = self.get_directed_edge_weights() if self._weighted else None
+            self._host = CSRGraph(indptr, indices[: self._nnz], name=self._name, directed=self._directed,
+                                  weights=weights)
         return self._host
 
     # -- accessors mirrored from ensmallen.Graph (see CSRGraph) --
@@ -88,9 +109,19 @@ class DeviceGraph:
         return self._nnz > 0
 
     def has_edge_weights(self) -> bool:
-        return False
+        return self._weighted
+
+    def get_directed_edge_weights(self) -> np.ndarray:
+        """The weight of every directed edge, in CSR order (a copy from HBM)."""
+        if not self._weighted:
+            raise ValueError("The graph has no edge weights.")
+        weights = np.empty(max(self._nnz, 1), dtype=np.float32)
+        check(self._lib.b2e_graph_export_weights(self._handle, weights.ctypes.data))
+        return weights[: self._nnz]
 
     def has_negative_edge_weights(self) -> bool:
+        """Always False: graph ingest refuses negative (and NaN) weights, so a resident graph never
+        holds one."""
         return False
 
     def has_node_types(self) -> bool:
@@ -118,26 +149,30 @@ class DeviceGraph:
         return self.get_number_of_disconnected_nodes() > 0
 
 
-def device_graph_from_csr(indptr, indices, name: str = "graph", device: int = 0) -> DeviceGraph:
-    """Upload a host CSR once (to share it between several engines)."""
+def device_graph_from_csr(indptr, indices, weights=None, name: str = "graph", device: int = 0) -> DeviceGraph:
+    """Upload a host CSR once (to share it between several engines), with its edge weights if given
+    (one per directed edge, never negative)."""
     indptr = np.ascontiguousarray(indptr, dtype=np.int64)
     indices = np.ascontiguousarray(indices, dtype=np.uint32)
+    if weights is not None:
+        weights = np.ascontiguousarray(weights, dtype=np.float32)
+        if weights.shape != indices.shape:
+            raise ValueError("weights must have one entry per directed edge.")
     handle = ctypes.c_void_p()
-    check(_lib.load().b2e_graph_from_csr(device, indptr.ctypes.data, indices.ctypes.data, indptr.shape[0] - 1,
-                                         indices.shape[0], ctypes.byref(handle)))
+    check(_lib.load().b2e_graph_from_csr_weighted(device, indptr.ctypes.data, indices.ctypes.data,
+                                                  None if weights is None else weights.ctypes.data,
+                                                  indptr.shape[0] - 1, indices.shape[0], ctypes.byref(handle)))
     return DeviceGraph(handle, device, name=name)
 
 
 def device_graph_from_edges(src, dst, n: int, symmetrise: bool = True, name: str = "graph",
-                            device: int = 0) -> DeviceGraph:
-    """:func:`csr_from_edges_gpu`, but the CSR stays in HBM."""
-    src = np.ascontiguousarray(src, dtype=np.uint32)
-    dst = np.ascontiguousarray(dst, dtype=np.uint32)
-    if src.shape != dst.shape or src.ndim != 1:
-        raise ValueError("src and dst must be 1-d arrays of the same length.")
+                            device: int = 0, weights=None) -> DeviceGraph:
+    """:func:`csr_from_edges_gpu`, but the CSR (and its weights) stays in HBM."""
+    src, dst, weights = _edge_list(src, dst, weights)
     handle = ctypes.c_void_p()
-    check(_lib.load().b2e_graph_from_edges(device, src.ctypes.data, dst.ctypes.data, src.shape[0], n,
-                                           int(symmetrise), ctypes.byref(handle)))
+    check(_lib.load().b2e_graph_from_edges_weighted(device, src.ctypes.data, dst.ctypes.data,
+                                                    None if weights is None else weights.ctypes.data,
+                                                    src.shape[0], n, int(symmetrise), ctypes.byref(handle)))
     return DeviceGraph(handle, device, name=name, directed=not symmetrise)
 
 

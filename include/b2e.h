@@ -258,6 +258,10 @@ int b2e_export_tables(b2e_handle *handle, float *table0, float *table1);
 int b2e_import_tables(b2e_handle *handle, const float *table0, const float *table1);
 /* alias table as built for the handle (n entries each); parity/debug export */
 int b2e_export_alias(b2e_handle *handle, uint32_t *threshold, uint32_t *alias);
+/* per-row alias tables of a weighted load (nnz x 2 words: {thr, alias index inside the row}, the
+ * layout of oracle/walks.c: orc_edge_alias), as built on the device; parity/debug export.
+ * B2E_ERR_STATE when the handle walks without weights. */
+int b2e_export_edge_alias(b2e_handle *handle, uint32_t *table);
 
 int b2e_counters_read(b2e_handle *handle, b2e_counters *out);
 int b2e_counters_reset(b2e_handle *handle);
@@ -276,6 +280,16 @@ uint64_t b2e_launch_count(const b2e_handle *handle);
 int b2e_csr_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
                        uint64_t n_nodes, int symmetrise, int64_t *indptr, uint32_t *indices,
                        uint64_t indices_capacity, uint64_t *nnz);
+/*
+ * Same with one float32 weight per input edge (weights == NULL is b2e_csr_from_edges); out_weights
+ * receives one per CSR edge, like indices.  The mirror of an edge carries its weight, and a
+ * duplicated edge keeps the weight of its first occurrence, taken over the input edges in input
+ * order and then their mirrors (embiggen_b200/graph.py: csr_from_edges).  A negative or NaN weight,
+ * self-loops included, fails with B2E_ERR_INVALID.
+ */
+int b2e_csr_from_edges_weighted(int device, const uint32_t *src, const uint32_t *dst, const float *weights,
+                                uint64_t n_edges, uint64_t n_nodes, int symmetrise, int64_t *indptr,
+                                uint32_t *indices, float *out_weights, uint64_t indices_capacity, uint64_t *nnz);
 
 /*
  * Seeded synthetic graphs of the BASELINE.json shapes: the first n_edges distinct undirected
@@ -295,17 +309,28 @@ int b2e_synthetic_csr(int device, int kind, uint64_t n_nodes, uint32_t scale, ui
  * b2e_graph is reference counted: b2e_load_graph makes the handle walk on the graph's own device
  * arrays, b2e_graph_destroy may be called right after it.  b2e_graph_export copies the CSR to host
  * buffers of n + 1 and nnz entries (b2e_graph_shape).
+ * A resident graph may carry edge weights (the _weighted builders; never negative): a handle then
+ * walks by weight, with its per-row alias tables built on the device from the resident weights.
+ * b2e_graph_weighted returns 1 for such a graph, 0 otherwise; b2e_graph_export_weights copies its
+ * nnz weights to the host (B2E_ERR_STATE without weights).
  */
 typedef struct b2e_graph b2e_graph;
 int b2e_graph_from_edges(int device, const uint32_t *src, const uint32_t *dst, uint64_t n_edges,
                          uint64_t n_nodes, int symmetrise, b2e_graph **graph);
+int b2e_graph_from_edges_weighted(int device, const uint32_t *src, const uint32_t *dst, const float *weights,
+                                  uint64_t n_edges, uint64_t n_nodes, int symmetrise, b2e_graph **graph);
 int b2e_graph_synthetic(int device, int kind, uint64_t n_nodes, uint32_t scale, uint64_t n_edges,
                         uint64_t seed, uint64_t t_a, uint64_t t_ab, uint64_t t_abc, b2e_graph **graph);
 /* a host CSR uploaded once, e.g. to be shared by the handles of the Walklets scales */
 int b2e_graph_from_csr(int device, const int64_t *indptr, const uint32_t *indices, uint64_t n_nodes,
                        uint64_t nnz, b2e_graph **graph);
+/* ... with nnz non-negative weights aligned with indices (weights == NULL is b2e_graph_from_csr) */
+int b2e_graph_from_csr_weighted(int device, const int64_t *indptr, const uint32_t *indices, const float *weights,
+                                uint64_t n_nodes, uint64_t nnz, b2e_graph **graph);
 int b2e_graph_shape(const b2e_graph *graph, uint64_t *n_nodes, uint64_t *nnz);
 int b2e_graph_export(const b2e_graph *graph, int64_t *indptr, uint32_t *indices);
+int b2e_graph_weighted(const b2e_graph *graph);
+int b2e_graph_export_weights(const b2e_graph *graph, float *weights);
 void b2e_graph_destroy(b2e_graph *graph);
 int b2e_load_graph(b2e_handle *handle, b2e_graph *graph);
 
