@@ -106,7 +106,7 @@ def lib():
         l.orc_exp_det.argtypes = [f32]
         l.orc_glove_train.restype = ctypes.c_int
         l.orc_glove_train.argtypes = [P(u32), P(u32), P(u32), u64, u32, u32, u32, f32, f32, f32,
-                                      P(f32), P(f32), P(ctypes.c_double), P(u64)]
+                                      ctypes.c_int, P(f32), P(f32), P(ctypes.c_double), P(u64)]
         l.orc_alias_build.restype = ctypes.c_int
         l.orc_alias_build.argtypes = [P(ctypes.c_int64), u64, ctypes.c_double, P(u32), P(u32)]
         l.orc_set_threads.restype = None
@@ -443,8 +443,12 @@ def log_det(x: float) -> float:
 
 def glove_train(centre, context, count, t0: np.ndarray, t1: np.ndarray, embedding_size: int,
                 alpha: float, learning_rate: float, clipping_value: float = 6.0,
-                max_count: Optional[int] = None) -> dict:
-    """One sequential pass over the triples (in place); returns loss_sum / trained."""
+                max_count: Optional[int] = None, tile_semantics: bool = False) -> dict:
+    """One sequential pass over the triples (in place); returns loss_sum / trained.
+
+    ``tile_semantics`` trains with the arithmetic of the production kernel (glove_tile_kernel:
+    context rows updated as ``old + (-g * h)``, centre rows written back as ``row + (h - h0)``)
+    instead of the specification's; see oracle/oracle.h."""
     centre = np.ascontiguousarray(centre, dtype=np.uint32)
     context = np.ascontiguousarray(context, dtype=np.uint32)
     count = np.ascontiguousarray(count, dtype=np.uint32)
@@ -454,7 +458,7 @@ def glove_train(centre, context, count, t0: np.ndarray, t1: np.ndarray, embeddin
     trained = ctypes.c_uint64(0)
     rc = lib().orc_glove_train(_ptr(centre, ctypes.c_uint32), _ptr(context, ctypes.c_uint32),
                                _ptr(count, ctypes.c_uint32), centre.shape[0], max_count, embedding_size,
-                               t0.shape[1], alpha, clipping_value, learning_rate,
+                               t0.shape[1], alpha, clipping_value, learning_rate, int(bool(tile_semantics)),
                                _ptr(t0, ctypes.c_float), _ptr(t1, ctypes.c_float), ctypes.byref(loss),
                                ctypes.byref(trained))
     if rc != 0:

@@ -36,10 +36,10 @@ float orc_log_det(float x) {
 int orc_glove_train(const uint32_t *centre, const uint32_t *context, const uint32_t *count,
                     uint64_t n_triples, uint32_t max_count, uint32_t embedding_size,
                     uint32_t row_stride, float alpha, float clipping_value, float learning_rate,
-                    float *t0, float *t1, double *loss_sum, uint64_t *trained) {
+                    int tile_semantics, float *t0, float *t1, double *loss_sum, uint64_t *trained) {
     if (!centre || !context || !count || !t0 || !t1 || max_count == 0) return -1;
     if ((row_stride & 3) || row_stride < embedding_size || row_stride > 4096) return -1;
-    float h[4096];
+    float h[4096], h0[4096];
     double loss = 0.0;
     uint64_t done = 0;
     uint64_t e = 0;
@@ -47,6 +47,7 @@ int orc_glove_train(const uint32_t *centre, const uint32_t *context, const uint3
         const uint32_t c = centre[e];
         float *crow = t0 + (uint64_t)c * row_stride;
         memcpy(h, crow, row_stride * sizeof(float));
+        memcpy(h0, crow, row_stride * sizeof(float));
         for (; e < n_triples && centre[e] == c; ++e) {
             float *row = t1 + (uint64_t)context[e] * row_stride;
             const float f = orc_dot(h, row, row_stride);
@@ -59,11 +60,23 @@ int orc_glove_train(const uint32_t *centre, const uint32_t *context, const uint3
             ++done;
             for (uint32_t k = 0; k < row_stride; ++k) {
                 const float old = row[k];
-                row[k] = fmaf(-g, h[k], old);
+                if (tile_semantics) {
+                    const float step = -g * h[k];
+                    row[k] = old + step;
+                } else {
+                    row[k] = fmaf(-g, h[k], old);
+                }
                 h[k] = fmaf(-g, old, h[k]);
             }
         }
-        memcpy(crow, h, row_stride * sizeof(float));
+        if (tile_semantics) {
+            for (uint32_t k = 0; k < row_stride; ++k) {
+                const float change = h[k] - h0[k];
+                crow[k] = crow[k] + change;
+            }
+        } else {
+            memcpy(crow, h, row_stride * sizeof(float));
+        }
     }
     if (loss_sum) *loss_sum += loss;
     if (trained) *trained += done;

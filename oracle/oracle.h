@@ -155,11 +155,17 @@ int orc_train(const orc_sgns_cfg *cfg, const uint32_t *walks, uint64_t n_walks,
  *   weight = exp(alpha * ln(count / max_count));  g = 2 * weight * (f - ln(count)) * lr
  *   h' = h - g * T1[o];  T1[o] -= g * h;  h = h'
  * loss_sum accumulates weight * (f - ln count)^2 over the triples that were not skipped.
+ *
+ * tile_semantics != 0 restates the arithmetic of the production GPU kernel (glove.cu:
+ * glove_tile_kernel) instead of the specification above, for runs of one centre that no tile
+ * boundary splits: the context row takes T1[o] + (-g * h) rounded twice (a product, then an
+ * atomic add) instead of one fused multiply-add, and the centre row is written back as
+ * T0[c] + (h - h0), h0 being the row as the run loaded it, instead of h.
  */
 int orc_glove_train(const uint32_t *centre, const uint32_t *context, const uint32_t *count,
                     uint64_t n_triples, uint32_t max_count, uint32_t embedding_size,
                     uint32_t row_stride, float alpha, float clipping_value, float learning_rate,
-                    float *t0, float *t1, double *loss_sum, uint64_t *trained);
+                    int tile_semantics, float *t0, float *t1, double *loss_sum, uint64_t *trained);
 
 #ifdef __cplusplus
 }
